@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the B200 visibility pipeline (BASELINE.json metric: Gmeshlets culled/s).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload (N=1): BASELINE config C2 — procedural 10k-entity / 2M-meshlet city, one 1920x1080 view, two-pass
 occlusion. One *step* = the reference's culling of one steady-state frame (BASELINE.md protocol):
@@ -24,6 +24,10 @@ Static assets (meshlets, mesh infos, materials) stay resident like the reference
 
 --impl reference: the reference's CPU implementation of the path = the oracle port (OpenMP, all host cores) on the
 same config; rank 0 only.
+
+--dump-outputs DIR: after the K timed steps, rank 0 writes what the last of them handed its caller as DIR/<name>.npy
+(see step_outputs). The inputs are generated from fixed seeds, so two builds (or the two --impl arms) run with the same
+arguments can be compared output for output.
 """
 import argparse
 import json
@@ -45,6 +49,7 @@ UNIT = "Gmeshlets/s"
 WORKLOAD = "C2 city 10k entities / 2M meshlets, one 1920x1080 view per GPU, steady-state frame: early cull + Hi-Z + late cull + main cull"
 N_COPIES = 4
 KERNELS_PER_STEP = 7    # early: entity_cull, meshlet test, meshlet_emit; hiz_build; late + main fused: entity_cull, meshlet test, one meshlet_emit launch for both lists
+DUMP_LIMIT_BYTES = 64 * 2 ** 20
 
 
 def c2_view(scenes, scene, index):
@@ -117,6 +122,36 @@ def late_meshlet_algorithmic_bytes(records, n_draws, n_materials=16, passes_vis=
     return 32 * lanes + 16 * R + 12 + 64 * E + 400 + 80 * n_materials + 4 * R * passes_vis + 4 + 28 * n_draws, lanes, R, E
 
 
+def step_outputs(passes, entity_visibility, meshlet_visibility, hiz_texels):
+    """What one step hands its caller: per pass ("early", "late", "main") the dispatch header, records, draw count and draw
+    commands (`passes[k]` = (header, records, draws) as read_dispatch / read_draws return them), the two visibility bitmasks
+    the next frame reads and the Hi-Z pyramid. 32-bit words become float64 (exact); the texels stay float32. A list with
+    no entries (the late pass emits nothing in the steady state) is left out; its count and header say it is empty."""
+    words = lambda a, cols: np.ascontiguousarray(a).view(np.uint32).reshape(-1, cols).astype(np.float64)
+    out = {}
+    for k, (hdr, recs, draws) in passes.items():
+        out[k + "_dispatch_header"] = np.asarray(hdr, np.uint32).astype(np.float64)
+        out[k + "_draw_count"] = np.array([len(draws)], np.float64)
+        if len(recs):
+            out[k + "_dispatch_records"] = words(recs, 4)
+        if len(draws):
+            out[k + "_draw_commands"] = words(draws, 7)
+    out["entity_visibility"] = words(entity_visibility, 1).reshape(-1)
+    out["meshlet_visibility"] = words(meshlet_visibility, 1).reshape(-1)
+    out["hiz_texels"] = np.asarray(hiz_texels, np.float32).reshape(-1)
+    return out
+
+
+def dump_outputs(out_dir, arrays):
+    # the dump is for comparing builds output for output, so it is refused rather than sampled (C2 dumps 16.5 MB)
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError("outputs of one step (%d bytes) exceed the %d-byte dump limit" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------------------
 def run_reference(args, rank, world):
     """Reference arm: the CPU restatement (oracle port, OpenMP) of the same step on the same config."""
@@ -132,16 +167,20 @@ def run_reference(args, rank, world):
     hs = O.HostScene(scene)
 
     def frame_once():
-        O.depth_prepass_culling(hs, view, depth)
-        O.main_pass_culling(hs, view)
+        out = O.depth_prepass_culling(hs, view, depth)
+        out["main"] = O.main_pass_culling(hs, view)
+        return out
     for _ in range(2):  # reach the steady state (frame 0 fills the visibility bits)
         frame_once()
     for _ in range(max(args.warmup, 1)):
         frame_once()
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        frame_once()
+        out = frame_once()
     dt = (time.perf_counter() - t0) / args.steps
+    if args.dump_outputs:
+        passes = {k: O.parse_dispatch(out[k][0]) + (O.parse_draws(out[k][1])[1],) for k in ("early", "late", "main")}
+        dump_outputs(args.dump_outputs, step_outputs(passes, hs.entity_visibility, hs.meshlet_visibility, hs.hiz_texels))
     value = scene.n_meshlet_instances / dt / 1e9
     cores = int(O.lib().oracle_threads())
     line = {"impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -407,6 +446,13 @@ def run_ours(args, rank, world, local_rank):
     barrier()
     step_ms = e0.elapsed_time(e1) / args.steps
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        last = copies[(args.steps - 1) % N_COPIES]
+        passes = {k: frame.read_dispatch(getattr(last, k + "_dispatch")) + (frame.read_draws(getattr(last, k + "_draws"))[1],)
+                  for k in ("early", "late", "main")}
+        vs = last.vstate
+        dump_outputs(args.dump_outputs, step_outputs(passes, vs.entity_visibility.cpu().numpy(), vs.meshlet_visibility.cpu().numpy(),
+                                                     vs.depth_pyramid.texels.cpu().numpy()))
     if args.step_only:   # for `ncu` launch lists: the last KERNELS_PER_STEP x steps kernels of the process are exactly the timed region
         if rank == 0:
             print(json.dumps({"step_only": True, "ms_per_step": step_ms, "steps": args.steps}), flush=True)
@@ -704,6 +750,7 @@ def main():
     ap.add_argument("--step-only", action="store_true", help="stop after the timed region (profiling aid)")
     ap.add_argument("--no-configs", action="store_true", help="skip the nested C3 / C5 measurements")
     ap.add_argument("--no-parity", action="store_true", help="skip the oracle parity bits of the extras")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
