@@ -49,7 +49,8 @@
 extern "C" {
 #endif
 
-/* 3: orbit_*_late_main + orbit_cull_pair_compatible, orbit_peer_put / orbit_peer_wait, OrbitStatus::peer_timeout (was reserved[0]),
+/* 3: orbit_entity_cull_views / orbit_meshlet_cull_views (batched pass-0 views; additive, no layout changed),
+ *    orbit_*_late_main + orbit_cull_pair_compatible, orbit_peer_put / orbit_peer_wait, OrbitStatus::peer_timeout (was reserved[0]),
  *    orbit_record_masks_put / region form of orbit_draws_from_masks (replace orbit_record_masks_scatter_ranked).
  * 2: device guards on every entry point, orbit_ctx_reserve, orbit_meshlet_test, scatter sources clamped to their capacity. */
 #define ORBIT_ABI_VERSION 3
@@ -186,6 +187,37 @@ int orbit_meshlet_cull_late_main(orbit_ctx* ctx, const OrbitCullInfo* late, cons
                                  uint64_t capacity_records, void* late_draw_command_buffer, void* main_draw_command_buffer,
                                  uint64_t capacity_draws, void* late_task_payloads /* nullable */,
                                  void* main_task_payloads /* nullable */, void* stream);
+
+/* ---- batched pass-0 views (the cascades of ShadowRenderer::render_cascaded_shadow, shadow_renderer.rs:466-712; many cameras
+ *      over one scene) ---------------------------------------------------------------------------------------------------
+ * n_views (1..ORBIT_MAX_BATCH_VIEWS) pass-0 views of ONE scene. View v's buffers are byte for byte what
+ *   orbit_entity_cull(&culls[v], ...) ; orbit_meshlet_cull(&culls[v], ...)
+ * write: header, records / commands in canonical order, and task payloads. 3 kernel launches per call pair, whatever n_views
+ * is: one entity kernel over n_views x ceil(draws / 256) tiles, one test kernel over the concatenation of the views' record
+ * lists, one emit kernel with a row of CTAs per view.
+ *   - every view has its own OrbitCullInfo (view matrix, 0..12 planes, LOD target / base / step / range, alpha filter), but
+ *     all views of a call have the same projection_type and occlusion_pass == 0;
+ *   - `scene` (draw_begin / draw_end included) is shared by all views; dispatch_buffers[v] / draw_command_buffers[v] are view
+ *     v's outputs (no two views may share one), all of `capacity_records` / `capacity_draws`; task_payloads may be NULL, and
+ *     so may any of its entries;
+ *   - ORBIT_ERR_INVALID_ARGUMENT, with nothing launched, for: n_views 0 or above the maximum, a view with occlusion_pass != 0,
+ *     mixed projection types, more than 12 planes, a NULL or misaligned buffer, two views sharing a buffer, and everything
+ *     orbit_entity_cull / orbit_meshlet_cull refuse;
+ *   - overflow as in the single-view calls: each view's header stays exact, records / commands beyond capacity are dropped,
+ *     OrbitStatus.dispatch_overflow / draw_overflow are set if any view overflowed;
+ *   - concurrency: orbit_entity_cull_views counts as an orbit_entity_cull call and orbit_meshlet_cull_views as an
+ *     orbit_meshlet_cull call; calls of both forms may be interleaved on one stream in any order (the batched meshlet stage
+ *     keeps its survivor counters apart from the single-view ones). Replay-safe under CUDA-graph capture.
+ *   - scratch: the per-record scratch of the meshlet stage grows to n_views x capacity_records records, 528 bytes per record
+ *     (C4's four cascades: ~0.74 GB; C5, 16 views: ~5.9 GB); orbit_ctx_reserve(ctx, .., n_views * capacity_records, ..)
+ *     pre-sizes it. The first orbit_meshlet_cull_views call of a context also allocates the batched stage's survivor counters
+ *     (256 KB): make one batched call before capturing batched calls into a CUDA graph. */
+#define ORBIT_MAX_BATCH_VIEWS 16
+int orbit_entity_cull_views(orbit_ctx* ctx, const OrbitCullInfo* culls, uint32_t n_views, const OrbitSceneBuffers* scene,
+                            void* const* dispatch_buffers, uint64_t capacity_records, void* stream);
+int orbit_meshlet_cull_views(orbit_ctx* ctx, const OrbitCullInfo* culls, uint32_t n_views, const OrbitSceneBuffers* scene,
+                             const void* const* dispatch_buffers, uint64_t capacity_records, void* const* draw_command_buffers,
+                             uint64_t capacity_draws, void* const* task_payloads /* NULL, or entries may be NULL */, void* stream);
 
 /* ---- compute_clusters (cluster.rs:368-591) + light_cluster/{mark_active,active_cluster_compaction,
  *      light_culling}.comp --------------------------------------------------------------------------------- */

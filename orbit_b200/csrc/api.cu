@@ -24,6 +24,8 @@ bool pdl_enabled() {
 }  // namespace orbit
 
 static thread_local int g_last_cuda_error = 0;
+static constexpr size_t kViewChunkWords = 2u * 2048u;   // per view: two parities of chunk counts
+static constexpr size_t kViewCounterWords = ORBIT_MAX_BATCH_VIEWS * (kViewChunkWords + 4u);
 #define CK(expr)                                                       \
     do {                                                               \
         cudaError_t e_ = (expr);                                       \
@@ -59,6 +61,11 @@ struct orbit_ctx {
     OrbitStatus* status_host = nullptr;
     OrbitStatus* status_dev = nullptr;
     uint32_t* chunk_counts = nullptr; // 2 x 2048 per-chunk survivor counts
+    uint32_t* view_counters = nullptr;// batched views (orbit_meshlet_cull_views): 16 x 2 x 2048 chunk counts, then 16 x {survivor totals
+                                      // per parity, parity words A/B} — apart from the single-view words, so both forms may interleave.
+                                      // Allocated by the first batched call, never in orbit_ctx_create: an allocation there moves the
+                                      // buffers created after it (the scan descriptors the entity kernel polls), and the single-view
+                                      // entity stage measured ~1 us slower on C2 with its descriptors at the shifted address
     // meshlet stage scratch: one draw mask per dispatch record
     uint4* draw_masks = nullptr;
     uint4* cmd_side = nullptr;        // 32 entries per dispatch record, same capacity as draw_masks
@@ -77,7 +84,9 @@ struct orbit_ctx {
     int emit_occupancy = 0;
     int debug_skip = 0;               // ORBIT_DEBUG_SKIP: 1 = skip emit kernel, 2 = skip test kernel (timing experiments only)
     int entity_occupancy = 0;
+    int entity_views_occupancy = 0;   // the same for the batched entity kernel (more registers: fewer CTAs per SM)
     int mc_occupancy[8] = {0, 0, 0, 0, 0, 0, 0, 0};   // cached occupancy per meshlet test-kernel variant
+    int views_occupancy[3] = {0, 0, 0};                // the same for the batched test kernel, per projection (0, 1, other)
     int emit_ctas_per_sm = 0;         // ORBIT_EMIT_CTAS_PER_SM (tuning knob, read once at creation)
     // Scratch that was outgrown is parked here until the context is destroyed: freeing it would need a device
     // synchronisation (work that uses it may still be in flight), and a stage call never synchronises.
@@ -273,7 +282,7 @@ void orbit_ctx_destroy(orbit_ctx* c) {
     DeviceGuard guard(c->device);
     cudaDeviceSynchronize();
     for (int i = 0; i < c->n_retired; ++i) cudaFree(c->retired[i]);
-    cudaFree(c->status); cudaFree(c->counters); cudaFree(c->light_view); cudaFree(c->light_hits); cudaFree(c->draw_masks); cudaFree(c->cmd_side); cudaFree(c->main_masks); cudaFree(c->chunk_counts); cudaFree(c->tile_sums);
+    cudaFree(c->status); cudaFree(c->counters); cudaFree(c->light_view); cudaFree(c->light_hits); cudaFree(c->draw_masks); cudaFree(c->cmd_side); cudaFree(c->main_masks); cudaFree(c->chunk_counts); cudaFree(c->view_counters); cudaFree(c->tile_sums);
     cudaFree(c->trace);
     cudaFreeHost(c->status_host);
     delete c;
@@ -410,33 +419,55 @@ static int check_cull(const OrbitCullInfo* cull, const OrbitSceneBuffers* scene,
     return ORBIT_OK;
 }
 
-static int entity_stage(orbit_ctx* c, const OrbitCullInfo* cull, const OrbitSceneBuffers* scene, const orbit_hiz* hiz,
-                        void* meshlet_dispatch_buffer, void* mirror_dispatch_buffer, uint64_t capacity_records, void* stream) {
-    if (!c || !meshlet_dispatch_buffer || ((uintptr_t)meshlet_dispatch_buffer & 3u)) return ORBIT_ERR_INVALID_ARGUMENT;
-    int rc = check_cull(cull, scene, hiz, false);
-    if (rc != ORBIT_OK) return rc;
-    uint32_t begin = scene->draw_begin, end = scene->draw_end;
-    if (begin == 0u && end == 0u) end = scene->entity_draw_count;
-    if (end > scene->entity_draw_count) end = scene->entity_draw_count;
-    if (begin > end) return ORBIT_ERR_INVALID_ARGUMENT;
-    const uint32_t n = end - begin;
-    GUARD(c);
-    rc = ensure_status(c, (size_t)(n + 255u) / 256u + 1u, (cudaStream_t)stream);
-    if (rc != ORBIT_OK) return rc;
+// draws [begin, end) a call covers (OrbitSceneBuffers::draw_begin / draw_end, 0,0 = all)
+static int draw_range(const OrbitSceneBuffers* scene, uint32_t* begin, uint32_t* end) {
+    *begin = scene->draw_begin; *end = scene->draw_end;
+    if (*begin == 0u && *end == 0u) *end = scene->entity_draw_count;
+    if (*end > scene->entity_draw_count) *end = scene->entity_draw_count;
+    return *begin > *end ? ORBIT_ERR_INVALID_ARGUMENT : ORBIT_OK;
+}
+
+static EntityCullParams entity_params(orbit_ctx* c, const OrbitCullInfo* cull, const OrbitSceneBuffers* scene, const orbit_hiz* hiz,
+                                      void* dispatch_buffer, uint64_t capacity_records, uint32_t begin, uint32_t end) {
     EntityCullParams p{};
     p.cull = *cull; p.hiz = hiz_device(hiz);
     p.entity_draw_words = (const uint32_t*)scene->entity_draws;
     p.mesh_infos = (const uint8_t*)scene->mesh_infos;
     p.entities = (const float4*)scene->entities;
     p.entity_visibility = scene->entity_visibility;
-    p.dispatch_words = (uint32_t*)meshlet_dispatch_buffer;
-    p.dispatch_mirror = (uint32_t*)mirror_dispatch_buffer;
+    p.dispatch_words = (uint32_t*)dispatch_buffer;
     p.overflow_flag = &c->status_dev->dispatch_overflow;
     p.capacity_records = capacity_records;
     p.draw_begin = begin; p.draw_end = end;
-    p.scan = next_scan(c);
+    return p;
+}
+
+static uint32_t entity_coresident_ctas(orbit_ctx* c) {
     if (c->entity_occupancy <= 0) c->entity_occupancy = entity_cull_max_ctas_per_sm();
-    CK(launch_entity_cull(p, n, (uint32_t)(c->sm_count * (c->entity_occupancy > 0 ? c->entity_occupancy : 1)), (cudaStream_t)stream));
+    return (uint32_t)(c->sm_count * (c->entity_occupancy > 0 ? c->entity_occupancy : 1));
+}
+
+static uint32_t entity_views_coresident_ctas(orbit_ctx* c) {
+    if (c->entity_views_occupancy <= 0) c->entity_views_occupancy = entity_cull_views_max_ctas_per_sm();
+    return (uint32_t)(c->sm_count * (c->entity_views_occupancy > 0 ? c->entity_views_occupancy : 1));
+}
+
+static int entity_stage(orbit_ctx* c, const OrbitCullInfo* cull, const OrbitSceneBuffers* scene, const orbit_hiz* hiz,
+                        void* meshlet_dispatch_buffer, void* mirror_dispatch_buffer, uint64_t capacity_records, void* stream) {
+    if (!c || !meshlet_dispatch_buffer || ((uintptr_t)meshlet_dispatch_buffer & 3u)) return ORBIT_ERR_INVALID_ARGUMENT;
+    int rc = check_cull(cull, scene, hiz, false);
+    if (rc != ORBIT_OK) return rc;
+    uint32_t begin, end;
+    rc = draw_range(scene, &begin, &end);
+    if (rc != ORBIT_OK) return rc;
+    const uint32_t n = end - begin;
+    GUARD(c);
+    rc = ensure_status(c, (size_t)(n + 255u) / 256u + 1u, (cudaStream_t)stream);
+    if (rc != ORBIT_OK) return rc;
+    EntityCullParams p = entity_params(c, cull, scene, hiz, meshlet_dispatch_buffer, capacity_records, begin, end);
+    p.dispatch_mirror = (uint32_t*)mirror_dispatch_buffer;
+    p.scan = next_scan(c);
+    CK(launch_entity_cull(p, n, entity_coresident_ctas(c), (cudaStream_t)stream));
     c->launches += 1;
     return ORBIT_OK;
 }
@@ -479,6 +510,34 @@ int orbit_entity_cull_late_main(orbit_ctx* c, const OrbitCullInfo* late, const O
 }
 
 // ---- meshlet stage ---------------------------------------------------------------------------------------
+// The CullInfo and the planes paired for the packed test kernel (MeshletCullParams::planes_t)
+static void set_cull(MeshletCullParams& p, const OrbitCullInfo* cull) {
+    p.cull = *cull;
+    p.pk_one = make_float2(1.0f, 1.0f); p.pk_mone = make_float2(-1.0f, -1.0f);
+    for (uint32_t j = 0; j < 6u; ++j) {
+        const uint32_t n = cull->cull_plane_count;
+        const uint32_t a = 2u * j < n ? 2u * j : (n ? n - 1u : 0u), b = 2u * j + 1u < n ? 2u * j + 1u : a;
+        for (int cc = 0; cc < 4; ++cc) p.planes_t[j][cc] = make_float2(cull->cull_planes[a][cc], cull->cull_planes[b][cc]);
+    }
+}
+
+// Emit grid for a dispatch buffer of max_records records; *small_grid = the CTAs that take part when the list is short.
+static uint64_t emit_grids(orbit_ctx* c, uint64_t max_records, uint32_t* small_grid) {
+    // emit kernel: two CTAs per SM (every CTA repeats the 2048-entry chunk scan; more CTAs only add to that)
+    if (c->emit_occupancy <= 0) c->emit_occupancy = meshlet_emit_max_ctas_per_sm();
+    // emit kernel: as many CTAs per SM as fit (3) for long lists; two per SM take part when the list is short (decided on the
+    // device from the survivor count, see meshlet_emit_body)
+    int emit_per_sm = c->emit_occupancy > 0 ? c->emit_occupancy : 1;
+    if (emit_per_sm > 4) emit_per_sm = 4;
+    // even CTAs that leave at once cost launch time (C2 frame: +1.6 us over its three emit launches), so a dispatch buffer too
+    // small for a long list (capacity below 2^18 records = 8 M meshlets) gets the two per SM of the short case outright
+    if (max_records < (1u << 18) && emit_per_sm > 2) emit_per_sm = 2;
+    int emit_small_per_sm = emit_per_sm < 2 ? emit_per_sm : 2;
+    if (c->emit_ctas_per_sm >= 1 && c->emit_ctas_per_sm <= c->emit_occupancy) emit_per_sm = emit_small_per_sm = c->emit_ctas_per_sm;   // tuning knob
+    *small_grid = (uint32_t)(c->sm_count * emit_small_per_sm);
+    return (uint64_t)c->sm_count * (uint64_t)emit_per_sm;
+}
+
 // mode 0: test + emit (orbit_meshlet_cull); mode 1: test only, record entries into `record_masks` (orbit_meshlet_test)
 struct MainPassOutputs { const OrbitCullInfo* cull; void* draw_command_buffer; void* task_payloads; };   // fused LATE + MAIN
 
@@ -506,7 +565,7 @@ static int meshlet_stage(orbit_ctx* c, const OrbitCullInfo* cull, const OrbitSce
         if (rc != ORBIT_OK) return rc;
     }
     MeshletCullParams p{};
-    p.cull = *cull; p.hiz = hiz_device(hiz);
+    p.hiz = hiz_device(hiz);
     p.dispatch_words = (const uint32_t*)meshlet_dispatch_buffer;
     p.meshlets = (const uint4*)scene->meshlets;
     p.entities = (const float4*)scene->entities;
@@ -541,12 +600,7 @@ static int meshlet_stage(orbit_ctx* c, const OrbitCullInfo* cull, const OrbitSce
     p.capacity_draws = capacity_draws;
     p.scan.trace = next_trace(c);
     p.trace_emit = next_trace(c);
-    p.pk_one = make_float2(1.0f, 1.0f); p.pk_mone = make_float2(-1.0f, -1.0f);
-    for (uint32_t j = 0; j < 6u; ++j) {
-        const uint32_t n = cull->cull_plane_count;
-        const uint32_t a = 2u * j < n ? 2u * j : (n ? n - 1u : 0u), b = 2u * j + 1u < n ? 2u * j + 1u : a;
-        for (int cc = 0; cc < 4; ++cc) p.planes_t[j][cc] = make_float2(cull->cull_planes[a][cc], cull->cull_planes[b][cc]);
-    }
+    set_cull(p, cull);
     // test kernel: persistent warps, cyclic tiles, no inter-CTA dependency -> one full wave of CTAs
     int& occ_slot = c->mc_occupancy[meshlet_cull_variant_index(*cull)];
     if (occ_slot <= 0) occ_slot = meshlet_cull_max_ctas_per_sm(p);
@@ -554,19 +608,9 @@ static int meshlet_stage(orbit_ctx* c, const OrbitCullInfo* cull, const OrbitSce
     int per_sm = c->mc_ctas_per_sm;
     if (per_sm <= 0) per_sm = occ > 0 ? occ : 1;
     const uint64_t grid = (uint64_t)c->sm_count * (uint64_t)per_sm;
-    // emit kernel: two CTAs per SM (every CTA repeats the 2048-entry chunk scan; more CTAs only add to that)
-    if (c->emit_occupancy <= 0) c->emit_occupancy = meshlet_emit_max_ctas_per_sm();
-    // emit kernel: as many CTAs per SM as fit (3) for long lists; two per SM take part when the list is short (decided on the
-    // device from the survivor count, see meshlet_emit_body)
-    int emit_per_sm = c->emit_occupancy > 0 ? c->emit_occupancy : 1;
-    if (emit_per_sm > 4) emit_per_sm = 4;
-    // even CTAs that leave at once cost launch time (C2 frame: +1.6 us over its three emit launches), so a dispatch buffer too
-    // small for a long list (capacity below 2^18 records = 8 M meshlets) gets the two per SM of the short case outright
-    if (max_records < (1u << 18) && emit_per_sm > 2) emit_per_sm = 2;
-    int emit_small_per_sm = emit_per_sm < 2 ? emit_per_sm : 2;
-    if (c->emit_ctas_per_sm >= 1 && c->emit_ctas_per_sm <= c->emit_occupancy) emit_per_sm = emit_small_per_sm = c->emit_ctas_per_sm;   // tuning knob
-    const uint64_t emit_grid = (uint64_t)c->sm_count * (uint64_t)emit_per_sm;
-    p.emit_small_grid = (uint32_t)(c->sm_count * emit_small_per_sm);
+    uint32_t emit_small_grid;
+    const uint64_t emit_grid = emit_grids(c, max_records, &emit_small_grid);
+    p.emit_small_grid = emit_small_grid;
     const bool skip_emit = test_only || c->debug_skip == 1;
     const bool pair = fused_main && !skip_emit;      // both lists leave in one emit launch
     CK(launch_meshlet_cull(p, c->debug_skip == 2 ? 0 : (int)grid, (skip_emit || pair) ? 0 : (int)emit_grid, (cudaStream_t)stream));
@@ -648,6 +692,106 @@ int orbit_draws_from_masks(orbit_ctx* c, const OrbitSceneBuffers* scene, const v
     if (emit_per_sm > 4) emit_per_sm = 4;
     p.emit_small_grid = (uint32_t)(c->sm_count * (emit_per_sm < 2 ? emit_per_sm : 2));
     CK(launch_draws_from_masks(p, c->counters + 16, c->sm_count * 4, c->sm_count * emit_per_sm, (cudaStream_t)stream));
+    c->launches += 2;
+    return ORBIT_OK;
+}
+
+// ---- batched pass-0 views ---------------------------------------------------------------------------------
+// Checks shared by both stages: the view count, every view's CullInfo (pass 0, one projection type, check_cull), and one
+// output buffer per view — present, 4-byte aligned, none shared with another view.
+static int check_views(const OrbitCullInfo* culls, uint32_t n_views, const OrbitSceneBuffers* scene, const void* const* buffers,
+                       bool meshlet_stage) {
+    if (!culls || !buffers || n_views == 0u || n_views > ORBIT_MAX_BATCH_VIEWS) return ORBIT_ERR_INVALID_ARGUMENT;
+    for (uint32_t v = 0; v < n_views; ++v) {
+        int rc = check_cull(&culls[v], scene, nullptr, meshlet_stage);
+        if (rc != ORBIT_OK) return rc;
+        if (culls[v].occlusion_pass != 0u || culls[v].projection_type != culls[0].projection_type) return ORBIT_ERR_INVALID_ARGUMENT;
+        if (!buffers[v] || ((uintptr_t)buffers[v] & 3u)) return ORBIT_ERR_INVALID_ARGUMENT;
+        for (uint32_t u = 0; u < v; ++u) if (buffers[u] == buffers[v]) return ORBIT_ERR_INVALID_ARGUMENT;
+    }
+    return ORBIT_OK;
+}
+
+int orbit_entity_cull_views(orbit_ctx* c, const OrbitCullInfo* culls, uint32_t n_views, const OrbitSceneBuffers* scene,
+                            void* const* dispatch_buffers, uint64_t capacity_records, void* stream) {
+    if (!c) return ORBIT_ERR_INVALID_ARGUMENT;
+    int rc = check_views(culls, n_views, scene, (const void* const*)dispatch_buffers, false);
+    if (rc != ORBIT_OK) return rc;
+    uint32_t begin, end;
+    rc = draw_range(scene, &begin, &end);
+    if (rc != ORBIT_OK) return rc;
+    const uint32_t n = end - begin;
+    GUARD(c);
+    rc = ensure_status(c, (size_t)n_views * ((n + 255u) / 256u + 1u), (cudaStream_t)stream);   // one descriptor block per view
+    if (rc != ORBIT_OK) return rc;
+    EntityViewsParams pv{};
+    pv.n_views = n_views;
+    for (uint32_t v = 0; v < n_views; ++v) pv.view[v] = entity_params(c, &culls[v], scene, nullptr, dispatch_buffers[v], capacity_records, begin, end);
+    pv.view[0].scan = next_scan(c);
+    CK(launch_entity_cull_views(pv, n, entity_views_coresident_ctas(c), (cudaStream_t)stream));
+    c->launches += 1;
+    return ORBIT_OK;
+}
+
+int orbit_meshlet_cull_views(orbit_ctx* c, const OrbitCullInfo* culls, uint32_t n_views, const OrbitSceneBuffers* scene,
+                             const void* const* dispatch_buffers, uint64_t capacity_records, void* const* draw_command_buffers,
+                             uint64_t capacity_draws, void* const* task_payloads, void* stream) {
+    if (!c) return ORBIT_ERR_INVALID_ARGUMENT;
+    int rc = check_views(culls, n_views, scene, dispatch_buffers, true);
+    if (rc == ORBIT_OK) rc = check_views(culls, n_views, scene, (const void* const*)draw_command_buffers, true);
+    if (rc != ORBIT_OK) return rc;
+    for (uint32_t v = 0; task_payloads && v < n_views; ++v) {
+        if ((uintptr_t)task_payloads[v] & 3u) return ORBIT_ERR_INVALID_ARGUMENT;
+        for (uint32_t u = 0; u < v; ++u) if (task_payloads[v] && task_payloads[u] == task_payloads[v]) return ORBIT_ERR_INVALID_ARGUMENT;
+    }
+    if (capacity_records > 0xFFFFFFFFull) capacity_records = 0xFFFFFFFFull;
+    GUARD(c);
+    // draw masks + side words of view v live at records [v * capacity_records, (v + 1) * capacity_records) of the grown scratch
+    rc = ensure_record_scratch(c, (uint64_t)n_views * capacity_records);
+    if (rc != ORBIT_OK) return rc;
+    if (!c->view_counters) {   // first batched call: the counter block, zeroed in stream order ahead of the kernels
+        CK(cudaMalloc(&c->view_counters, kViewCounterWords * sizeof(uint32_t)));
+        CK(cudaMemsetAsync(c->view_counters, 0, kViewCounterWords * sizeof(uint32_t), (cudaStream_t)stream));
+    }
+    // emit: a row of CTAs per view. Every row gets the single-view grid, so a long list is walked by as many CTAs as a
+    // single-view call gives it and the rows of short lists leave the machine to it (the lists of one batch differ by up to
+    // four orders of magnitude: C5 cameras 1.4 k .. 9.4 M draws; rows of emit_grid / n_views CTAs made the 16-camera batch
+    // 1.5x slower than separate calls, tools/bench_views.py). Short lists are emitted by small_grid / n_views CTAs of their
+    // row, so a batch of short lists keeps the single-view number of working CTAs; the others leave at once.
+    uint32_t small_grid;
+    const uint64_t emit_grid = emit_grids(c, capacity_records, &small_grid);
+    const uint32_t emit_per_view = (uint32_t)emit_grid;
+    const uint32_t small_per_view = (small_grid + n_views - 1u) / n_views;
+    MeshletViewsParams pv{};
+    pv.n_views = n_views;
+    for (uint32_t v = 0; v < n_views; ++v) {
+        MeshletCullParams& p = pv.view[v];
+        set_cull(p, &culls[v]);
+        p.dispatch_words = (const uint32_t*)dispatch_buffers[v];
+        p.meshlets = (const uint4*)scene->meshlets;
+        p.entities = (const float4*)scene->entities;
+        p.materials = (const uint8_t*)scene->materials;
+        p.meshlet_visibility = scene->meshlet_visibility;
+        p.draw_words = (uint32_t*)draw_command_buffers[v];
+        p.task_payloads = task_payloads ? (uint32_t*)task_payloads[v] : nullptr;
+        p.overflow_flag = &c->status_dev->draw_overflow;
+        p.draw_masks = c->draw_masks + (size_t)v * capacity_records;
+        p.cmd_side = c->cmd_side + (size_t)v * capacity_records * 32u;
+        p.chunk_counts = c->view_counters + v * kViewChunkWords;
+        p.draw_total = c->view_counters + ORBIT_MAX_BATCH_VIEWS * kViewChunkWords + 4u * v;   // [0],[1]
+        p.chunk_parity = p.draw_total + 2;                                                   // [2] word A, [3] word B
+        p.capacity_records = capacity_records;
+        p.capacity_draws = capacity_draws;
+        p.emit_small_grid = small_per_view;
+    }
+    pv.view[0].scan.trace = next_trace(c);
+    pv.view[0].trace_emit = next_trace(c);
+    const uint32_t proj = culls[0].projection_type;
+    int& occ_slot = c->views_occupancy[proj <= 1u ? proj : 2u];
+    if (occ_slot <= 0) occ_slot = meshlet_cull_views_max_ctas_per_sm(proj);
+    int per_sm = c->mc_ctas_per_sm;
+    if (per_sm <= 0) per_sm = occ_slot > 0 ? occ_slot : 1;
+    CK(launch_meshlet_cull_views(pv, c->sm_count * per_sm, (int)emit_per_view, (cudaStream_t)stream));
     c->launches += 2;
     return ORBIT_OK;
 }

@@ -503,9 +503,17 @@ __device__ __forceinline__ void tile_model_view(const float4* rows, float* mv_ba
 // words are stored as 0 when their tile starts and visible candidates OR their bit in afterwards (RED.OR; a __syncwarp
 // between the stores and the first drain orders the two), likewise the draw masks and the chunks' survivor counts — so
 // a record never waits for its candidates and there are no per-record result masks to carry.
-template <int R, bool kPass2, int kProj>
-__global__ void __launch_bounds__(kDwThreads, ORBIT_DIRECT_MIN_CTAS) meshlet_test_direct_kernel(const __grid_constant__ MeshletCullParams p) {
+//
+// kBatch (orbit_meshlet_cull_views, pass 0): the tiles are those of the CONCATENATION of views[0..n_views)'s record lists,
+// each view's list cut into tiles of its own (a tile never straddles two views). Every CTA reads the views' record counts
+// once (one round trip; lane v of every warp holds view v's count and one past its last tile); a tile takes view matrix, paired
+// planes and alpha filter from its view's block, and its draw masks, side words and survivor counts go to that view's scratch.
+// The scene fields (meshlets, entities, materials) are read from views[0].
+template <int R, bool kPass2, int kProj, bool kBatch>
+__device__ __forceinline__ void meshlet_test_direct_body(const MeshletCullParams* views, uint32_t n_views) {
     static_assert(R == 2 || R == 4 || R == 8, "records per warp tile");
+    static_assert(!(kBatch && kPass2), "batched views are pass 0");
+    const MeshletCullParams& p = views[0];
     extern __shared__ __align__(128) unsigned char s_raw[];
     WarpSmem<R>* const all = reinterpret_cast<WarpSmem<R>*>(s_raw + 128);
     uint32_t* const s_next_tile = reinterpret_cast<uint32_t*>(s_raw);
@@ -539,18 +547,52 @@ __global__ void __launch_bounds__(kDwThreads, ORBIT_DIRECT_MIN_CTAS) meshlet_tes
         if (lane < 4u * R && (uint64_t)tile * R + (lane >> 2) < bound) w = __ldcg(p.dispatch_words + 3u + (size_t)tile * R * 4u + lane);
         return w;
     };
-    uint32_t cur_word = load_words(t_cur, p.capacity_records), next_word = load_words(t_next, p.capacity_records);
-    uint32_t nrec = __ldcg(p.dispatch_words);  // workgroup_count_x written by the entity stage
-    if ((uint64_t)nrec > p.capacity_records) nrec = (uint32_t)p.capacity_records;
+    // batched views: lane v < n_views holds view v's record count, its survivor-counter parity and one past its last tile
+    uint32_t v_nrec = 0u, v_half = 0u, v_tile_end = 0u;
+    if constexpr (kBatch) {
+        if (lane < n_views) {
+            v_nrec = (uint32_t)min((uint64_t)__ldcg(views[lane].dispatch_words), views[lane].capacity_records);
+            v_half = __ldcg(views[lane].chunk_parity) & 1u;                   // see below: one parity per view
+            if (blockIdx.x == 0 && warp == 0u) views[lane].chunk_parity[1] = v_half;
+        }
+        v_tile_end = (v_nrec + R - 1) / R;
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) {
+            const uint32_t t = __shfl_up_sync(0xFFFFFFFFu, v_tile_end, d);
+            if (lane >= (uint32_t)d) v_tile_end += t;
+        }
+    }
+    // tile t of the concatenation (warp-uniform, t < tiles_total) -> view, first record inside the view, the view's record count
+    struct ViewTile { uint32_t view, rec0, nrec; };
+    auto locate = [&](uint32_t t) -> ViewTile {
+        const uint32_t v = (uint32_t)__popc(__ballot_sync(0xFFFFFFFFu, lane < n_views && v_tile_end <= t));
+        const uint32_t first = __shfl_sync(0xFFFFFFFFu, v_tile_end, (v - 1u) & 31u);
+        return ViewTile{v, (t - (v ? first : 0u)) * R, __shfl_sync(0xFFFFFFFFu, v_nrec, v & 31u)};
+    };
+    auto load_view_words = [&](uint32_t tile) -> uint32_t {
+        const ViewTile w = locate(tile);
+        uint32_t x = 0u;
+        if (lane < 4u * R && w.rec0 + (lane >> 2) < w.nrec) x = __ldcg(views[w.view].dispatch_words + 3u + (size_t)w.rec0 * 4u + lane);
+        return x;
+    };
+    uint32_t cur_word = 0u, next_word = 0u, nrec = 0u;
+    if constexpr (!kBatch) {
+        cur_word = load_words(t_cur, p.capacity_records); next_word = load_words(t_next, p.capacity_records);
+        nrec = __ldcg(p.dispatch_words);  // workgroup_count_x written by the entity stage
+        if ((uint64_t)nrec > p.capacity_records) nrec = (uint32_t)p.capacity_records;
+    }
     ORBIT_TRACE_STAMP(p.scan.trace, 1, 1 + 0 * (nrec & 1u));
-    const uint32_t chunk_shift = chunk_shift_of(nrec);
+    uint32_t chunk_shift = chunk_shift_of(nrec);     // batched views: those of the current tile's view (set per tile below)
     // Scratch is double-buffered by a parity that lives in device memory (CUDA-graph replays must see fresh state).
     // Word A is read by test kernels and written by emit kernels; word B the other way round: a kernel never writes
     // a word that CTAs of the same launch read, so the stream order of the launches is the only synchronisation.
-    const uint32_t half = __ldcg(p.chunk_parity) & 1u;
-    if (blockIdx.x == 0 && threadIdx.x == 0) p.chunk_parity[1] = half;
-    uint32_t* const chunk_counts = p.chunk_counts + half * kMaxChunks;
-    uint32_t* const draw_total = p.draw_total + half;
+    uint32_t half = 0u;
+    if constexpr (!kBatch) {
+        half = __ldcg(p.chunk_parity) & 1u;
+        if (blockIdx.x == 0 && threadIdx.x == 0) p.chunk_parity[1] = half;
+    }
+    uint32_t* chunk_counts = p.chunk_counts + half * kMaxChunks;
+    uint32_t* draw_total = p.draw_total + half;
     uint32_t* main_chunk_counts = nullptr;            // fused MAIN pass (pass 2 only): its own double-buffered scratch
     uint32_t main_total = 0u, mhalf = 0u;
     if (kPass2 && p.main_masks != nullptr) {
@@ -558,11 +600,16 @@ __global__ void __launch_bounds__(kDwThreads, ORBIT_DIRECT_MIN_CTAS) meshlet_tes
         if (blockIdx.x == 0 && threadIdx.x == 0) p.main_chunk_parity[1] = mhalf;
         main_chunk_counts = p.main_chunk_counts + mhalf * kMaxChunks;
     }
-    const uint32_t tiles_total = (nrec + R - 1) / R;
-    // row `lane&3` of the view matrix, for the 16-lane view*model product
+    const uint32_t tiles_total = kBatch ? __shfl_sync(0xFFFFFFFFu, v_tile_end, 31) : (nrec + R - 1) / R;
+    if constexpr (kBatch) {
+        if (t_cur < tiles_total) cur_word = load_view_words(t_cur);
+        if (t_next < tiles_total) next_word = load_view_words(t_next);
+    }
+    // row `lane&3` of the view matrix, for the 16-lane view*model product (batched views: the current tile's view)
     const uint32_t vrow_i = lane & 3u;
-    const float v0 = ci.view_matrix.m[0][vrow_i], v1 = ci.view_matrix.m[1][vrow_i];
-    const float v2 = ci.view_matrix.m[2][vrow_i], v3 = ci.view_matrix.m[3][vrow_i];
+    float v0 = ci.view_matrix.m[0][vrow_i], v1 = ci.view_matrix.m[1][vrow_i];
+    float v2 = ci.view_matrix.m[2][vrow_i], v3 = ci.view_matrix.m[3][vrow_i];
+    uint32_t cur_view = kBatch ? 0xFFFFFFFFu : 0u;    // no view yet: the first tile loads its view's state
     const uint32_t hiz_lw = 31u - (uint32_t)__clz((int)max(p.hiz.width, 1u)), hiz_lh = 31u - (uint32_t)__clz((int)max(p.hiz.height, 1u));
     float* const mv_base = &ws.mv[0][0];
     const uint32_t bar = smem_addr(&ws.bar);
@@ -600,7 +647,7 @@ __global__ void __launch_bounds__(kDwThreads, ORBIT_DIRECT_MIN_CTAS) meshlet_tes
             }
         }
     };
-    {   // the two speculative loads were bounded by the buffer capacity; now apply the real record count
+    if constexpr (!kBatch) {   // the two speculative loads were bounded by the buffer capacity; now apply the real record count
         if (!(lane < 4u * R && (uint64_t)t_cur * R + (lane >> 2) < (uint64_t)nrec)) cur_word = 0u;
         if (!(lane < 4u * R && (uint64_t)t_next * R + (lane >> 2) < (uint64_t)nrec)) next_word = 0u;
     }
@@ -613,13 +660,33 @@ __global__ void __launch_bounds__(kDwThreads, ORBIT_DIRECT_MIN_CTAS) meshlet_tes
     // One extra, empty iteration after the last tile flushes what is left in the ring through the same drain code.
     bool final_pass = t_cur >= tiles_total;
     while (true) {
-        const uint32_t rec0 = t_cur * R;
+        uint32_t rec0 = t_cur * R;
+        if constexpr (kBatch) {
+            if (!final_pass) {
+                const ViewTile w = locate(t_cur);
+                rec0 = w.rec0; nrec = w.nrec;
+                if (w.view != cur_view) {                                     // warp-uniform; a warp's tiles ascend, so do their views
+                    if (lane == 0u && warp_total != 0u) atomicAdd(draw_total, warp_total);
+                    warp_total = 0u;
+                    cur_view = w.view;
+                    const uint32_t h = __shfl_sync(0xFFFFFFFFu, v_half, cur_view);
+                    chunk_shift = chunk_shift_of(nrec);
+                    chunk_counts = views[cur_view].chunk_counts + h * kMaxChunks;
+                    draw_total = views[cur_view].draw_total + h;
+                    const OrbitCullInfo& cv = views[cur_view].cull;
+                    v0 = cv.view_matrix.m[0][vrow_i]; v1 = cv.view_matrix.m[1][vrow_i];
+                    v2 = cv.view_matrix.m[2][vrow_i]; v3 = cv.view_matrix.m[3][vrow_i];
+                }
+            }
+        }
+        const MeshletCullParams& pt = kBatch ? views[cur_view & (ORBIT_MAX_BATCH_VIEWS - 1)] : p;   // the tile's view
         const uint32_t my_word = final_pass ? 0u : cur_word;
         uint32_t my_mask = 0u;       // lane r < R: draw mask of record r (passes without Hi-Z)
         uint32_t vw = 0u;            // lane r < R, pass 2: last frame's visibility word of record r (decides should_draw)
         if (!final_pass) {
             cur_word = next_word;
-            next_word = t_next2 < tiles_total ? load_words(t_next2, nrec) : 0u;
+            if constexpr (kBatch) next_word = t_next2 < tiles_total ? load_view_words(t_next2) : 0u;
+            else next_word = t_next2 < tiles_total ? load_words(t_next2, nrec) : 0u;
             if (kPass2) {
                 // lane r: the record's visibility word is read, then stored as 0 — visible candidates OR their bits in
                 // afterwards (meshlet_cull.comp:235-242); likewise the draw mask
@@ -664,18 +731,18 @@ __global__ void __launch_bounds__(kDwThreads, ORBIT_DIRECT_MIN_CTAS) meshlet_tes
                 uint32_t alpha = 32u;                                               // out-of-record lanes: no alpha bit
                 if (in_rec) alpha = __ldg(reinterpret_cast<const uint32_t*>(      // L1-resident table; issued here, used after the test
                     p.materials + (size_t)(b.w & 0xFFFFu) * ORBIT_MATERIAL_STRIDE_BYTES + ORBIT_MATERIAL_ALPHA_MODE_OFFSET));
-                const ItemXY t = test_item_xy<kProj>(ci, p, k, c0, c1, c2, c3, scale, __uint_as_float(a.x), __uint_as_float(a.y),
+                const ItemXY t = test_item_xy<kProj>(pt.cull, pt, k, c0, c1, c2, c3, scale, __uint_as_float(a.x), __uint_as_float(a.y),
                                                      __uint_as_float(a.z), __uint_as_float(a.w), b.x);
                 const bool pre = in_rec && t.pre_visible;
                 if (!kPass2) {
                     // should_draw = visible && alpha passes the filter (meshlet_cull.comp:207)
-                    const bool draw = pre && (shl1(alpha) & ci.alpha_mode_flags) != 0u;
+                    const bool draw = pre && (shl1(alpha) & pt.cull.alpha_mode_flags) != 0u;
                     const uint32_t mask = __ballot_sync(0xFFFFFFFFu, draw);
                     if (lane == r) my_mask = mask;
                     // the command words of a survivor travel to the emit kernel through a side array (L2-resident at the sizes
                     // where the emit kernel is latency-bound; at C5 scale it replaces a second 32-byte read of every surviving meshlet)
                     const uint32_t ent_r = __shfl_sync(0xFFFFFFFFu, my_word, r * 4u);
-                    if (draw && p.cmd_side != nullptr) p.cmd_side[(size_t)(rec0 + r) * 32u + lane] = make_uint4(b.y, b.z, b.w, ent_r);
+                    if (draw && pt.cmd_side != nullptr) pt.cmd_side[(size_t)(rec0 + r) * 32u + lane] = make_uint4(b.y, b.z, b.w, ent_r);
                 } else {
                     // queue the survivors for the Hi-Z test
                     const uint32_t pre_mask = __ballot_sync(0xFFFFFFFFu, pre);
@@ -713,7 +780,7 @@ __global__ void __launch_bounds__(kDwThreads, ORBIT_DIRECT_MIN_CTAS) meshlet_tes
             // load per record and never touches the dispatch buffer); survivors counted per chunk
             const uint32_t ent = __shfl_sync(0xFFFFFFFFu, my_word, (lane * 4u + 0u) & 31u);
             const uint32_t mof = __shfl_sync(0xFFFFFFFFu, my_word, (lane * 4u + 1u) & 31u);
-            if (lane < (uint32_t)R && rec0 + lane < nrec) p.draw_masks[rec0 + lane] = make_uint4(my_mask, ent, mof, p.cmd_side != nullptr ? 0u : 1u);
+            if (lane < (uint32_t)R && rec0 + lane < nrec) pt.draw_masks[rec0 + lane] = make_uint4(my_mask, ent, mof, pt.cmd_side != nullptr ? 0u : 1u);
             const uint32_t tile_total = __reduce_add_sync(0xFFFFFFFFu, __popc(my_mask));
             if (lane == 0u && tile_total != 0u) atomicAdd(chunk_counts + (rec0 >> chunk_shift), tile_total);   // a tile never straddles a chunk
             warp_total += tile_total;
@@ -730,6 +797,17 @@ __global__ void __launch_bounds__(kDwThreads, ORBIT_DIRECT_MIN_CTAS) meshlet_tes
     __syncthreads();
     ORBIT_TRACE_STAMP(p.scan.trace, 1, 4);
 #endif
+}
+
+template <int R, bool kPass2, int kProj>
+__global__ void __launch_bounds__(kDwThreads, ORBIT_DIRECT_MIN_CTAS) meshlet_test_direct_kernel(const __grid_constant__ MeshletCullParams p) {
+    meshlet_test_direct_body<R, kPass2, kProj, false>(&p, 1u);
+}
+
+// orbit_meshlet_cull_views: pass 0 over the concatenation of up to 16 views' record lists
+template <int R, int kProj>
+__global__ void __launch_bounds__(kDwThreads, ORBIT_DIRECT_MIN_CTAS) meshlet_test_views_kernel(const __grid_constant__ MeshletViewsParams pv) {
+    meshlet_test_direct_body<R, false, kProj, true>(pv.view, pv.n_views);
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -1296,6 +1374,8 @@ __global__ void __launch_bounds__(kEmitWarps * 32) meshlet_emit_kernel(const __g
 // look at blockIdx.x / gridDim.x): the LATE list of a steady frame is empty, and its emit kernel was 3 us of launch + look.
 struct EmitPair { MeshletCullParams list[2]; };
 __global__ void __launch_bounds__(kEmitWarps * 32) meshlet_emit_pair_kernel(const __grid_constant__ EmitPair pp) { meshlet_emit_body(pp.list[blockIdx.y]); }
+// The same for up to 16 lists (orbit_meshlet_cull_views): blockIdx.y = view.
+__global__ void __launch_bounds__(kEmitWarps * 32) meshlet_emit_views_kernel(const __grid_constant__ MeshletViewsParams pv) { meshlet_emit_body(pv.view[blockIdx.y]); }
 
 // ---------------------------------------------------------------------------------------------------------
 // Multi-GPU (SURVEY §8e, meshlet ranges of one view): a rank that only TESTS its records ships the 16-byte
@@ -1406,6 +1486,11 @@ cudaError_t meshlet_cull_configure_device() {
     if (e != cudaSuccess) return e;
     ORBIT_SET(false, 0) ORBIT_SET(false, 1) ORBIT_SET(false, -1) ORBIT_SET(true, 0) ORBIT_SET(true, 1) ORBIT_SET(true, -1)
 #undef ORBIT_SET
+#define ORBIT_SET(proj) \
+    e = cudaFuncSetAttribute(meshlet_test_views_kernel<kTileR, proj>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)direct_smem_bytes()); \
+    if (e != cudaSuccess) return e;
+    ORBIT_SET(0) ORBIT_SET(1) ORBIT_SET(-1)
+#undef ORBIT_SET
     return cudaSuccess;
 }
 
@@ -1454,6 +1539,34 @@ cudaError_t launch_meshlet_cull(const MeshletCullParams& p, int grid, int emit_g
     }
     if (emit_grid > 0) return launch_kernel(meshlet_emit_kernel, dim3(emit_grid), dim3(kEmitWarps * 32), 0, stream, p);
     return cudaSuccess;
+}
+
+template <int kProj>
+static cudaError_t launch_views_test(const MeshletViewsParams& pv, int grid, cudaStream_t stream, int* occupancy) {
+    if (occupancy) {
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(occupancy, meshlet_test_views_kernel<kTileR, kProj>, kDwThreads, direct_smem_bytes());
+        return cudaSuccess;
+    }
+    return launch_kernel(meshlet_test_views_kernel<kTileR, kProj>, dim3(grid), dim3(kDwThreads), direct_smem_bytes(), stream, pv);
+}
+
+static cudaError_t launch_views_test_any(const MeshletViewsParams& pv, uint32_t projection_type, int grid, cudaStream_t stream, int* occupancy) {
+    if (projection_type == 0u) return launch_views_test<0>(pv, grid, stream, occupancy);
+    if (projection_type == 1u) return launch_views_test<1>(pv, grid, stream, occupancy);
+    return launch_views_test<-1>(pv, grid, stream, occupancy);
+}
+
+int meshlet_cull_views_max_ctas_per_sm(uint32_t projection_type) {
+    int n = 0;
+    launch_views_test_any(MeshletViewsParams{}, projection_type, 0, nullptr, &n);
+    return n;
+}
+
+// test kernel over the concatenated lists (one persistent wave), then one emit launch with a row of emit_grid_per_view CTAs per view
+cudaError_t launch_meshlet_cull_views(const MeshletViewsParams& pv, int grid, int emit_grid_per_view, cudaStream_t stream) {
+    cudaError_t e = launch_views_test_any(pv, pv.view[0].cull.projection_type, grid, stream, nullptr);
+    if (e != cudaSuccess) return e;
+    return launch_kernel(meshlet_emit_views_kernel, dim3(emit_grid_per_view, pv.n_views), dim3(kEmitWarps * 32), 0, stream, pv);
 }
 
 int meshlet_emit_max_ctas_per_sm() {

@@ -74,6 +74,18 @@ struct EntityCullParams {
     ScanState scan;
 };
 
+// Batched pass-0 views of one scene (orbit_entity_cull_views / orbit_meshlet_cull_views): one full parameter block per view,
+// passed by value like the single-view blocks, so everything a replayed CUDA graph needs travels in the kernel parameters.
+struct EntityViewsParams {
+    EntityCullParams view[ORBIT_MAX_BATCH_VIEWS];   // scene fields and scan state are read from view[0]
+    uint32_t n_views;
+};
+struct MeshletViewsParams {
+    MeshletCullParams view[ORBIT_MAX_BATCH_VIEWS];  // scene fields are read from view[0]; per view: CullInfo, planes_t, buffers, scratch
+    uint32_t n_views;
+};
+static_assert(sizeof(EntityViewsParams) <= 32764 && sizeof(MeshletViewsParams) <= 32764, "kernel parameter space is 32 764 bytes");
+
 struct SceneUpdateParams {
     const uint8_t* transforms;           // OrbitTransform[], 48 B each
     const uint32_t* mesh_slots;
@@ -145,7 +157,11 @@ cudaError_t launch_meshlet_emit(const MeshletCullParams& p, int emit_grid, cudaS
 cudaError_t launch_meshlet_emit_pair(const MeshletCullParams& a, const MeshletCullParams& b, int emit_grid, cudaStream_t s);
 cudaError_t launch_draws_from_masks(const MeshletCullParams& p, uint32_t* header, int grid, int emit_grid, cudaStream_t s);
 cudaError_t launch_entity_cull(const EntityCullParams&, uint32_t n_draws, uint32_t coresident_ctas, cudaStream_t);
+cudaError_t launch_entity_cull_views(const EntityViewsParams&, uint32_t n_draws, uint32_t coresident_ctas, cudaStream_t);
+cudaError_t launch_meshlet_cull_views(const MeshletViewsParams&, int grid, int emit_grid_per_view, cudaStream_t);
+int meshlet_cull_views_max_ctas_per_sm(uint32_t projection_type);
 int entity_cull_max_ctas_per_sm();
+int entity_cull_views_max_ctas_per_sm();
 cudaError_t launch_hiz_build(const HizBuildParams&, cudaStream_t);
 cudaError_t launch_meshlet_bounds(const MeshletBoundsParams&, int grid, cudaStream_t);
 cudaError_t launch_mesh_bounds(const MeshBoundsParams&, int grid, cudaStream_t);

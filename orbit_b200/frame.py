@@ -118,6 +118,42 @@ def late_and_main_culling(context, dscene, vstate, view, meshlet_occlusion=True,
     return out
 
 
+def cull_views(context, dscene, cull_infos, name="views", task_payloads=None):
+    """Pass-0 culling of several views of one scene (the cascades of ShadowRenderer::render_cascaded_shadow,
+    shadow_renderer.rs:466-712, or many cameras) through orbit_entity_cull_views / orbit_meshlet_cull_views: 3 kernel launches
+    per group of up to MAX_BATCH_VIEWS views. Returns one (dispatch_buffer, draw_buffer) pair per CullInfo, byte for byte what
+    cull_pass returns for it. `task_payloads`: None, or one flag per view (a payload buffer is returned as a third element of
+    the views whose flag is set). Every view must be pass 0 with the same projection type."""
+    import ctypes as C
+    from . import _lib
+    from .passes import _scene_buffers, _stream
+    lib = _lib.lib()
+    sc = dscene.scene
+    rcap, dcap = int(sc.record_capacity) or 1_000_000, int(sc.draw_capacity) or 1_000_000
+    mk = context.create_transient
+    infos = list(cull_infos)
+    want = list(task_payloads) if task_payloads is not None else [False] * len(infos)
+    out = []
+    for g0 in range(0, len(infos), L.MAX_BATCH_VIEWS):
+        group = infos[g0:g0 + L.MAX_BATCH_VIEWS]
+        n = len(group)
+        gs = (L.CullInfo * n)(*[ci.to_gpu() for ci in group])
+        bufs = []
+        for v in range(g0, g0 + n):
+            tag = "%s%d" % (name, v)
+            pay = mk(tag + "_task_payloads", 44 * rcap) if want[v] else None
+            bufs.append((mk(tag + "_meshlet_dispatch_buffer", L.DISPATCH_HEADER + 16 * rcap),
+                         mk(tag + "_meshlet_draw_command_buffer", L.DRAW_HEADER + 28 * dcap), pay))
+        ptrs = lambda k: (C.c_void_p * n)(*[b[k].data_ptr() if b[k] is not None else None for b in bufs])
+        sb = _scene_buffers(dscene.assets, sc, group[0])
+        _lib.check(lib.orbit_entity_cull_views(context._h, gs, n, C.byref(sb), ptrs(0), rcap, _stream(context)), "orbit_entity_cull_views")
+        _lib.check(lib.orbit_meshlet_cull_views(context._h, gs, n, C.byref(sb), ptrs(0), rcap, ptrs(1), dcap,
+                                                ptrs(2) if any(b[2] is not None for b in bufs) else None, _stream(context)),
+                   "orbit_meshlet_cull_views")
+        out.extend((d, w) if p is None else (d, w, p) for d, w, p in bufs)
+    return out
+
+
 def shadow_pass_culling(context, dscene, view, name="shadow"):
     """One cascade (shadow_renderer.rs:693-707): pass 0, no occlusion."""
     return cull_pass(context, name, dscene, cull_info_for(view, OcclusionCullInfo("none")))

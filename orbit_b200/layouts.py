@@ -9,6 +9,7 @@ import ctypes as C
 import numpy as np
 
 MAX_CULL_PLANES = 12
+MAX_BATCH_VIEWS = 16          # ORBIT_MAX_BATCH_VIEWS: views per orbit_entity_cull_views / orbit_meshlet_cull_views call
 MESHLET_DISPATCH_SIZE = 32
 MAX_MESH_LODS = 8
 NO_BUFFER = 0xFFFFFFFF

@@ -7,6 +7,8 @@
 use std::ffi::c_void;
 
 pub const ORBIT_OK: i32 = 0;
+pub const ORBIT_ERR_INVALID_ARGUMENT: i32 = -1;
+pub const ORBIT_MAX_BATCH_VIEWS: u32 = 16;
 pub const ORBIT_NO_BUFFER: u32 = 0xFFFF_FFFF;
 pub const ORBIT_HIZ_MAX_LEVELS: usize = 16;
 
@@ -145,6 +147,11 @@ extern "C" {
                                         hiz: *const orbit_hiz, late_dispatch_buffer: *const c_void, capacity_records: u64,
                                         late_draw_command_buffer: *mut c_void, main_draw_command_buffer: *mut c_void, capacity_draws: u64,
                                         late_task_payloads: *mut c_void, main_task_payloads: *mut c_void, stream: *mut c_void) -> c_int;
+    pub fn orbit_entity_cull_views(ctx: *mut orbit_ctx, culls: *const OrbitCullInfo, n_views: u32, scene: *const OrbitSceneBuffers,
+                                   dispatch_buffers: *const *mut c_void, capacity_records: u64, stream: *mut c_void) -> c_int;
+    pub fn orbit_meshlet_cull_views(ctx: *mut orbit_ctx, culls: *const OrbitCullInfo, n_views: u32, scene: *const OrbitSceneBuffers,
+                                    dispatch_buffers: *const *const c_void, capacity_records: u64, draw_command_buffers: *const *mut c_void,
+                                    capacity_draws: u64, task_payloads: *const *mut c_void, stream: *mut c_void) -> c_int;
     pub fn orbit_draws_scatter_ranked(ctx: *mut orbit_ctx, src_draw_buffer: *const c_void, src_capacity_draws: u64, dst_draw_buffer: *mut c_void,
                                       rank_counts: *const u32, rank: u32, world: u32, dst_capacity_draws: u64, stream: *mut c_void) -> i32;
     pub fn orbit_meshlet_test(ctx: *mut orbit_ctx, cull: *const OrbitCullInfo, scene: *const OrbitSceneBuffers, hiz: *const orbit_hiz,
@@ -200,6 +207,20 @@ impl Context {
         check(orbit_meshlet_cull_late_main(self.0, late, main_pass, scene, hiz, late_dispatch_buffer, capacity_records, late_draw_command_buffer,
                                            main_draw_command_buffer, capacity_draws, std::ptr::null_mut(), std::ptr::null_mut(), stream))?;
         Ok(true)
+    }
+    /// Pass-0 culling of up to ORBIT_MAX_BATCH_VIEWS views of one scene (the cascades of render_cascaded_shadow,
+    /// shadow_renderer.rs:466-712): buffer v receives what create_meshlet_dispatch_command / create_meshlet_draw_commands
+    /// write for `culls[v]`, from 3 kernel launches in all. The three slices have one entry per view.
+    pub unsafe fn create_views_commands(&self, culls: &[OrbitCullInfo], scene: &OrbitSceneBuffers, dispatch_buffers: &[*mut c_void],
+                                        capacity_records: u64, draw_command_buffers: &[*mut c_void], capacity_draws: u64,
+                                        stream: *mut c_void) -> Result<(), Error> {
+        if culls.len() > ORBIT_MAX_BATCH_VIEWS as usize || dispatch_buffers.len() != culls.len() || draw_command_buffers.len() != culls.len() {
+            return Err(Error(ORBIT_ERR_INVALID_ARGUMENT));
+        }
+        let n = culls.len() as u32;
+        check(orbit_entity_cull_views(self.0, culls.as_ptr(), n, scene, dispatch_buffers.as_ptr(), capacity_records, stream))?;
+        check(orbit_meshlet_cull_views(self.0, culls.as_ptr(), n, scene, dispatch_buffers.as_ptr() as *const *const c_void, capacity_records,
+                                       draw_command_buffers.as_ptr(), capacity_draws, std::ptr::null(), stream))
     }
 }
 impl Drop for Context { fn drop(&mut self) { unsafe { orbit_ctx_destroy(self.0) } } }
