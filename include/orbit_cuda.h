@@ -219,6 +219,47 @@ int orbit_meshlet_cull_views(orbit_ctx* ctx, const OrbitCullInfo* culls, uint32_
                              const void* const* dispatch_buffers, uint64_t capacity_records, void* const* draw_command_buffers,
                              uint64_t capacity_draws, void* const* task_payloads /* NULL, or entries may be NULL */, void* stream);
 
+/* ---- batched two-pass occlusion views (split-screen, stereo, probe cameras: several cameras with EARLY -> Hi-Z -> LATE -> MAIN
+ *      over one scene, forward.rs:213-548 per camera) ------------------------------------------------------------------------
+ * orbit_hiz_build_views: DepthPyramid::update for n_views (1..ORBIT_MAX_BATCH_VIEWS) pyramids of the same geometry in ONE launch
+ * (the reference's update_multiple_depth_pyramids, draw_gen.rs). Pyramid v is byte for byte what
+ * orbit_hiz_build(ctx, hizs[v], depths[v], depth_width, depth_height) writes. Refused (ORBIT_ERR_INVALID_ARGUMENT, nothing
+ * launched): n_views 0 or above the maximum, a NULL pyramid or depth buffer, a pyramid not created for depth_width x
+ * depth_height, two pyramids on the same texels. Counts as an orbit_hiz_build call; needs no scratch of its own.
+ *
+ * orbit_entity_cull_views_occlusion / orbit_meshlet_cull_views_occlusion: two-pass occlusion culling of n_views cameras over
+ * ONE scene, 3 kernel launches per call pair whatever n_views is. View v's outputs are byte for byte what
+ *   orbit_entity_cull(&culls[v], &scenes[v], hizs ? hizs[v] : NULL, ...) ; orbit_meshlet_cull(&culls[v], &scenes[v], ...)
+ * write: dispatch header and records, draw count and commands, task payloads, and (pass 2) the view's entity and meshlet
+ * visibility words. A frame of N cameras is EARLY (pass 1), orbit_hiz_build_views, LATE (pass 2), MAIN (pass 1): 10 launches.
+ *   - views: n_views is 1..ORBIT_MAX_BATCH_VIEWS;
+ *   - same pass: every view has the same occlusion_pass, and it is 1 or 2 (pass 0 is orbit_*_cull_views);
+ *   - same projection: every view has the same projection_type;
+ *   - same meshlet-occlusion setting: either every view has a meshlet visibility buffer (meshlet_visibility_buffer !=
+ *     ORBIT_NO_BUFFER) or none does;
+ *   - one scene: scenes[v] equals scenes[0] in every field except entity_visibility and meshlet_visibility (draw_begin /
+ *     draw_end included);
+ *   - no shared buffers: no two views share a visibility buffer (the entity call: entity_visibility; the meshlet call with
+ *     meshlet occlusion: meshlet_visibility), a dispatch buffer, a draw buffer or a task payload buffer;
+ *   - pyramids: hizs is required for pass 2 and ignored for pass 1; it holds one distinct pyramid per view, all of the same
+ *     geometry;
+ *   - everything orbit_entity_cull / orbit_meshlet_cull refuse for one view is refused here too;
+ *   every refusal returns ORBIT_ERR_INVALID_ARGUMENT with nothing launched.
+ *   - overflow, status flags and CUDA-graph replay follow the single-view rules;
+ *   - concurrency: the entity call counts as an orbit_entity_cull call and the meshlet call as an orbit_meshlet_cull call;
+ *   - scratch: as orbit_meshlet_cull_views (n_views x capacity_records records; the batched survivor counters are allocated
+ *     by the first batched meshlet call of either form: make one before capturing batched calls into a CUDA graph). */
+int orbit_hiz_build_views(orbit_ctx* ctx, orbit_hiz* const* hizs, const float* const* depths, uint32_t n_views,
+                          uint32_t depth_width, uint32_t depth_height, void* stream);
+int orbit_entity_cull_views_occlusion(orbit_ctx* ctx, const OrbitCullInfo* culls, uint32_t n_views,
+                                      const OrbitSceneBuffers* scenes, const orbit_hiz* const* hizs,
+                                      void* const* dispatch_buffers, uint64_t capacity_records, void* stream);
+int orbit_meshlet_cull_views_occlusion(orbit_ctx* ctx, const OrbitCullInfo* culls, uint32_t n_views,
+                                       const OrbitSceneBuffers* scenes, const orbit_hiz* const* hizs,
+                                       const void* const* dispatch_buffers, uint64_t capacity_records,
+                                       void* const* draw_command_buffers, uint64_t capacity_draws,
+                                       void* const* task_payloads /* NULL, or entries NULL */, void* stream);
+
 /* ---- compute_clusters (cluster.rs:368-591) + light_cluster/{mark_active,active_cluster_compaction,
  *      light_culling}.comp --------------------------------------------------------------------------------- */
 /* tile_masks: u32[cx*cy]; depth_bounds: OrbitClusterDepthBounds[cx*cy*cz]; unique_clusters:

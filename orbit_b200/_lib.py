@@ -48,6 +48,13 @@ PROTOTYPES = {
                                           C.c_uint64, C.c_void_p]),
     "orbit_meshlet_cull_views": (C.c_int, [C.c_void_p, C.POINTER(L.CullInfo), C.c_uint32, C.POINTER(L.SceneBuffers), C.POINTER(C.c_void_p),
                                            C.c_uint64, C.POINTER(C.c_void_p), C.c_uint64, C.POINTER(C.c_void_p), C.c_void_p]),
+    "orbit_hiz_build_views": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_uint32, C.c_uint32, C.c_uint32,
+                                        C.c_void_p]),
+    "orbit_entity_cull_views_occlusion": (C.c_int, [C.c_void_p, C.POINTER(L.CullInfo), C.c_uint32, C.POINTER(L.SceneBuffers),
+                                                    C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_uint64, C.c_void_p]),
+    "orbit_meshlet_cull_views_occlusion": (C.c_int, [C.c_void_p, C.POINTER(L.CullInfo), C.c_uint32, C.POINTER(L.SceneBuffers),
+                                                     C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_uint64, C.POINTER(C.c_void_p),
+                                                     C.c_uint64, C.POINTER(C.c_void_p), C.c_void_p]),
     "orbit_meshlet_test": (C.c_int, [C.c_void_p, C.POINTER(L.CullInfo), C.POINTER(L.SceneBuffers), C.c_void_p, C.c_void_p, C.c_uint64,
                                      C.c_void_p, C.c_void_p]),
     "orbit_record_masks_put": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p]),

@@ -84,10 +84,11 @@ struct orbit_ctx {
     int emit_occupancy = 0;
     int debug_skip = 0;               // ORBIT_DEBUG_SKIP: 1 = skip emit kernel, 2 = skip test kernel (timing experiments only)
     int entity_occupancy = 0;
-    int entity_views_occupancy = 0;   // the same for the batched entity kernel (more registers: fewer CTAs per SM)
+    int entity_views_occupancy[3] = {0, 0, 0};        // the same for the batched entity kernel, per pass (more registers: fewer CTAs per SM)
     int mc_occupancy[8] = {0, 0, 0, 0, 0, 0, 0, 0};   // cached occupancy per meshlet test-kernel variant
-    int views_occupancy[3] = {0, 0, 0};                // the same for the batched test kernel, per projection (0, 1, other)
+    int views_occupancy[8] = {0, 0, 0, 0, 0, 0, 0, 0}; // the same for the batched test kernels, per variant
     int emit_ctas_per_sm = 0;         // ORBIT_EMIT_CTAS_PER_SM (tuning knob, read once at creation)
+    bool views_pass2_configured = false;   // meshlet_cull_configure_views_pass2 done (first batched pass-2 call with meshlet occlusion)
     // Scratch that was outgrown is parked here until the context is destroyed: freeing it would need a device
     // synchronisation (work that uses it may still be in flight), and a stage call never synchronises.
     void* retired[64] = {};
@@ -397,6 +398,33 @@ int orbit_hiz_build(orbit_ctx* c, orbit_hiz* h, const float* depth, uint32_t dw,
     return ORBIT_OK;
 }
 
+// Batched form: one launch, a row of CTAs per pyramid. Pyramid v's ticket is counter word 40 + v (words 40..55 are used by
+// nothing else and were zeroed with the rest at context creation; each row's last CTA re-zeroes its own).
+int orbit_hiz_build_views(orbit_ctx* c, orbit_hiz* const* hizs, const float* const* depths, uint32_t n_views, uint32_t dw, uint32_t dh,
+                          void* stream) {
+    if (!c || !hizs || !depths || n_views == 0u || n_views > ORBIT_MAX_BATCH_VIEWS) return ORBIT_ERR_INVALID_ARGUMENT;
+    for (uint32_t v = 0; v < n_views; ++v) {
+        const orbit_hiz* h = hizs[v];
+        if (!h || !depths[v] || dw != h->depth_w || dh != h->depth_h) return ORBIT_ERR_INVALID_ARGUMENT;
+        for (uint32_t u = 0; u < v; ++u) if (hizs[u]->info.texels == h->info.texels) return ORBIT_ERR_INVALID_ARGUMENT;
+    }
+    GUARD(c);
+    HizBuildViewsParams pv{};
+    pv.n_views = n_views;
+    for (uint32_t v = 0; v < n_views; ++v) {
+        const orbit_hiz* h = hizs[v];
+        HizBuildParams& p = pv.view[v];
+        p.depth = depths[v]; p.texels = h->info.texels; p.depth_w = dw; p.depth_h = dh;
+        p.width = h->info.width; p.height = h->info.height; p.levels = h->info.levels;
+        for (int i = 0; i < ORBIT_HIZ_MAX_LEVELS; ++i) p.level_offset[i] = h->info.level_offset[i];
+        p.ticket = c->counters + 40 + v;
+    }
+    pv.view[0].trace = next_trace(c);
+    CK(launch_hiz_build_views(pv, (cudaStream_t)stream));
+    c->launches += 1;
+    return ORBIT_OK;
+}
+
 // ---- entity stage ----------------------------------------------------------------------------------------
 static int check_cull(const OrbitCullInfo* cull, const OrbitSceneBuffers* scene, const orbit_hiz* hiz, bool meshlet_stage) {
     if (!cull || !scene) return ORBIT_ERR_INVALID_ARGUMENT;
@@ -447,9 +475,10 @@ static uint32_t entity_coresident_ctas(orbit_ctx* c) {
     return (uint32_t)(c->sm_count * (c->entity_occupancy > 0 ? c->entity_occupancy : 1));
 }
 
-static uint32_t entity_views_coresident_ctas(orbit_ctx* c) {
-    if (c->entity_views_occupancy <= 0) c->entity_views_occupancy = entity_cull_views_max_ctas_per_sm();
-    return (uint32_t)(c->sm_count * (c->entity_views_occupancy > 0 ? c->entity_views_occupancy : 1));
+static uint32_t entity_views_coresident_ctas(orbit_ctx* c, uint32_t pass) {
+    int& occ = c->entity_views_occupancy[pass];
+    if (occ <= 0) occ = entity_cull_views_max_ctas_per_sm(pass);
+    return (uint32_t)(c->sm_count * (occ > 0 ? occ : 1));
 }
 
 static int entity_stage(orbit_ctx* c, const OrbitCullInfo* cull, const OrbitSceneBuffers* scene, const orbit_hiz* hiz,
@@ -697,6 +726,16 @@ int orbit_draws_from_masks(orbit_ctx* c, const OrbitSceneBuffers* scene, const v
 }
 
 // ---- batched pass-0 views ---------------------------------------------------------------------------------
+// one output buffer per view: present, 4-byte aligned, none shared with another view
+static int check_view_buffers(const void* const* buffers, uint32_t n_views) {
+    if (!buffers) return ORBIT_ERR_INVALID_ARGUMENT;
+    for (uint32_t v = 0; v < n_views; ++v) {
+        if (!buffers[v] || ((uintptr_t)buffers[v] & 3u)) return ORBIT_ERR_INVALID_ARGUMENT;
+        for (uint32_t u = 0; u < v; ++u) if (buffers[u] == buffers[v]) return ORBIT_ERR_INVALID_ARGUMENT;
+    }
+    return ORBIT_OK;
+}
+
 // Checks shared by both stages: the view count, every view's CullInfo (pass 0, one projection type, check_cull), and one
 // output buffer per view — present, 4-byte aligned, none shared with another view.
 static int check_views(const OrbitCullInfo* culls, uint32_t n_views, const OrbitSceneBuffers* scene, const void* const* buffers,
@@ -706,10 +745,8 @@ static int check_views(const OrbitCullInfo* culls, uint32_t n_views, const Orbit
         int rc = check_cull(&culls[v], scene, nullptr, meshlet_stage);
         if (rc != ORBIT_OK) return rc;
         if (culls[v].occlusion_pass != 0u || culls[v].projection_type != culls[0].projection_type) return ORBIT_ERR_INVALID_ARGUMENT;
-        if (!buffers[v] || ((uintptr_t)buffers[v] & 3u)) return ORBIT_ERR_INVALID_ARGUMENT;
-        for (uint32_t u = 0; u < v; ++u) if (buffers[u] == buffers[v]) return ORBIT_ERR_INVALID_ARGUMENT;
     }
-    return ORBIT_OK;
+    return check_view_buffers(buffers, n_views);
 }
 
 int orbit_entity_cull_views(orbit_ctx* c, const OrbitCullInfo* culls, uint32_t n_views, const OrbitSceneBuffers* scene,
@@ -728,17 +765,17 @@ int orbit_entity_cull_views(orbit_ctx* c, const OrbitCullInfo* culls, uint32_t n
     pv.n_views = n_views;
     for (uint32_t v = 0; v < n_views; ++v) pv.view[v] = entity_params(c, &culls[v], scene, nullptr, dispatch_buffers[v], capacity_records, begin, end);
     pv.view[0].scan = next_scan(c);
-    CK(launch_entity_cull_views(pv, n, entity_views_coresident_ctas(c), (cudaStream_t)stream));
+    CK(launch_entity_cull_views(pv, n, entity_views_coresident_ctas(c, 0u), (cudaStream_t)stream));
     c->launches += 1;
     return ORBIT_OK;
 }
 
-int orbit_meshlet_cull_views(orbit_ctx* c, const OrbitCullInfo* culls, uint32_t n_views, const OrbitSceneBuffers* scene,
-                             const void* const* dispatch_buffers, uint64_t capacity_records, void* const* draw_command_buffers,
-                             uint64_t capacity_draws, void* const* task_payloads, void* stream) {
-    if (!c) return ORBIT_ERR_INVALID_ARGUMENT;
-    int rc = check_views(culls, n_views, scene, dispatch_buffers, true);
-    if (rc == ORBIT_OK) rc = check_views(culls, n_views, scene, (const void* const*)draw_command_buffers, true);
+// The meshlet stage of both batched forms, after their own checks: view v reads scenes[v] (per_view_scene) or scenes[0], and
+// the pyramid hizs[v] (pass 2 with meshlet occlusion; NULL otherwise).
+static int meshlet_views_stage(orbit_ctx* c, const OrbitCullInfo* culls, uint32_t n_views, const OrbitSceneBuffers* scenes, bool per_view_scene,
+                               const orbit_hiz* const* hizs, const void* const* dispatch_buffers, uint64_t capacity_records,
+                               void* const* draw_command_buffers, uint64_t capacity_draws, void* const* task_payloads, void* stream) {
+    int rc = check_view_buffers((const void* const*)draw_command_buffers, n_views);
     if (rc != ORBIT_OK) return rc;
     for (uint32_t v = 0; task_payloads && v < n_views; ++v) {
         if ((uintptr_t)task_payloads[v] & 3u) return ORBIT_ERR_INVALID_ARGUMENT;
@@ -746,6 +783,10 @@ int orbit_meshlet_cull_views(orbit_ctx* c, const OrbitCullInfo* culls, uint32_t 
     }
     if (capacity_records > 0xFFFFFFFFull) capacity_records = 0xFFFFFFFFull;
     GUARD(c);
+    if (hizs && !c->views_pass2_configured) {   // the batched pass-2 test kernels' shared-memory opt-in, on first use
+        CK(meshlet_cull_configure_views_pass2());
+        c->views_pass2_configured = true;
+    }
     // draw masks + side words of view v live at records [v * capacity_records, (v + 1) * capacity_records) of the grown scratch
     rc = ensure_record_scratch(c, (uint64_t)n_views * capacity_records);
     if (rc != ORBIT_OK) return rc;
@@ -766,7 +807,9 @@ int orbit_meshlet_cull_views(orbit_ctx* c, const OrbitCullInfo* culls, uint32_t 
     pv.n_views = n_views;
     for (uint32_t v = 0; v < n_views; ++v) {
         MeshletCullParams& p = pv.view[v];
+        const OrbitSceneBuffers* scene = per_view_scene ? &scenes[v] : scenes;
         set_cull(p, &culls[v]);
+        p.hiz = hiz_device(hizs ? hizs[v] : nullptr);
         p.dispatch_words = (const uint32_t*)dispatch_buffers[v];
         p.meshlets = (const uint4*)scene->meshlets;
         p.entities = (const float4*)scene->entities;
@@ -786,14 +829,91 @@ int orbit_meshlet_cull_views(orbit_ctx* c, const OrbitCullInfo* culls, uint32_t 
     }
     pv.view[0].scan.trace = next_trace(c);
     pv.view[0].trace_emit = next_trace(c);
-    const uint32_t proj = culls[0].projection_type;
-    int& occ_slot = c->views_occupancy[proj <= 1u ? proj : 2u];
-    if (occ_slot <= 0) occ_slot = meshlet_cull_views_max_ctas_per_sm(proj);
+    int& occ_slot = c->views_occupancy[meshlet_cull_variant_index(culls[0])];
+    if (occ_slot <= 0) occ_slot = meshlet_cull_views_max_ctas_per_sm(culls[0]);
     int per_sm = c->mc_ctas_per_sm;
     if (per_sm <= 0) per_sm = occ_slot > 0 ? occ_slot : 1;
     CK(launch_meshlet_cull_views(pv, c->sm_count * per_sm, (int)emit_per_view, (cudaStream_t)stream));
     c->launches += 2;
     return ORBIT_OK;
+}
+
+int orbit_meshlet_cull_views(orbit_ctx* c, const OrbitCullInfo* culls, uint32_t n_views, const OrbitSceneBuffers* scene,
+                             const void* const* dispatch_buffers, uint64_t capacity_records, void* const* draw_command_buffers,
+                             uint64_t capacity_draws, void* const* task_payloads, void* stream) {
+    if (!c) return ORBIT_ERR_INVALID_ARGUMENT;
+    int rc = check_views(culls, n_views, scene, dispatch_buffers, true);
+    if (rc != ORBIT_OK) return rc;
+    return meshlet_views_stage(c, culls, n_views, scene, false, nullptr, dispatch_buffers, capacity_records, draw_command_buffers,
+                               capacity_draws, task_payloads, stream);
+}
+
+// ---- batched two-pass occlusion views ----------------------------------------------------------------------
+// Checks shared by both stages: view count; one pass (1 or 2), one projection type and one meshlet-occlusion setting for all
+// views; check_cull per view; scenes[v] equal to scenes[0] except for the two visibility pointers, which no two views share (the
+// entity stage's entity bits, the meshlet stage's meshlet words when meshlet occlusion is on); pass 2: one distinct pyramid per
+// view, all of one geometry; one distinct, aligned output buffer per view.
+static int check_views_occlusion(const OrbitCullInfo* culls, uint32_t n_views, const OrbitSceneBuffers* scenes, const orbit_hiz* const* hizs,
+                                 const void* const* buffers, bool meshlet_stage) {
+    if (!culls || !scenes || n_views == 0u || n_views > ORBIT_MAX_BATCH_VIEWS) return ORBIT_ERR_INVALID_ARGUMENT;
+    const uint32_t pass = culls[0].occlusion_pass;
+    const bool mocc = culls[0].meshlet_visibility_buffer != ORBIT_NO_BUFFER;
+    if (pass != 1u && pass != 2u) return ORBIT_ERR_INVALID_ARGUMENT;
+    if (pass == 2u && !hizs) return ORBIT_ERR_INVALID_ARGUMENT;
+    for (uint32_t v = 0; v < n_views; ++v) {
+        const OrbitCullInfo& ci = culls[v];
+        if (ci.occlusion_pass != pass || ci.projection_type != culls[0].projection_type) return ORBIT_ERR_INVALID_ARGUMENT;
+        if ((ci.meshlet_visibility_buffer != ORBIT_NO_BUFFER) != mocc) return ORBIT_ERR_INVALID_ARGUMENT;
+        const orbit_hiz* h = pass == 2u ? hizs[v] : nullptr;
+        if (pass == 2u) {
+            if (!h || h->info.width != hizs[0]->info.width || h->info.height != hizs[0]->info.height || h->info.levels != hizs[0]->info.levels)
+                return ORBIT_ERR_INVALID_ARGUMENT;
+            for (uint32_t u = 0; u < v; ++u) if (hizs[u]->info.texels == h->info.texels) return ORBIT_ERR_INVALID_ARGUMENT;
+        }
+        int rc = check_cull(&ci, &scenes[v], h, meshlet_stage);
+        if (rc != ORBIT_OK) return rc;
+        OrbitSceneBuffers same = scenes[v];
+        same.entity_visibility = scenes[0].entity_visibility; same.meshlet_visibility = scenes[0].meshlet_visibility;
+        if (std::memcmp(&same, &scenes[0], sizeof(same)) != 0) return ORBIT_ERR_INVALID_ARGUMENT;
+        for (uint32_t u = 0; u < v; ++u) {
+            if (!meshlet_stage && scenes[u].entity_visibility == scenes[v].entity_visibility) return ORBIT_ERR_INVALID_ARGUMENT;
+            if (meshlet_stage && mocc && scenes[u].meshlet_visibility == scenes[v].meshlet_visibility) return ORBIT_ERR_INVALID_ARGUMENT;
+        }
+    }
+    return check_view_buffers(buffers, n_views);
+}
+
+int orbit_entity_cull_views_occlusion(orbit_ctx* c, const OrbitCullInfo* culls, uint32_t n_views, const OrbitSceneBuffers* scenes,
+                                      const orbit_hiz* const* hizs, void* const* dispatch_buffers, uint64_t capacity_records, void* stream) {
+    if (!c) return ORBIT_ERR_INVALID_ARGUMENT;
+    int rc = check_views_occlusion(culls, n_views, scenes, hizs, (const void* const*)dispatch_buffers, false);
+    if (rc != ORBIT_OK) return rc;
+    uint32_t begin, end;
+    rc = draw_range(&scenes[0], &begin, &end);
+    if (rc != ORBIT_OK) return rc;
+    const uint32_t n = end - begin, pass = culls[0].occlusion_pass;
+    GUARD(c);
+    rc = ensure_status(c, (size_t)n_views * ((n + 255u) / 256u + 1u), (cudaStream_t)stream);   // one descriptor block per view
+    if (rc != ORBIT_OK) return rc;
+    EntityViewsParams pv{};
+    pv.n_views = n_views;
+    for (uint32_t v = 0; v < n_views; ++v)
+        pv.view[v] = entity_params(c, &culls[v], &scenes[v], pass == 2u ? hizs[v] : nullptr, dispatch_buffers[v], capacity_records, begin, end);
+    pv.view[0].scan = next_scan(c);
+    CK(launch_entity_cull_views(pv, n, entity_views_coresident_ctas(c, pass), (cudaStream_t)stream));
+    c->launches += 1;
+    return ORBIT_OK;
+}
+
+int orbit_meshlet_cull_views_occlusion(orbit_ctx* c, const OrbitCullInfo* culls, uint32_t n_views, const OrbitSceneBuffers* scenes,
+                                       const orbit_hiz* const* hizs, const void* const* dispatch_buffers, uint64_t capacity_records,
+                                       void* const* draw_command_buffers, uint64_t capacity_draws, void* const* task_payloads, void* stream) {
+    if (!c) return ORBIT_ERR_INVALID_ARGUMENT;
+    int rc = check_views_occlusion(culls, n_views, scenes, hizs, dispatch_buffers, true);
+    if (rc != ORBIT_OK) return rc;
+    const bool with_hiz = culls[0].occlusion_pass == 2u && culls[0].meshlet_visibility_buffer != ORBIT_NO_BUFFER;
+    return meshlet_views_stage(c, culls, n_views, scenes, true, with_hiz ? hizs : nullptr, dispatch_buffers, capacity_records,
+                               draw_command_buffers, capacity_draws, task_payloads, stream);
 }
 
 // ---- clustered lights ------------------------------------------------------------------------------------

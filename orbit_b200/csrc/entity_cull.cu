@@ -210,14 +210,15 @@ __global__ void __launch_bounds__(kEcThreads) entity_cull_kernel(const __grid_co
     ORBIT_TRACE_STAMP(p.scan.trace, 0, 7);
 }
 
-// orbit_entity_cull_views: entity_cull_kernel for views[0..n_views), pass-0 views of one scene, in one launch (pass 0 only: no
-// visibility words, no Hi-Z, no mirror buffer — the host refuses other passes). It is a kernel of its own rather than a template
-// parameter of entity_cull_kernel because the single-view kernel's SASS must stay as it is, and every folded form tried reordered
-// it. The scene fields (draw words, mesh infos, entities, draw range, scan state) are read from views[0]. Tickets are handed out
+// orbit_entity_cull_views (kPass 0) and orbit_entity_cull_views_occlusion (kPass 1, 2): entity_cull_kernel for views[0..n_views)
+// of one scene, in one launch (no mirror buffer). kPass 1 reads each view's entity visibility bit, kPass 2 runs the Hi-Z test
+// against each view's pyramid and writes each view's visibility words; every view of a launch has that pass (the host refuses
+// mixed passes). It is a kernel of its own rather than a template parameter of entity_cull_kernel because the single-view
+// kernel's SASS must stay as it is, and every folded form tried reordered it. The scene fields (draw words, mesh infos, entities, draw range, scan state) are read from views[0]. Tickets are handed out
 // tile-major, view-minor: ticket t covers draw tile t / n_views for view t % n_views, so the lower draw tiles of a view always
 // hold lower tickets and the waits below keep their no-deadlock argument. The scan descriptors of view v are the block
 // [v * draw tiles, (v + 1) * draw tiles): each view's prefix (flat gather or look-back) sees only its own tiles.
-template <bool kFlat>
+template <bool kFlat, int kPass>
 __global__ void __launch_bounds__(kEcThreads) entity_cull_views_kernel(const __grid_constant__ EntityViewsParams params) {
     const EntityCullParams* const views = params.view;
     __shared__ uint4 s_recs[kEcBatch];            // the tile's records, staged for coalesced stores
@@ -276,6 +277,7 @@ __global__ void __launch_bounds__(kEcThreads) entity_cull_views_kernel(const __g
     ORBIT_TRACE_STAMP(p0.scan.trace, 0, 1 + 0 * (count + epoch));
 
     uint32_t chunks = 0u, lod_off = 0u, lod_cnt = 0u;
+    bool visible = false;                                        // kPass 2: this view's new visibility bit of the draw
     const bool in_range = gid < count;
     if (in_range) {
         // every load that depends only on the draw words, issued back to back (ordered loads, orbit_device.cuh): what
@@ -285,10 +287,13 @@ __global__ void __launch_bounds__(kEcThreads) entity_cull_views_kernel(const __g
 #pragma unroll
         for (int k = 0; k < 4; ++k) lods[k] = ld_v4_ordered(mi + 64 + 16 * k);
         const uint4 mi_hdr = ld_v4_ordered(mi + 48);                              // vertex_offset, data_offset, lod_count, pad
+        uint32_t vword = 0xFFFFFFFFu;
+        if constexpr (kPass != 0) vword = ld_u32_ordered(p.entity_visibility + (gid >> 5));
         const float4 sph = as_float4(ld_v4_ordered(mi));
         float4 mcol[4];
 #pragma unroll
         for (int k = 0; k < 4; ++k) mcol[k] = as_float4(ld_v4_ordered(p.entities + (size_t)entity_index * 8u + k));
+        const bool vib = ((vword >> (gid & 31u)) & 1u) != 0u;
         ORBIT_TRACE_STAMP(p.scan.trace, 0, 2 + 0 * (uint32_t)(mcol[3].w != 0.0f) + 0 * (lods[0].x & sph.x != 0.0f));
 
         // view * model (entity_cull.comp:131-133)
@@ -303,7 +308,17 @@ __global__ void __launch_bounds__(kEcThreads) entity_cull_views_kernel(const __g
         }
         mv.scale = largest_scale(mv.m);
         Sphere s = transform_sphere(mv, sph.x, sph.y, sph.z, sph.w);
-        if (frustum_test(ci, s)) {                                   // pass 0: should_draw = visible (entity_cull.comp:137-189)
+        bool should_draw;                                            // entity_cull.comp:137-189, as in entity_cull_kernel
+        if constexpr (kPass == 0) {
+            should_draw = frustum_test(ci, s);                       // pass 0: should_draw = visible
+        } else {
+            const bool mocc = ci.meshlet_visibility_buffer != ORBIT_NO_BUFFER;
+            visible = (kPass == 1) ? vib : true;
+            if (visible) visible = frustum_test(ci, s);
+            if (kPass == 2 && visible) visible = occlusion_test(ci, s, p.hiz);
+            should_draw = (kPass == 2) ? visible && (!vib || mocc) : visible;
+        }
+        if (should_draw) {
             const float dx = sub(ci.lod_target_pos_view_space[0], s.x);
             const float dy = sub(ci.lod_target_pos_view_space[1], s.y);
             const float dz = sub(ci.lod_target_pos_view_space[2], s.z);
@@ -322,6 +337,10 @@ __global__ void __launch_bounds__(kEcThreads) entity_cull_views_kernel(const __g
             chunks = (L.y + 31u) >> 5;
             lod_off = L.x; lod_cnt = L.y;
         }
+    }
+    if constexpr (kPass == 2) {   // this view's visibility word of these 32 draws (lanes past `count` contribute 0)
+        const uint32_t vis_mask = __ballot_sync(0xFFFFFFFFu, visible);
+        if (lane == 0u && gid < count) p.entity_visibility[gid >> 5] = vis_mask;
     }
 
     // ---- CTA exclusive scan of chunk counts
@@ -398,12 +417,21 @@ cudaError_t launch_entity_cull(const EntityCullParams& p, uint32_t n_draws, uint
     return launch_kernel(entity_cull_kernel<false>, dim3(grid), dim3(kEcThreads), 0, stream, p);
 }
 
+template <int kPass>
+static cudaError_t launch_entity_views_pass(const EntityViewsParams& pv, uint32_t grid, uint32_t coresident_ctas, cudaStream_t stream) {
+    if (grid <= coresident_ctas) return launch_kernel(entity_cull_views_kernel<true, kPass>, dim3(grid), dim3(kEcThreads), 0, stream, pv);
+    return launch_kernel(entity_cull_views_kernel<false, kPass>, dim3(grid), dim3(kEcThreads), 0, stream, pv);
+}
+
+// coresident_ctas: from entity_cull_views_max_ctas_per_sm of the same pass
 cudaError_t launch_entity_cull_views(const EntityViewsParams& pv, uint32_t n_draws, uint32_t coresident_ctas, cudaStream_t stream) {
     uint32_t tiles = (n_draws + kEcThreads - 1) / kEcThreads;
     if (tiles == 0) tiles = 1;
     const uint32_t grid = tiles * pv.n_views;
-    if (grid <= coresident_ctas) return launch_kernel(entity_cull_views_kernel<true>, dim3(grid), dim3(kEcThreads), 0, stream, pv);
-    return launch_kernel(entity_cull_views_kernel<false>, dim3(grid), dim3(kEcThreads), 0, stream, pv);
+    const uint32_t pass = pv.view[0].cull.occlusion_pass;
+    if (pass == 1u) return launch_entity_views_pass<1>(pv, grid, coresident_ctas, stream);
+    if (pass == 2u) return launch_entity_views_pass<2>(pv, grid, coresident_ctas, stream);
+    return launch_entity_views_pass<0>(pv, grid, coresident_ctas, stream);
 }
 
 int entity_cull_max_ctas_per_sm() {
@@ -412,9 +440,11 @@ int entity_cull_max_ctas_per_sm() {
     return n;
 }
 
-int entity_cull_views_max_ctas_per_sm() {
+int entity_cull_views_max_ctas_per_sm(uint32_t occlusion_pass) {
     int n = 0;
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, entity_cull_views_kernel<true>, kEcThreads, 0);
+    if (occlusion_pass == 1u) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, entity_cull_views_kernel<true, 1>, kEcThreads, 0);
+    else if (occlusion_pass == 2u) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, entity_cull_views_kernel<true, 2>, kEcThreads, 0);
+    else cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, entity_cull_views_kernel<true, 0>, kEcThreads, 0);
     return n;
 }
 

@@ -82,7 +82,8 @@ __global__ void __launch_bounds__(256) hiz_small_kernel(const __grid_constant__ 
     hiz_tail(p, 0u);
 }
 
-__global__ void __launch_bounds__(256) hiz_build_kernel(const __grid_constant__ HizBuildParams p) {
+// One pyramid, one CTA per 64x64 tile of level 0 (blockIdx.x); the batched kernel runs one row of the grid per pyramid.
+__device__ __forceinline__ void hiz_build_body(const HizBuildParams& p) {
     __shared__ float s_l3[8][8];
     __shared__ bool s_last;
     __shared__ float s_top_a[4096], s_top_b[1024];
@@ -201,6 +202,15 @@ __global__ void __launch_bounds__(256) hiz_build_kernel(const __grid_constant__ 
     ORBIT_TRACE_STAMP(p.trace, 4, 4);
 }
 
+__global__ void __launch_bounds__(256) hiz_build_kernel(const __grid_constant__ HizBuildParams p) { hiz_build_body(p); }
+
+// orbit_hiz_build_views: pyramid blockIdx.y; each has its own ticket, so each row's last CTA reduces that pyramid's top levels
+__global__ void __launch_bounds__(256) hiz_build_views_kernel(const __grid_constant__ HizBuildViewsParams pv) { hiz_build_body(pv.view[blockIdx.y]); }
+__global__ void __launch_bounds__(256) hiz_small_views_kernel(const __grid_constant__ HizBuildViewsParams pv) {
+    pdl_wait();
+    hiz_tail(pv.view[blockIdx.y], 0u);
+}
+
 cudaError_t launch_hiz_build(const HizBuildParams& p, cudaStream_t stream) {
     if (p.width >= 64u && p.height >= 64u && p.levels >= 7u) {
         const uint32_t grid = (p.width >> 6) * (p.height >> 6);
@@ -209,6 +219,13 @@ cudaError_t launch_hiz_build(const HizBuildParams& p, cudaStream_t stream) {
         return launch_kernel(hiz_small_kernel, dim3(1), dim3(256), 0, stream, p);
     }
     return cudaGetLastError();
+}
+
+cudaError_t launch_hiz_build_views(const HizBuildViewsParams& pv, cudaStream_t stream) {
+    const HizBuildParams& p = pv.view[0];   // every pyramid of the call has this geometry
+    if (p.width >= 64u && p.height >= 64u && p.levels >= 7u)
+        return launch_kernel(hiz_build_views_kernel, dim3((p.width >> 6) * (p.height >> 6), pv.n_views), dim3(256), 0, stream, pv);
+    return launch_kernel(hiz_small_views_kernel, dim3(1, pv.n_views), dim3(256), 0, stream, pv);
 }
 
 }  // namespace orbit

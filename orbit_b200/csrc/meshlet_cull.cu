@@ -42,9 +42,10 @@ struct ItemTest {
 };
 
 // frustum + cone for one meshlet against the model-view matrix (columns c0..c3, largest column scale `scale`)
-// kProj: 0 perspective, 1 orthographic, -1 decided at run time from ci.projection_type
-template <int kProj>
-__device__ __forceinline__ ItemTest test_item(const OrbitCullInfo& ci, const float4 c0, const float4 c1, const float4 c2, const float4 c3,
+// kProj: 0 perspective, 1 orthographic, -1 decided at run time from ci.projection_type. CI: OrbitCullInfo, or ViewCull (the
+// fields this test reads, staged in shared memory by the batched packed kernel)
+template <int kProj, typename CI>
+__device__ __forceinline__ ItemTest test_item(const CI& ci, const float4 c0, const float4 c1, const float4 c2, const float4 c3,
                                               const float scale, const float cx, const float cy, const float cz, const float r_model,
                                               const uint32_t cone) {
     ItemTest out;
@@ -504,15 +505,18 @@ __device__ __forceinline__ void tile_model_view(const float4* rows, float* mv_ba
 // between the stores and the first drain orders the two), likewise the draw masks and the chunks' survivor counts — so
 // a record never waits for its candidates and there are no per-record result masks to carry.
 //
-// kBatch (orbit_meshlet_cull_views, pass 0): the tiles are those of the CONCATENATION of views[0..n_views)'s record lists,
-// each view's list cut into tiles of its own (a tile never straddles two views). Every CTA reads the views' record counts
-// once (one round trip; lane v of every warp holds view v's count and one past its last tile); a tile takes view matrix, paired
-// planes and alpha filter from its view's block, and its draw masks, side words and survivor counts go to that view's scratch.
-// The scene fields (meshlets, entities, materials) are read from views[0].
+// kBatch (orbit_meshlet_cull_views, pass 0; orbit_meshlet_cull_views_occlusion, pass 1 without and pass 2 with or without
+// meshlet occlusion): the tiles are those of the CONCATENATION of views[0..n_views)'s record lists, each view's list cut into
+// tiles of its own (a tile never straddles two views). Every CTA reads the views' record counts once (one round trip; lane v
+// of every warp holds view v's count and one past its last tile); a tile takes view matrix, paired planes and alpha filter from
+// its view's block, and its draw masks, side words and survivor counts go to that view's scratch. The scene fields (meshlets,
+// entities, materials) are read from views[0]. Pass 2: a tile's last-frame visibility words come from its view's buffer, and
+// the Hi-Z ring holds the candidates of ONE view at a time — when a warp's next tile belongs to another view, an extra empty
+// iteration drains what is left against the old view's pyramid, CullInfo and buffers first (a warp's tiles ascend through
+// the concatenation, so that is at most n_views - 1 partial drains per warp). All pyramids of a call have the same geometry.
 template <int R, bool kPass2, int kProj, bool kBatch>
 __device__ __forceinline__ void meshlet_test_direct_body(const MeshletCullParams* views, uint32_t n_views) {
     static_assert(R == 2 || R == 4 || R == 8, "records per warp tile");
-    static_assert(!(kBatch && kPass2), "batched views are pass 0");
     const MeshletCullParams& p = views[0];
     extern __shared__ __align__(128) unsigned char s_raw[];
     WarpSmem<R>* const all = reinterpret_cast<WarpSmem<R>*>(s_raw + 128);
@@ -623,7 +627,7 @@ __device__ __forceinline__ void meshlet_test_direct_body(const MeshletCullParams
     // lane r < R issues the bulk copy of record r (count x 32 B) and arrives on the barrier
     // ... and the tile's model matrices (lane l < 4R: column l&3 of record l>>2) and, in pass 2, last frame's visibility
     // words (lane 16+r... of record r) go through cp.async into their staging slots: none of the three waits for a load
-    auto issue_tma = [&](uint32_t words) {
+    auto issue_tma = [&](uint32_t words, uint32_t tile) {
         const uint32_t off = __shfl_sync(0xFFFFFFFFu, words, (lane * 4u + 1u) & 31u);
         const uint32_t cnt = __shfl_sync(0xFFFFFFFFu, words, (lane * 4u + 2u) & 31u);
         {
@@ -631,9 +635,11 @@ __device__ __forceinline__ void meshlet_test_direct_body(const MeshletCullParams
             const uint32_t ent_r = __shfl_sync(0xFFFFFFFFu, words, rr * 4u + 0u), cnt_r = __shfl_sync(0xFFFFFFFFu, words, rr * 4u + 2u);
             if (lane < 4u * R && cnt_r != 0u) cp_async_16(rows_s + lane * 16u, p.entities + (size_t)ent_r * 8u + (lane & 3u));
             if (kPass2) {
+                const uint32_t* mvis = p.meshlet_visibility;                  // batched: the visibility words of the tile's view
+                if constexpr (kBatch) mvis = views[locate(tile).view].meshlet_visibility;
                 const uint32_t rv = lane & (uint32_t)(R - 1);
                 const uint32_t vo_r = __shfl_sync(0xFFFFFFFFu, words, rv * 4u + 3u), cnt_v = __shfl_sync(0xFFFFFFFFu, words, rv * 4u + 2u);
-                if (lane >= 16u && lane < 16u + (uint32_t)R && cnt_v != 0u) cp_async_4(vis_s + rv * 4u, p.meshlet_visibility + vo_r);
+                if (lane >= 16u && lane < 16u + (uint32_t)R && cnt_v != 0u) cp_async_4(vis_s + rv * 4u, mvis + vo_r);
             }
             cp_async_commit();
         }
@@ -656,16 +662,18 @@ __device__ __forceinline__ void meshlet_test_direct_body(const MeshletCullParams
     bool trace_first = true;
 #endif
     uint32_t qhead = 0u, qn = 0u;   // ring-buffer read position and fill (entries [qhead, qhead+qn) mod 128 are pending)
-    if (t_cur < tiles_total) issue_tma(cur_word);
+    if (t_cur < tiles_total) issue_tma(cur_word, t_cur);
     // One extra, empty iteration after the last tile flushes what is left in the ring through the same drain code.
     bool final_pass = t_cur >= tiles_total;
     while (true) {
         uint32_t rec0 = t_cur * R;
+        bool view_flush = false;   // batched pass 2: this iteration only drains the ring, the tile waits for the next one
         if constexpr (kBatch) {
             if (!final_pass) {
                 const ViewTile w = locate(t_cur);
                 rec0 = w.rec0; nrec = w.nrec;
-                if (w.view != cur_view) {                                     // warp-uniform; a warp's tiles ascend, so do their views
+                if constexpr (kPass2) view_flush = w.view != cur_view && qn != 0u;   // the ring holds the previous view's candidates
+                if (w.view != cur_view && !view_flush) {                      // warp-uniform; a warp's tiles ascend, so do their views
                     if (lane == 0u && warp_total != 0u) atomicAdd(draw_total, warp_total);
                     warp_total = 0u;
                     cur_view = w.view;
@@ -679,11 +687,12 @@ __device__ __forceinline__ void meshlet_test_direct_body(const MeshletCullParams
                 }
             }
         }
+        const bool flush = final_pass || view_flush;   // an iteration without a tile: only the drain below runs
         const MeshletCullParams& pt = kBatch ? views[cur_view & (ORBIT_MAX_BATCH_VIEWS - 1)] : p;   // the tile's view
-        const uint32_t my_word = final_pass ? 0u : cur_word;
+        const uint32_t my_word = flush ? 0u : cur_word;
         uint32_t my_mask = 0u;       // lane r < R: draw mask of record r (passes without Hi-Z)
         uint32_t vw = 0u;            // lane r < R, pass 2: last frame's visibility word of record r (decides should_draw)
-        if (!final_pass) {
+        if (!flush) {
             cur_word = next_word;
             if constexpr (kBatch) next_word = t_next2 < tiles_total ? load_view_words(t_next2) : 0u;
             else next_word = t_next2 < tiles_total ? load_words(t_next2, nrec) : 0u;
@@ -698,10 +707,10 @@ __device__ __forceinline__ void meshlet_test_direct_body(const MeshletCullParams
                 __syncwarp();
                 if (lane < (uint32_t)R && my_cnt != 0u) {
                     vw = ws.vis[lane];
-                    p.meshlet_visibility[my_vo] = 0u;
+                    pt.meshlet_visibility[my_vo] = 0u;
                 }
                 if (lane < (uint32_t)R && rec0 + lane < nrec) {
-                    p.draw_masks[rec0 + lane] = make_uint4(0u, ent, mof, 1u);   // .w = 1: no side-array entries, the emit kernel reads the meshlet
+                    pt.draw_masks[rec0 + lane] = make_uint4(0u, ent, mof, 1u);   // .w = 1: no side-array entries, the emit kernel reads the meshlet
                     if (main_chunk_counts != nullptr) p.main_masks[rec0 + lane] = make_uint4(0u, ent, mof, 1u);
                 }
             } else {
@@ -715,8 +724,9 @@ __device__ __forceinline__ void meshlet_test_direct_body(const MeshletCullParams
             if (p.scan.trace != nullptr && threadIdx.x == 0 && trace_first) { trace_first = false; ORBIT_TRACE_STAMP(p.scan.trace, 1, 2); }
 #endif
         }
-        // The record loop is deliberately NOT unrolled (instruction cache). The extra, empty iteration after a warp's last
-        // tile (final_pass) only runs the drain below, on whatever is left in the ring.
+        // The record loop is deliberately NOT unrolled (instruction cache). The extra, empty iterations after a warp's last
+        // tile (final_pass) and before a batched warp's first tile of another view (view_flush) only run the drain below, on
+        // whatever is left in the ring.
 #pragma unroll 1
         for (uint32_t r = 0; r < (uint32_t)R; ++r) {
             const uint32_t cnt = __shfl_sync(0xFFFFFFFFu, my_word, r * 4u + 2u);   // 0 for records past the end
@@ -762,19 +772,24 @@ __device__ __forceinline__ void meshlet_test_direct_body(const MeshletCullParams
             }
             // ---- Hi-Z test of 64 queued candidates (the ring holds the < 64 left over plus a record's 32); the warp's
             // very last drain takes whatever is left
-            if (kPass2 && (qn >= 64u || (final_pass && qn != 0u))) {
+            if (kPass2 && (qn >= 64u || (flush && qn != 0u))) {
                 const uint32_t n = min(qn, 64u);
                 __syncwarp();
-                warp_total += drain_candidates<kProj>(p, k, qbase, kRing - 1u, qhead, n, chunk_counts, chunk_shift, hiz_lw, hiz_lh, lane,
+                warp_total += drain_candidates<kProj>(pt, k, qbase, kRing - 1u, qhead, n, chunk_counts, chunk_shift, hiz_lw, hiz_lh, lane,
                                                       main_chunk_counts, main_total);
                 qhead = (qhead + n) & (kRing - 1u);
                 qn -= n;
             }
         }
+        if constexpr (kBatch && kPass2) {
+            // the same tile again, now with an empty ring; its head back at 0: drain_candidates reads candidate pairs with 8-byte
+            // loads and needs an even head, which the odd-sized flush may have left behind
+            if (view_flush) { qhead = 0u; continue; }
+        }
         if (final_pass) break;
         // every lane has read its meshlets: the staging buffer is free -> start the next tile's copy now
         __syncwarp();
-        if (t_next < tiles_total) issue_tma(cur_word);
+        if (t_next < tiles_total) issue_tma(cur_word, t_next);
         if (!kPass2) {
             // one {draw mask, entity, meshlet offset} per record, kept L2-resident for the emit kernel (so it needs one
             // load per record and never touches the dispatch buffer); survivors counted per chunk
@@ -804,10 +819,11 @@ __global__ void __launch_bounds__(kDwThreads, ORBIT_DIRECT_MIN_CTAS) meshlet_tes
     meshlet_test_direct_body<R, kPass2, kProj, false>(&p, 1u);
 }
 
-// orbit_meshlet_cull_views: pass 0 over the concatenation of up to 16 views' record lists
-template <int R, int kProj>
+// orbit_meshlet_cull_views (pass 0) and orbit_meshlet_cull_views_occlusion (kPass2: pass 2 with meshlet occlusion; else pass 1
+// or 2 without it) over the concatenation of up to 16 views' record lists
+template <int R, bool kPass2, int kProj>
 __global__ void __launch_bounds__(kDwThreads, ORBIT_DIRECT_MIN_CTAS) meshlet_test_views_kernel(const __grid_constant__ MeshletViewsParams pv) {
-    meshlet_test_direct_body<R, false, kProj, true>(pv.view, pv.n_views);
+    meshlet_test_direct_body<R, kPass2, kProj, true>(pv.view, pv.n_views);
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -1020,6 +1036,181 @@ __global__ void __launch_bounds__(kMcThreads, ORBIT_PACKED_MIN_CTAS) meshlet_tes
     __syncthreads();
     ORBIT_TRACE_STAMP(p.scan.trace, 2, 4);
 #endif
+}
+
+// orbit_meshlet_cull_views_occlusion, pass 1 with meshlet visibility buffers: meshlet_test_packed_kernel over the concatenation
+// of the views' record lists (each view's list cut into tiles of its own, located as in meshlet_test_direct_body). A CTA's
+// queue mixes the candidates of several views: every warp notes the view and first record of its tile of the round in shared
+// memory, and the fields of each view's CullInfo that the test reads — paired with nothing, the plain test_item arithmetic —
+// are staged once per CTA (16 x 208 bytes), so a candidate is tested against its own view's planes and alpha filter. A warp's
+// tile takes view matrix, visibility words, draw masks, side words and survivor counters from its view.
+struct ViewCull {
+    float cull_planes[ORBIT_MAX_CULL_PLANES][4];
+    uint32_t cull_plane_count, projection_type, alpha_mode_flags, pad;
+};
+template <int R>
+__global__ void __launch_bounds__(kMcThreads, ORBIT_PACKED_MIN_CTAS) meshlet_test_packed_views_kernel(const __grid_constant__ MeshletViewsParams pv) {
+    static_assert(R == 2 || R == 4 || R == 8, "records per warp tile");
+    __shared__ PackedCtaSmem<R> sm;
+    __shared__ ViewCull s_cull[ORBIT_MAX_BATCH_VIEWS];
+    __shared__ uint32_t s_view[kMcWarps], s_rec0[kMcWarps];   // view and first record (inside the view) of each warp's tile
+    const MeshletCullParams* const views = pv.view;
+    const MeshletCullParams& p = views[0];                     // scene fields
+    const uint32_t n_views = pv.n_views;
+    const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
+    const uint32_t lt = (1u << lane) - 1u;
+    pdl_wait();
+    ORBIT_TRACE_STAMP(p.scan.trace, 2, 0);
+    if (threadIdx.x < 2u) sm.qcount[threadIdx.x] = 0u;
+    for (uint32_t v = warp; v < n_views; v += kMcWarps) {      // warp-uniform view, lane = word
+        const OrbitCullInfo& cv = views[v].cull;
+        for (uint32_t i = lane; i < 4u * ORBIT_MAX_CULL_PLANES; i += 32u) (&s_cull[v].cull_planes[0][0])[i] = (&cv.cull_planes[0][0])[i];
+        if (lane == 0u) { s_cull[v].cull_plane_count = cv.cull_plane_count; s_cull[v].projection_type = cv.projection_type; s_cull[v].alpha_mode_flags = cv.alpha_mode_flags; }
+    }
+    // lane v < n_views: view v's record count, its survivor-counter parity and one past its last tile (meshlet_test_direct_body)
+    uint32_t v_nrec = 0u, v_half = 0u, v_tile_end = 0u;
+    if (lane < n_views) {
+        v_nrec = (uint32_t)min((uint64_t)__ldcg(views[lane].dispatch_words), views[lane].capacity_records);
+        v_half = __ldcg(views[lane].chunk_parity) & 1u;
+        if (blockIdx.x == 0 && warp == 0u) views[lane].chunk_parity[1] = v_half;
+    }
+    v_tile_end = (v_nrec + R - 1) / R;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+        const uint32_t t = __shfl_up_sync(0xFFFFFFFFu, v_tile_end, d);
+        if (lane >= (uint32_t)d) v_tile_end += t;
+    }
+    const uint64_t tiles_total = __shfl_sync(0xFFFFFFFFu, v_tile_end, 31);
+    struct ViewTile { uint32_t view, rec0, nrec; };
+    auto locate = [&](uint64_t t) -> ViewTile {                 // t < tiles_total, warp-uniform
+        const uint32_t v = (uint32_t)__popc(__ballot_sync(0xFFFFFFFFu, lane < n_views && v_tile_end <= t));
+        const uint32_t first = __shfl_sync(0xFFFFFFFFu, v_tile_end, (v - 1u) & 31u);
+        return ViewTile{v, ((uint32_t)t - (v ? first : 0u)) * R, __shfl_sync(0xFFFFFFFFu, v_nrec, v & 31u)};
+    };
+    auto tile_words = [&](uint64_t t) -> uint32_t {             // record words of tile t (0 past the end)
+        if (t >= tiles_total) return 0u;
+        const ViewTile w = locate(t);
+        return (lane < 4u * R && w.rec0 + (lane >> 2) < w.nrec) ? __ldcg(views[w.view].dispatch_words + 3u + (size_t)w.rec0 * 4u + lane) : 0u;
+    };
+    auto view_of = [&](uint64_t t) -> uint32_t { return t < tiles_total ? locate(t).view : 0u; };
+    const uint64_t round_stride = (uint64_t)kMcWarps * gridDim.x;
+    const uint64_t tile_first = (uint64_t)warp * gridDim.x + blockIdx.x;
+    uint32_t cur_word = tile_words(tile_first), next_word = tile_words(tile_first + round_stride);
+    ORBIT_TRACE_STAMP_AFTER(p.scan.trace, 2, 1, cur_word);
+    uint32_t cur_view = kNone;                                  // the view whose counters warp_total belongs to
+    uint32_t chunk_rec = 1u;
+    uint32_t* chunk_counts = nullptr;
+    uint32_t* draw_total = nullptr;
+    float v0 = 0.f, v1 = 0.f, v2 = 0.f, v3 = 0.f;
+    const uint32_t vrow_i = lane & 3u;
+    uint32_t warp_total = 0u;
+    PackedPrefetch<R> cur = packed_issue_loads<R>(views[view_of(tile_first)], cur_word, lane);
+    __syncthreads();                                                        // qcount zeroed, CullInfos staged
+    for (uint32_t round = 0; (uint64_t)round * round_stride + blockIdx.x < tiles_total; ++round) {   // CTA-uniform
+        const uint64_t tile = tile_first + (uint64_t)round * round_stride;
+        ViewTile w{0u, 0u, 0u};
+        if (tile < tiles_total) {
+            w = locate(tile);
+            if (w.view != cur_view) {                           // warp-uniform; a warp's tiles ascend, so do their views
+                if (lane == 0u && warp_total != 0u) atomicAdd(draw_total, warp_total);
+                warp_total = 0u;
+                cur_view = w.view;
+                const MeshletCullParams& pv_ = views[cur_view];
+                chunk_rec = 1u << chunk_shift_of(w.nrec);
+                const uint32_t h = __shfl_sync(0xFFFFFFFFu, v_half, cur_view);
+                chunk_counts = pv_.chunk_counts + h * kMaxChunks;
+                draw_total = pv_.draw_total + h;
+                v0 = pv_.cull.view_matrix.m[0][vrow_i]; v1 = pv_.cull.view_matrix.m[1][vrow_i];
+                v2 = pv_.cull.view_matrix.m[2][vrow_i]; v3 = pv_.cull.view_matrix.m[3][vrow_i];
+            }
+        }
+        const uint32_t rec0 = w.rec0;
+        const uint32_t my_word = cur_word;
+        const uint32_t vw = cur.vw;
+        const uint32_t qpar = round & 1u;
+        // ---- A. this warp's tile: record words and matrices into shared memory, candidates into the CTA's queue
+        if (lane < 4u * R) sm.words[warp][lane] = my_word;
+        if (lane < (uint32_t)R) sm.mask[warp][lane] = 0u;
+        if (lane == 0u) { s_view[warp] = w.view; s_rec0[warp] = rec0; }
+        const uint32_t any_vw = __ballot_sync(0xFFFFFFFFu, vw != 0u);
+        if (any_vw != 0u) {                                                 // warp-uniform: tiles without candidates skip the matrix math
+            packed_finish_model_view<R>(cur, &sm.mv[warp][0][0], lane, v0, v1, v2, v3);
+            uint32_t n_items = 0u;
+#pragma unroll
+            for (int r = 0; r < R; ++r) n_items += __popc(__shfl_sync(0xFFFFFFFFu, vw, r));
+            uint32_t base = 0u;
+            if (lane == 0u) base = atomicAdd(&sm.qcount[qpar], n_items);
+            base = __shfl_sync(0xFFFFFFFFu, base, 0);
+#pragma unroll
+            for (int r = 0; r < R; ++r) {
+                const uint32_t m = __shfl_sync(0xFFFFFFFFu, vw, r);
+                if ((m >> lane) & 1u) sm.queue[base + __popc(m & lt)] = (warp << 8) | ((uint32_t)r << 5) | lane;
+                base += __popc(m);
+            }
+        }
+        // ---- start the next round's chain (its record words arrived while the previous round was tested)
+        PackedPrefetch<R> nxt = packed_issue_loads<R>(views[view_of(tile + round_stride)], next_word, lane);
+        const uint32_t next2_word = tile_words(tile + 2u * round_stride);
+        __syncthreads();
+        // ---- C. all warps drain the queue: batches warp, warp + 8, ...; two batches per step
+        const uint32_t total = sm.qcount[qpar];
+        if (threadIdx.x == 0) sm.qcount[qpar ^ 1u] = 0u;                    // the next round's counter (last read two barriers ago)
+        for (uint32_t b0 = warp * 32u; b0 < total; b0 += 2u * kMcWarps * 32u) {
+            uint32_t id[2]; uint4 ma[2], mb[2]; bool live[2]; uint32_t alpha[2];
+#pragma unroll
+            for (int u = 0; u < 2; ++u) {
+                const uint32_t i = b0 + (uint32_t)u * kMcWarps * 32u + lane;
+                live[u] = i < total;
+                id[u] = sm.queue[live[u] ? i : 0u];                         // dead lanes redo candidate 0 and drop the result
+                const uint32_t moff = sm.words[id[u] >> 8][((id[u] >> 5) & 7u) * 4u + 1u];
+                const uint4* m = p.meshlets + 2u * ((size_t)moff + (id[u] & 31u));
+                ma[u] = __ldg(m); mb[u] = __ldg(m + 1);
+            }
+#pragma unroll
+            for (int u = 0; u < 2; ++u)
+                alpha[u] = __ldg(reinterpret_cast<const uint32_t*>(p.materials + (size_t)(mb[u].w & 0xFFFFu) * ORBIT_MATERIAL_STRIDE_BYTES + ORBIT_MATERIAL_ALPHA_MODE_OFFSET));
+            bool pre[2];
+#pragma unroll
+            for (int u = 0; u < 2; ++u) {
+                const float* mvr = &sm.mv[id[u] >> 8][(id[u] >> 5) & 7u][0];
+                const ItemTest t = test_item<-1>(s_cull[s_view[id[u] >> 8]], *reinterpret_cast<const float4*>(mvr), *reinterpret_cast<const float4*>(mvr + 4),
+                                                 *reinterpret_cast<const float4*>(mvr + 8), *reinterpret_cast<const float4*>(mvr + 12), mvr[16],
+                                                 __uint_as_float(ma[u].x), __uint_as_float(ma[u].y), __uint_as_float(ma[u].z), __uint_as_float(ma[u].w), mb[u].x);
+                pre[u] = t.pre_visible;
+            }
+#pragma unroll
+            for (int u = 0; u < 2; ++u) {
+                // should_draw = visible && alpha passes the view's filter (meshlet_cull.comp:207); pass 1: visible_last_frame holds for every candidate
+                const uint32_t w_ = id[u] >> 8, vv = s_view[w_];
+                if (live[u] && pre[u] && (shl1(alpha[u]) & s_cull[vv].alpha_mode_flags) != 0u) {
+                    const uint32_t r = (id[u] >> 5) & 7u, j = id[u] & 31u;
+                    atomicOr(&sm.mask[w_][r], 1u << j);
+                    // the command words of a survivor travel to the emit kernel through its view's side array
+                    uint4* const side = views[vv].cmd_side;
+                    if (side != nullptr) side[((size_t)s_rec0[w_] + r) * 32u + j] = make_uint4(mb[u].y, mb[u].z, mb[u].w, sm.words[w_][r * 4u]);
+                }
+            }
+        }
+        __syncthreads();
+        // ---- E. this warp's tile: draw masks out, survivors counted per chunk of its view
+        uint32_t my_draw_mask = 0u;
+        if (lane < (uint32_t)R) my_draw_mask = sm.mask[warp][lane];
+        if (tile < tiles_total) {
+            const MeshletCullParams& pt = views[w.view];
+            const uint32_t ent = __shfl_sync(0xFFFFFFFFu, my_word, (lane * 4u + 0u) & 31u);
+            const uint32_t mof = __shfl_sync(0xFFFFFFFFu, my_word, (lane * 4u + 1u) & 31u);
+            if (lane < (uint32_t)R && rec0 + lane < w.nrec) pt.draw_masks[rec0 + lane] = make_uint4(my_draw_mask, ent, mof, pt.cmd_side != nullptr ? 0u : 1u);
+            const uint32_t tile_total = __reduce_add_sync(0xFFFFFFFFu, __popc(my_draw_mask));
+            if (lane == 0u && tile_total != 0u) atomicAdd(chunk_counts + rec0 / chunk_rec, tile_total);
+            warp_total += tile_total;
+        }
+        cur = nxt;
+        cur_word = next_word;
+        next_word = next2_word;
+    }
+    ORBIT_TRACE_STAMP(p.scan.trace, 2, 3);
+    pdl_launch_dependents();
+    if (lane == 0u && warp_total != 0u) atomicAdd(draw_total, warp_total);
 }
 
 // Position of the n-th (0-based) set bit of m (n < popc(m)): branch-free binary search on popcounts of halves.
@@ -1486,10 +1677,19 @@ cudaError_t meshlet_cull_configure_device() {
     if (e != cudaSuccess) return e;
     ORBIT_SET(false, 0) ORBIT_SET(false, 1) ORBIT_SET(false, -1) ORBIT_SET(true, 0) ORBIT_SET(true, 1) ORBIT_SET(true, -1)
 #undef ORBIT_SET
-#define ORBIT_SET(proj) \
-    e = cudaFuncSetAttribute(meshlet_test_views_kernel<kTileR, proj>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)direct_smem_bytes()); \
+#define ORBIT_SET(kp2, proj) \
+    e = cudaFuncSetAttribute(meshlet_test_views_kernel<kTileR, kp2, proj>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)direct_smem_bytes()); \
     if (e != cudaSuccess) return e;
-    ORBIT_SET(0) ORBIT_SET(1) ORBIT_SET(-1)
+    ORBIT_SET(false, 0) ORBIT_SET(false, 1) ORBIT_SET(false, -1)
+    return cudaSuccess;
+}
+
+// The same for the batched pass-2 test kernels, called by the first orbit_meshlet_cull_views_occlusion call that needs them
+// rather than by orbit_ctx_create: setting the attribute loads the kernel, and what orbit_ctx_create loads or allocates shifts
+// the device memory allocated after it, to which the single-view stages are sensitive (DESIGN.md §4, batched views).
+cudaError_t meshlet_cull_configure_views_pass2() {
+    cudaError_t e;
+    ORBIT_SET(true, 0) ORBIT_SET(true, 1) ORBIT_SET(true, -1)
 #undef ORBIT_SET
     return cudaSuccess;
 }
@@ -1541,30 +1741,41 @@ cudaError_t launch_meshlet_cull(const MeshletCullParams& p, int grid, int emit_g
     return cudaSuccess;
 }
 
-template <int kProj>
+template <bool kPass2, int kProj>
 static cudaError_t launch_views_test(const MeshletViewsParams& pv, int grid, cudaStream_t stream, int* occupancy) {
     if (occupancy) {
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(occupancy, meshlet_test_views_kernel<kTileR, kProj>, kDwThreads, direct_smem_bytes());
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(occupancy, meshlet_test_views_kernel<kTileR, kPass2, kProj>, kDwThreads, direct_smem_bytes());
         return cudaSuccess;
     }
-    return launch_kernel(meshlet_test_views_kernel<kTileR, kProj>, dim3(grid), dim3(kDwThreads), direct_smem_bytes(), stream, pv);
+    return launch_kernel(meshlet_test_views_kernel<kTileR, kPass2, kProj>, dim3(grid), dim3(kDwThreads), direct_smem_bytes(), stream, pv);
 }
 
-static cudaError_t launch_views_test_any(const MeshletViewsParams& pv, uint32_t projection_type, int grid, cudaStream_t stream, int* occupancy) {
-    if (projection_type == 0u) return launch_views_test<0>(pv, grid, stream, occupancy);
-    if (projection_type == 1u) return launch_views_test<1>(pv, grid, stream, occupancy);
-    return launch_views_test<-1>(pv, grid, stream, occupancy);
+// the batched test kernel of the variant the views' CullInfo selects (all views of a call select the same one): as for a single view
+static cudaError_t launch_views_test_any(const MeshletViewsParams& pv, const OrbitCullInfo& ci, int grid, cudaStream_t stream, int* occupancy) {
+    const TestVariant v = variant_of(ci);
+    if (v.packed) {
+        if (occupancy) { cudaOccupancyMaxActiveBlocksPerMultiprocessor(occupancy, meshlet_test_packed_views_kernel<kPackedR>, kMcThreads, 0); return cudaSuccess; }
+        return launch_kernel(meshlet_test_packed_views_kernel<kPackedR>, dim3(grid), dim3(kMcThreads), 0, stream, pv);
+    }
+    if (v.pass2) {
+        if (v.proj == 0) return launch_views_test<true, 0>(pv, grid, stream, occupancy);
+        if (v.proj == 1) return launch_views_test<true, 1>(pv, grid, stream, occupancy);
+        return launch_views_test<true, -1>(pv, grid, stream, occupancy);
+    }
+    if (v.proj == 0) return launch_views_test<false, 0>(pv, grid, stream, occupancy);
+    if (v.proj == 1) return launch_views_test<false, 1>(pv, grid, stream, occupancy);
+    return launch_views_test<false, -1>(pv, grid, stream, occupancy);
 }
 
-int meshlet_cull_views_max_ctas_per_sm(uint32_t projection_type) {
+int meshlet_cull_views_max_ctas_per_sm(const OrbitCullInfo& ci) {
     int n = 0;
-    launch_views_test_any(MeshletViewsParams{}, projection_type, 0, nullptr, &n);
+    launch_views_test_any(MeshletViewsParams{}, ci, 0, nullptr, &n);
     return n;
 }
 
 // test kernel over the concatenated lists (one persistent wave), then one emit launch with a row of emit_grid_per_view CTAs per view
 cudaError_t launch_meshlet_cull_views(const MeshletViewsParams& pv, int grid, int emit_grid_per_view, cudaStream_t stream) {
-    cudaError_t e = launch_views_test_any(pv, pv.view[0].cull.projection_type, grid, stream, nullptr);
+    cudaError_t e = launch_views_test_any(pv, pv.view[0].cull, grid, stream, nullptr);
     if (e != cudaSuccess) return e;
     return launch_kernel(meshlet_emit_views_kernel, dim3(emit_grid_per_view, pv.n_views), dim3(kEmitWarps * 32), 0, stream, pv);
 }

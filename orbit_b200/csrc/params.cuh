@@ -126,6 +126,11 @@ struct HizBuildParams {
     unsigned int* ticket;  // zero on entry, re-zeroed by the last CTA
     unsigned long long* trace;
 };
+// orbit_hiz_build_views: one block per pyramid (same geometry, own depth buffer, texels and ticket); row blockIdx.y of the grid
+struct HizBuildViewsParams {
+    HizBuildParams view[ORBIT_MAX_BATCH_VIEWS];
+    uint32_t n_views;
+};
 
 struct ClusterParams {
     OrbitClusterCullInfo info;
@@ -150,6 +155,7 @@ int meshlet_emit_max_ctas_per_sm();
 int meshlet_cull_max_ctas_per_sm(const MeshletCullParams&);
 int meshlet_cull_variant_index(const OrbitCullInfo&);
 cudaError_t meshlet_cull_configure_device();
+cudaError_t meshlet_cull_configure_views_pass2();
 cudaError_t light_cluster_configure_device();
 cudaError_t launch_record_masks_put(const uint4* src, const uint32_t* dispatch_words, uint4* dst_region, uint32_t* dst_count, uint64_t capacity,
                                     int grid, cudaStream_t s);
@@ -159,10 +165,11 @@ cudaError_t launch_draws_from_masks(const MeshletCullParams& p, uint32_t* header
 cudaError_t launch_entity_cull(const EntityCullParams&, uint32_t n_draws, uint32_t coresident_ctas, cudaStream_t);
 cudaError_t launch_entity_cull_views(const EntityViewsParams&, uint32_t n_draws, uint32_t coresident_ctas, cudaStream_t);
 cudaError_t launch_meshlet_cull_views(const MeshletViewsParams&, int grid, int emit_grid_per_view, cudaStream_t);
-int meshlet_cull_views_max_ctas_per_sm(uint32_t projection_type);
+int meshlet_cull_views_max_ctas_per_sm(const OrbitCullInfo&);
 int entity_cull_max_ctas_per_sm();
-int entity_cull_views_max_ctas_per_sm();
+int entity_cull_views_max_ctas_per_sm(uint32_t occlusion_pass);
 cudaError_t launch_hiz_build(const HizBuildParams&, cudaStream_t);
+cudaError_t launch_hiz_build_views(const HizBuildViewsParams&, cudaStream_t);
 cudaError_t launch_meshlet_bounds(const MeshletBoundsParams&, int grid, cudaStream_t);
 cudaError_t launch_mesh_bounds(const MeshBoundsParams&, int grid, cudaStream_t);
 cudaError_t launch_scene_update(const SceneUpdateParams&, cudaStream_t);

@@ -17,7 +17,7 @@ import torch
 
 from . import layouts as L
 from .passes import (AssetGraphData, Context, CullInfo, DepthPyramid, OcclusionCullInfo, Projection, SceneGraphData,
-                     create_meshlet_dispatch_command, create_meshlet_draw_commands)
+                     _stream, create_meshlet_dispatch_command, create_meshlet_draw_commands)
 
 
 @dataclass
@@ -152,6 +152,156 @@ def cull_views(context, dscene, cull_infos, name="views", task_payloads=None):
                    "orbit_meshlet_cull_views")
         out.extend((d, w) if p is None else (d, w, p) for d, w, p in bufs)
     return out
+
+
+class _ViewsPass:
+    """One batched occlusion pass (EARLY, LATE or MAIN) of up to MAX_BATCH_VIEWS views, every argument packed once:
+    orbit_entity_cull_views_occlusion + orbit_meshlet_cull_views_occlusion, 3 launches. `infos`: one CullInfo per view (one
+    pass, one projection type); `pyramids`: the views' DepthPyramids (pass 2) or None; `task_payloads`: None or one flag per view."""
+
+    def __init__(self, context, dscene, infos, pyramids, tags, task_payloads=None):
+        import ctypes as C
+        from . import _lib
+        from .passes import _scene_buffers
+        self.context, self._lib, self._C = context, _lib.lib(), C
+        n = self.n = len(infos)
+        sc = dscene.scene
+        self.rcap, self.dcap = int(sc.record_capacity) or 1_000_000, int(sc.draw_capacity) or 1_000_000
+        mk = context.create_transient
+        self.gs = (L.CullInfo * n)(*[ci.to_gpu() for ci in infos])
+        self.sbs = (L.SceneBuffers * n)(*[_scene_buffers(dscene.assets, sc, ci) for ci in infos])
+        self.hizs = (C.c_void_p * n)(*[p._h.value for p in pyramids]) if pyramids is not None else None
+        want = list(task_payloads) if task_payloads is not None else [False] * n
+        self.outputs = [(mk(t + "_meshlet_dispatch_buffer", L.DISPATCH_HEADER + 16 * self.rcap),
+                         mk(t + "_meshlet_draw_command_buffer", L.DRAW_HEADER + 28 * self.dcap),
+                         mk(t + "_task_payloads", 44 * self.rcap) if w else None) for t, w in zip(tags, want)]
+        ptrs = lambda k: (C.c_void_p * n)(*[o[k].data_ptr() if o[k] is not None else None for o in self.outputs])
+        self.dispatch, self.draws = ptrs(0), ptrs(1)
+        self.payloads = ptrs(2) if any(want) else None
+
+    def launch(self, s):
+        from . import _lib
+        h = self.context._h
+        _lib.check(self._lib.orbit_entity_cull_views_occlusion(h, self.gs, self.n, self.sbs, self.hizs, self.dispatch, self.rcap, s),
+                   "orbit_entity_cull_views_occlusion")
+        _lib.check(self._lib.orbit_meshlet_cull_views_occlusion(h, self.gs, self.n, self.sbs, self.hizs, self.dispatch, self.rcap,
+                                                                self.draws, self.dcap, self.payloads, s), "orbit_meshlet_cull_views_occlusion")
+
+    def results(self):
+        return [(d, w) if p is None else (d, w, p) for d, w, p in self.outputs]
+
+
+class _HizViews:
+    """orbit_hiz_build_views for the pyramids of up to MAX_BATCH_VIEWS views (one depth buffer each, all of one size)."""
+
+    def __init__(self, context, pyramids, depth_buffers):
+        import ctypes as C
+        from . import _lib
+        self.context, self._lib, self.pyramids = context, _lib.lib(), list(pyramids)
+        n = self.n = len(self.pyramids)
+        shapes = {tuple(d.shape) for d in depth_buffers}
+        assert len(shapes) == 1, "every depth buffer of a batch has the same size"
+        self.h, self.w = shapes.pop()
+        assert all(d.dtype == torch.float32 and d.is_contiguous() for d in depth_buffers)
+        self.depths = list(depth_buffers)
+        self.hizs = (C.c_void_p * n)(*[p._h.value for p in self.pyramids])
+        self.dptrs = (C.c_void_p * n)(*[d.data_ptr() for d in self.depths])
+
+    def launch(self, s):
+        from . import _lib
+        _lib.check(self._lib.orbit_hiz_build_views(self.context._h, self.hizs, self.dptrs, self.n, self.w, self.h, s), "orbit_hiz_build_views")
+        for p in self.pyramids:
+            p.usable = True
+
+
+def _groups(n):
+    return [range(g0, min(g0 + L.MAX_BATCH_VIEWS, n)) for g0 in range(0, n, L.MAX_BATCH_VIEWS)]
+
+
+def _early_info(vstate, view, meshlet_occlusion):
+    return cull_info_for(view, OcclusionCullInfo("read", vstate.entity_visibility, vstate.meshlet_visibility if meshlet_occlusion else None))
+
+
+def _late_info(vstate, view, meshlet_occlusion):
+    mvis = vstate.meshlet_visibility if meshlet_occlusion else None
+    return cull_info_for(view, OcclusionCullInfo("write", vstate.entity_visibility, mvis, vstate.depth_pyramid, noskip_alphamode=0,
+                                                 aspect_ratio=view.aspect))
+
+
+def depth_prepass_views(context, dscene, vstates, views, depth_buffers, meshlet_occlusion=True, name="forward_depth_prepass"):
+    """depth_prepass_culling for several cameras over one scene: EARLY, Hi-Z and LATE of every group of up to MAX_BATCH_VIEWS
+    cameras in 3 + 1 + 3 launches (orbit_*_cull_views_occlusion, orbit_hiz_build_views). `vstates`, `views`, `depth_buffers`:
+    one per camera (one projection type, depth buffers of one size). Returns one {"early": .., "late": ..} per camera, each
+    (dispatch_buffer, draw_buffer), byte for byte what depth_prepass_culling returns for that camera alone."""
+    s = _stream(context)
+    out = []
+    for g in _groups(len(views)):
+        early = _ViewsPass(context, dscene, [_early_info(vstates[v], views[v], meshlet_occlusion) for v in g], None,
+                           ["early_%s%d" % (name, v) for v in g])
+        early.launch(s)
+        _HizViews(context, [vstates[v].depth_pyramid for v in g], [depth_buffers[v] for v in g]).launch(s)
+        late = _ViewsPass(context, dscene, [_late_info(vstates[v], views[v], meshlet_occlusion) for v in g],
+                          [vstates[v].depth_pyramid for v in g], ["late_%s%d" % (name, v) for v in g])
+        late.launch(s)
+        out.extend({"early": e, "late": l} for e, l in zip(early.results(), late.results()))
+    return out
+
+
+def main_pass_views(context, dscene, vstates, views, meshlet_occlusion=True, name="forward"):
+    """main_pass_culling for several cameras: MAIN (pass 1 over the bits the LATE pass wrote) of every group of up to
+    MAX_BATCH_VIEWS cameras in 3 launches. Returns one (dispatch_buffer, draw_buffer) per camera."""
+    s = _stream(context)
+    out = []
+    for g in _groups(len(views)):
+        main = _ViewsPass(context, dscene, [_early_info(vstates[v], views[v], meshlet_occlusion) for v in g], None,
+                          ["%s%d" % (name, v) for v in g])
+        main.launch(s)
+        out.extend(main.results())
+    return out
+
+
+class PreparedViews:
+    """PreparedFrame for several cameras over one scene: EARLY -> Hi-Z -> LATE (and, with `main_pass`, MAIN) of every camera,
+    every argument packed once, 3 + 1 + 3 (+ 3) launches per group of up to MAX_BATCH_VIEWS cameras instead of 7 (10) per
+    camera. `capture()` / `replay()` put the whole multi-camera frame into one CUDA graph. `outputs[v]`: camera v's
+    {"early", "late"[, "main"]} -> (dispatch_buffer, draw_buffer)."""
+
+    def __init__(self, context, dscene, vstates, views, depth_buffers, meshlet_occlusion=True, name="views", main_pass=True):
+        self.context = context
+        self.stages = []
+        self.outputs = [dict() for _ in views]
+        for g in _groups(len(views)):
+            pyr = [vstates[v].depth_pyramid for v in g]
+            early_infos = [_early_info(vstates[v], views[v], meshlet_occlusion) for v in g]
+            passes = [("early", _ViewsPass(context, dscene, early_infos, None, ["early_%s%d" % (name, v) for v in g])),
+                      ("hiz", _HizViews(context, pyr, [depth_buffers[v] for v in g])),
+                      ("late", _ViewsPass(context, dscene, [_late_info(vstates[v], views[v], meshlet_occlusion) for v in g], pyr,
+                                          ["late_%s%d" % (name, v) for v in g]))]
+            if main_pass:
+                passes.append(("main", _ViewsPass(context, dscene, early_infos, None, ["main_%s%d" % (name, v) for v in g])))
+            for k, st in passes:
+                if k != "hiz":
+                    for v, r in zip(g, st.results()):
+                        self.outputs[v][k] = r
+            self.stages.extend(st for _, st in passes)
+        self.graph = None
+
+    def launch(self):
+        s = _stream(self.context)
+        for st in self.stages:
+            st.launch(s)
+
+    def capture(self):
+        self.launch()  # warm: scratch growth / occupancy queries must not happen during capture
+        torch.cuda.synchronize()
+        g = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(g):
+            self.launch()
+        self.graph = g
+        return g
+
+    def replay(self):
+        self.graph.replay()
 
 
 def shadow_pass_culling(context, dscene, view, name="shadow"):

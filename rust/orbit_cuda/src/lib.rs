@@ -152,6 +152,15 @@ extern "C" {
     pub fn orbit_meshlet_cull_views(ctx: *mut orbit_ctx, culls: *const OrbitCullInfo, n_views: u32, scene: *const OrbitSceneBuffers,
                                     dispatch_buffers: *const *const c_void, capacity_records: u64, draw_command_buffers: *const *mut c_void,
                                     capacity_draws: u64, task_payloads: *const *mut c_void, stream: *mut c_void) -> c_int;
+    pub fn orbit_hiz_build_views(ctx: *mut orbit_ctx, hizs: *const *mut orbit_hiz, depths: *const *const f32, n_views: u32,
+                                 depth_width: u32, depth_height: u32, stream: *mut c_void) -> c_int;
+    pub fn orbit_entity_cull_views_occlusion(ctx: *mut orbit_ctx, culls: *const OrbitCullInfo, n_views: u32, scenes: *const OrbitSceneBuffers,
+                                             hizs: *const *const orbit_hiz, dispatch_buffers: *const *mut c_void, capacity_records: u64,
+                                             stream: *mut c_void) -> c_int;
+    pub fn orbit_meshlet_cull_views_occlusion(ctx: *mut orbit_ctx, culls: *const OrbitCullInfo, n_views: u32, scenes: *const OrbitSceneBuffers,
+                                              hizs: *const *const orbit_hiz, dispatch_buffers: *const *const c_void, capacity_records: u64,
+                                              draw_command_buffers: *const *mut c_void, capacity_draws: u64, task_payloads: *const *mut c_void,
+                                              stream: *mut c_void) -> c_int;
     pub fn orbit_draws_scatter_ranked(ctx: *mut orbit_ctx, src_draw_buffer: *const c_void, src_capacity_draws: u64, dst_draw_buffer: *mut c_void,
                                       rank_counts: *const u32, rank: u32, world: u32, dst_capacity_draws: u64, stream: *mut c_void) -> i32;
     pub fn orbit_meshlet_test(ctx: *mut orbit_ctx, cull: *const OrbitCullInfo, scene: *const OrbitSceneBuffers, hiz: *const orbit_hiz,
@@ -221,6 +230,39 @@ impl Context {
         check(orbit_entity_cull_views(self.0, culls.as_ptr(), n, scene, dispatch_buffers.as_ptr(), capacity_records, stream))?;
         check(orbit_meshlet_cull_views(self.0, culls.as_ptr(), n, scene, dispatch_buffers.as_ptr() as *const *const c_void, capacity_records,
                                        draw_command_buffers.as_ptr(), capacity_draws, std::ptr::null(), stream))
+    }
+    /// One occlusion pass (EARLY or MAIN: pass 1; LATE: pass 2) of up to ORBIT_MAX_BATCH_VIEWS cameras over one scene: buffer v
+    /// receives what create_meshlet_dispatch_command / create_meshlet_draw_commands write for `culls[v]` with `scenes[v]` (the
+    /// scene with camera v's visibility buffers) and, for pass 2, `pyramids[v]`; 3 kernel launches in all. Every slice has one
+    /// entry per camera (`pyramids` is empty for pass 1).
+    pub unsafe fn create_views_occlusion_commands(&self, culls: &[OrbitCullInfo], scenes: &[OrbitSceneBuffers], pyramids: &[DepthPyramid],
+                                                  dispatch_buffers: &[*mut c_void], capacity_records: u64,
+                                                  draw_command_buffers: &[*mut c_void], capacity_draws: u64,
+                                                  stream: *mut c_void) -> Result<(), Error> {
+        let n = culls.len();
+        if n > ORBIT_MAX_BATCH_VIEWS as usize || scenes.len() != n || dispatch_buffers.len() != n || draw_command_buffers.len() != n
+            || !(pyramids.is_empty() || pyramids.len() == n) {
+            return Err(Error(ORBIT_ERR_INVALID_ARGUMENT));
+        }
+        let hizs: Vec<*const orbit_hiz> = pyramids.iter().map(|p| p.hiz as *const orbit_hiz).collect();
+        let hz = if hizs.is_empty() { std::ptr::null() } else { hizs.as_ptr() };
+        check(orbit_entity_cull_views_occlusion(self.0, culls.as_ptr(), n as u32, scenes.as_ptr(), hz, dispatch_buffers.as_ptr(),
+                                                capacity_records, stream))?;
+        check(orbit_meshlet_cull_views_occlusion(self.0, culls.as_ptr(), n as u32, scenes.as_ptr(), hz,
+                                                 dispatch_buffers.as_ptr() as *const *const c_void, capacity_records,
+                                                 draw_command_buffers.as_ptr(), capacity_draws, std::ptr::null(), stream))
+    }
+    /// update_multiple_depth_pyramids (draw_gen.rs): DepthPyramid::update for up to ORBIT_MAX_BATCH_VIEWS pyramids of one size in
+    /// one launch; depth buffer v feeds pyramid v.
+    pub unsafe fn update_depth_pyramids(&self, pyramids: &mut [DepthPyramid], depths: &[*const f32], stream: *mut c_void) -> Result<(), Error> {
+        if pyramids.is_empty() || pyramids.len() > ORBIT_MAX_BATCH_VIEWS as usize || depths.len() != pyramids.len() {
+            return Err(Error(ORBIT_ERR_INVALID_ARGUMENT));
+        }
+        let size = pyramids[0].size;
+        let hizs: Vec<*mut orbit_hiz> = pyramids.iter().map(|p| p.hiz).collect();
+        check(orbit_hiz_build_views(self.0, hizs.as_ptr(), depths.as_ptr(), pyramids.len() as u32, size[0], size[1], stream))?;
+        for p in pyramids.iter_mut() { p.usable = true; }
+        Ok(())
     }
 }
 impl Drop for Context { fn drop(&mut self) { unsafe { orbit_ctx_destroy(self.0) } } }
