@@ -188,6 +188,21 @@ int orbit_meshlet_cull_late_main(orbit_ctx* ctx, const OrbitCullInfo* late, cons
                                  uint64_t capacity_draws, void* late_task_payloads /* nullable */,
                                  void* main_task_payloads /* nullable */, void* stream);
 
+/* ---- Hi-Z build + LATE entity cull in one call ------------------------------------------------------------------------------
+ * Byte for byte what
+ *   orbit_hiz_build(ctx, hiz, depth, depth_width, depth_height) ; orbit_entity_cull(ctx, late, scene, hiz, late_dispatch_buffer)
+ * write when main_pass is NULL (main_dispatch_buffer must then be NULL too), and what
+ *   orbit_hiz_build(...) ; orbit_entity_cull_late_main(ctx, late, main_pass, scene, hiz, late_dispatch_buffer, main_dispatch_buffer)
+ * write otherwise: every pyramid texel, the entity visibility words, the dispatch buffers and the status words. Two launches,
+ * as the separate calls, but the entity kernel does everything that does not read the pyramid while the build is still
+ * running. Every argument rule of the two calls applies, and late->occlusion_pass must be 2; a refused call
+ * (ORBIT_ERR_INVALID_ARGUMENT) launches nothing. Counts as an orbit_hiz_build call and an orbit_entity_cull call (concurrency rules at the top).
+ * Only sound because the call enqueues the build itself: the entity stage after any other predecessor is orbit_entity_cull. */
+int orbit_hiz_build_entity_cull_late(orbit_ctx* ctx, orbit_hiz* hiz, const float* depth, uint32_t depth_width,
+                                     uint32_t depth_height, const OrbitCullInfo* late, const OrbitCullInfo* main_pass /* nullable */,
+                                     const OrbitSceneBuffers* scene, void* late_dispatch_buffer,
+                                     void* main_dispatch_buffer /* nullable */, uint64_t capacity_records, void* stream);
+
 /* ---- batched pass-0 views (the cascades of ShadowRenderer::render_cascaded_shadow, shadow_renderer.rs:466-712; many cameras
  *      over one scene) ---------------------------------------------------------------------------------------------------
  * n_views (1..ORBIT_MAX_BATCH_VIEWS) pass-0 views of ONE scene. View v's buffers are byte for byte what

@@ -83,7 +83,7 @@ struct orbit_ctx {
     int mc_ctas_per_sm = 0;
     int emit_occupancy = 0;
     int debug_skip = 0;               // ORBIT_DEBUG_SKIP: 1 = skip emit kernel, 2 = skip test kernel (timing experiments only)
-    int entity_occupancy = 0;
+    int entity_occupancy[2] = {0, 0};                  // entity_cull_kernel CTAs per SM: [0] as launched by orbit_entity_cull, [1] deferred wait
     int entity_views_occupancy[3] = {0, 0, 0};        // the same for the batched entity kernel, per pass (more registers: fewer CTAs per SM)
     int mc_occupancy[8] = {0, 0, 0, 0, 0, 0, 0, 0};   // cached occupancy per meshlet test-kernel variant
     int views_occupancy[8] = {0, 0, 0, 0, 0, 0, 0, 0}; // the same for the batched test kernels, per variant
@@ -384,16 +384,24 @@ int orbit_hiz_info(const orbit_hiz* h, OrbitHizInfo* out) {
     return ORBIT_OK;
 }
 
-int orbit_hiz_build(orbit_ctx* c, orbit_hiz* h, const float* depth, uint32_t dw, uint32_t dh, void* stream) {
-    if (!c || !h || !depth || dw != h->depth_w || dh != h->depth_h) return ORBIT_ERR_INVALID_ARGUMENT;
-    GUARD(c);
+static bool hiz_build_args_ok(orbit_ctx* c, orbit_hiz* h, const float* depth, uint32_t dw, uint32_t dh) {
+    return c && h && depth && dw == h->depth_w && dh == h->depth_h;
+}
+
+static HizBuildParams hiz_build_params(orbit_ctx* c, orbit_hiz* h, const float* depth, uint32_t dw, uint32_t dh) {
     HizBuildParams p{};
     p.depth = depth; p.texels = h->info.texels; p.depth_w = dw; p.depth_h = dh;
     p.width = h->info.width; p.height = h->info.height; p.levels = h->info.levels;
     for (int i = 0; i < ORBIT_HIZ_MAX_LEVELS; ++i) p.level_offset[i] = h->info.level_offset[i];
     p.ticket = c->counters + 2;
     p.trace = next_trace(c);
-    CK(launch_hiz_build(p, (cudaStream_t)stream));
+    return p;
+}
+
+int orbit_hiz_build(orbit_ctx* c, orbit_hiz* h, const float* depth, uint32_t dw, uint32_t dh, void* stream) {
+    if (!hiz_build_args_ok(c, h, depth, dw, dh)) return ORBIT_ERR_INVALID_ARGUMENT;
+    GUARD(c);
+    CK(launch_hiz_build(hiz_build_params(c, h, depth, dw, dh), (cudaStream_t)stream));
     c->launches += 1;
     return ORBIT_OK;
 }
@@ -470,9 +478,10 @@ static EntityCullParams entity_params(orbit_ctx* c, const OrbitCullInfo* cull, c
     return p;
 }
 
-static uint32_t entity_coresident_ctas(orbit_ctx* c) {
-    if (c->entity_occupancy <= 0) c->entity_occupancy = entity_cull_max_ctas_per_sm();
-    return (uint32_t)(c->sm_count * (c->entity_occupancy > 0 ? c->entity_occupancy : 1));
+static uint32_t entity_coresident_ctas(orbit_ctx* c, bool defer_wait) {
+    int& occ = c->entity_occupancy[defer_wait ? 1 : 0];
+    if (occ <= 0) occ = entity_cull_max_ctas_per_sm(defer_wait);
+    return (uint32_t)(c->sm_count * (occ > 0 ? occ : 1));
 }
 
 static uint32_t entity_views_coresident_ctas(orbit_ctx* c, uint32_t pass) {
@@ -481,24 +490,37 @@ static uint32_t entity_views_coresident_ctas(orbit_ctx* c, uint32_t pass) {
     return (uint32_t)(c->sm_count * (occ > 0 ? occ : 1));
 }
 
-static int entity_stage(orbit_ctx* c, const OrbitCullInfo* cull, const OrbitSceneBuffers* scene, const orbit_hiz* hiz,
-                        void* meshlet_dispatch_buffer, void* mirror_dispatch_buffer, uint64_t capacity_records, void* stream) {
+// Every argument rule of one entity-stage call; on success, the draw range it covers. Launches nothing.
+static int entity_stage_args(orbit_ctx* c, const OrbitCullInfo* cull, const OrbitSceneBuffers* scene, const orbit_hiz* hiz,
+                             void* meshlet_dispatch_buffer, uint32_t* begin, uint32_t* end) {
     if (!c || !meshlet_dispatch_buffer || ((uintptr_t)meshlet_dispatch_buffer & 3u)) return ORBIT_ERR_INVALID_ARGUMENT;
     int rc = check_cull(cull, scene, hiz, false);
     if (rc != ORBIT_OK) return rc;
-    uint32_t begin, end;
-    rc = draw_range(scene, &begin, &end);
-    if (rc != ORBIT_OK) return rc;
-    const uint32_t n = end - begin;
-    GUARD(c);
-    rc = ensure_status(c, (size_t)(n + 255u) / 256u + 1u, (cudaStream_t)stream);
-    if (rc != ORBIT_OK) return rc;
+    return draw_range(scene, begin, end);
+}
+
+// One entity-stage launch over draws [begin, end), arguments already checked, device already current. `defer_wait`: the
+// kernel variant that may only follow this library's Hi-Z build directly (orbit_hiz_build_entity_cull_late).
+static int entity_launch(orbit_ctx* c, const OrbitCullInfo* cull, const OrbitSceneBuffers* scene, const orbit_hiz* hiz,
+                         void* meshlet_dispatch_buffer, void* mirror_dispatch_buffer, uint64_t capacity_records, uint32_t begin, uint32_t end,
+                         void* stream, bool defer_wait) {
     EntityCullParams p = entity_params(c, cull, scene, hiz, meshlet_dispatch_buffer, capacity_records, begin, end);
     p.dispatch_mirror = (uint32_t*)mirror_dispatch_buffer;
     p.scan = next_scan(c);
-    CK(launch_entity_cull(p, n, entity_coresident_ctas(c), (cudaStream_t)stream));
+    CK(launch_entity_cull(p, end - begin, entity_coresident_ctas(c, defer_wait), (cudaStream_t)stream, defer_wait));
     c->launches += 1;
     return ORBIT_OK;
+}
+
+static int entity_stage(orbit_ctx* c, const OrbitCullInfo* cull, const OrbitSceneBuffers* scene, const orbit_hiz* hiz,
+                        void* meshlet_dispatch_buffer, void* mirror_dispatch_buffer, uint64_t capacity_records, void* stream) {
+    uint32_t begin, end;
+    int rc = entity_stage_args(c, cull, scene, hiz, meshlet_dispatch_buffer, &begin, &end);
+    if (rc != ORBIT_OK) return rc;
+    GUARD(c);
+    rc = ensure_status(c, (size_t)(end - begin + 255u) / 256u + 1u, (cudaStream_t)stream);
+    if (rc != ORBIT_OK) return rc;
+    return entity_launch(c, cull, scene, hiz, meshlet_dispatch_buffer, mirror_dispatch_buffer, capacity_records, begin, end, stream, false);
 }
 
 int orbit_entity_cull(orbit_ctx* c, const OrbitCullInfo* cull, const OrbitSceneBuffers* scene, const orbit_hiz* hiz,
@@ -530,12 +552,42 @@ int orbit_cull_pair_compatible(const OrbitCullInfo* late, const OrbitCullInfo* m
     return 1;
 }
 
+static bool late_main_args_ok(const OrbitCullInfo* late, const OrbitCullInfo* main_pass, const void* late_dispatch_buffer,
+                              const void* main_dispatch_buffer) {
+    if (!main_dispatch_buffer || ((uintptr_t)main_dispatch_buffer & 3u) || main_dispatch_buffer == late_dispatch_buffer) return false;
+    return orbit_cull_pair_compatible(late, main_pass) != 0;
+}
+
 int orbit_entity_cull_late_main(orbit_ctx* c, const OrbitCullInfo* late, const OrbitCullInfo* main_pass, const OrbitSceneBuffers* scene,
                                 const orbit_hiz* hiz, void* late_dispatch_buffer, void* main_dispatch_buffer, uint64_t capacity_records,
                                 void* stream) {
-    if (!main_dispatch_buffer || ((uintptr_t)main_dispatch_buffer & 3u) || main_dispatch_buffer == late_dispatch_buffer) return ORBIT_ERR_INVALID_ARGUMENT;
-    if (!orbit_cull_pair_compatible(late, main_pass)) return ORBIT_ERR_INVALID_ARGUMENT;
+    if (!late_main_args_ok(late, main_pass, late_dispatch_buffer, main_dispatch_buffer)) return ORBIT_ERR_INVALID_ARGUMENT;
     return entity_stage(c, late, scene, hiz, late_dispatch_buffer, main_dispatch_buffer, capacity_records, stream);
+}
+
+// ---- Hi-Z build + LATE entity cull in one call -----------------------------------------------------------
+// orbit_hiz_build, then orbit_entity_cull (pass 2) or, with main_pass, orbit_entity_cull_late_main, on the pyramid just built.
+// Because the call itself enqueues the build right before the entity kernel, the entity kernel may run everything that does
+// not read the pyramid before its griddepcontrol.wait (entity_cull_kernel<., true>; DESIGN.md §4 has the hazard proof). The
+// build triggers its dependents where orbit_hiz_build does, once its tile is reduced: triggering right after its own wait
+// made the C2 frame 1.3 us slower instead of 2.6 us faster (entity CTAs beside a running build slow both). Every argument is checked, and
+// the scan descriptors are grown (ensure_status may enqueue a memset), before the build is launched: a refused call launches
+// nothing, and nothing but the build sits between the two kernels on the stream.
+int orbit_hiz_build_entity_cull_late(orbit_ctx* c, orbit_hiz* h, const float* depth, uint32_t dw, uint32_t dh, const OrbitCullInfo* late,
+                                     const OrbitCullInfo* main_pass, const OrbitSceneBuffers* scene, void* late_dispatch_buffer,
+                                     void* main_dispatch_buffer, uint64_t capacity_records, void* stream) {
+    if (!hiz_build_args_ok(c, h, depth, dw, dh) || !late || late->occlusion_pass != 2u) return ORBIT_ERR_INVALID_ARGUMENT;
+    if (main_pass ? !late_main_args_ok(late, main_pass, late_dispatch_buffer, main_dispatch_buffer) : main_dispatch_buffer != nullptr)
+        return ORBIT_ERR_INVALID_ARGUMENT;
+    uint32_t begin, end;
+    int rc = entity_stage_args(c, late, scene, h, late_dispatch_buffer, &begin, &end);
+    if (rc != ORBIT_OK) return rc;
+    GUARD(c);
+    rc = ensure_status(c, (size_t)(end - begin + 255u) / 256u + 1u, (cudaStream_t)stream);
+    if (rc != ORBIT_OK) return rc;
+    CK(launch_hiz_build(hiz_build_params(c, h, depth, dw, dh), (cudaStream_t)stream));
+    c->launches += 1;
+    return entity_launch(c, late, scene, h, late_dispatch_buffer, main_dispatch_buffer, capacity_records, begin, end, stream, true);
 }
 
 // ---- meshlet stage ---------------------------------------------------------------------------------------

@@ -24,7 +24,33 @@ constexpr int kEcThreads = ORBIT_EC_THREADS;   // entity draws per CTA (tuning e
 constexpr uint32_t kEcBatch = 2048u;           // records staged in shared memory per round of the emission (32 KB)
 
 
-template <bool kFlat>
+// LOD selection of one drawn entity (as in entity_cull.comp): its meshlet range (offset, count) from the MeshInfo's LOD table
+__device__ __forceinline__ uint2 select_lod(const OrbitCullInfo& ci, const Sphere& s, const uint4 mi_hdr, const uint4 (&lods)[4]) {
+    const float dx = sub(ci.lod_target_pos_view_space[0], s.x);
+    const float dy = sub(ci.lod_target_pos_view_space[1], s.y);
+    const float dz = sub(ci.lod_target_pos_view_space[2], s.z);
+    const float lod_distance = sub(fsqrt(dot3(dx, dy, dz, dx, dy, dz)), s.r);
+    const float f = fdiv(orbit_log2f(fdiv(fmaxf(lod_distance, 0.0f), ci.lod_base)), orbit_log2f(ci.lod_step));
+    uint32_t lod = f2u(fmaxf(add(f, 1.0f), 0.0f));
+    lod = min(max(lod, ci.min_mesh_lod), ci.max_mesh_lod);
+    const uint32_t lod_count = mi_hdr.z;
+    const uint32_t li = min(lod, lod_count - 1u) & 7u;
+    uint2 L = make_uint2(lods[0].x, lods[0].y);
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        if (li == 2u * k) L = make_uint2(lods[k].x, lods[k].y);
+        if (li == 2u * k + 1u) L = make_uint2(lods[k].z, lods[k].w);
+    }
+    return L;
+}
+
+// kDeferWait (orbit_hiz_build_entity_cull_late only: pass 2, launched right behind this library's own Hi-Z build) moves
+// griddepcontrol.wait from the first line to just before the first pyramid texel is read. Everything before it reads only
+// data the Hi-Z build never writes, through L2 (DESIGN.md §4, "Hi-Z build + LATE entity cull in one call": the hazard proof),
+// and stores nothing but the tile ticket: ticket, draw words, MeshInfo / matrix / visibility-bit loads, view * model, sphere,
+// frustum, the projection half of the occlusion test, and the LOD of every frustum-visible draw (speculative: it is dropped
+// when the texel test rejects the draw). So that work runs while the build's tail is still reducing.
+template <bool kFlat, bool kDeferWait = false>
 __global__ void __launch_bounds__(kEcThreads) entity_cull_kernel(const __grid_constant__ EntityCullParams p) {
     __shared__ uint4 s_recs[kEcBatch];            // the tile's records, staged for coalesced stores
     __shared__ uint32_t s_warp[kEcThreads / 32];
@@ -32,7 +58,7 @@ __global__ void __launch_bounds__(kEcThreads) entity_cull_kernel(const __grid_co
 
     const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
     const OrbitCullInfo& ci = p.cull;
-    pdl_wait();
+    if (!kDeferWait) pdl_wait();
     ORBIT_TRACE_STAMP(p.scan.trace, 0, 0);
     const unsigned int epoch = scan_epoch(p.scan);
     // Tiles are handed out by an atomic ticket in BOTH variants, so the CTAs that own a tile's predecessors are always running
@@ -51,12 +77,14 @@ __global__ void __launch_bounds__(kEcThreads) entity_cull_kernel(const __grid_co
 
     // The draw words are requested before the device-side count is known (gid < draw_end <= the host's
     // entity_draw_count, which sized the buffer): one dependent round trip less on a latency-bound kernel.
+    // (before the wait, kDeferWait: through L2, never the non-coherent L1 path — see the hazard proof)
+    auto draw_word = [&](size_t i) -> uint32_t { return kDeferWait ? __ldcg(p.entity_draw_words + i) : __ldg(p.entity_draw_words + i); };
     uint32_t gid = p.draw_begin + tile * kEcThreads + tid;
     uint32_t entity_index = 0u, mesh_index = 0u, vis_offset = 0u;
     if (gid < p.draw_end) {
-        entity_index = __ldg(p.entity_draw_words + 1u + 3u * (size_t)gid + 0u);
-        mesh_index = __ldg(p.entity_draw_words + 1u + 3u * (size_t)gid + 1u);
-        vis_offset = __ldg(p.entity_draw_words + 1u + 3u * (size_t)gid + 2u);
+        entity_index = draw_word(1u + 3u * (size_t)gid + 0u);
+        mesh_index = draw_word(1u + 3u * (size_t)gid + 1u);
+        vis_offset = draw_word(1u + 3u * (size_t)gid + 2u);
     }
     if (kFlat) {
         __syncthreads();
@@ -65,19 +93,22 @@ __global__ void __launch_bounds__(kEcThreads) entity_cull_kernel(const __grid_co
             gid = p.draw_begin + tile * kEcThreads + tid;
             entity_index = mesh_index = vis_offset = 0u;
             if (gid < p.draw_end) {
-                entity_index = __ldg(p.entity_draw_words + 1u + 3u * (size_t)gid + 0u);
-                mesh_index = __ldg(p.entity_draw_words + 1u + 3u * (size_t)gid + 1u);
-                vis_offset = __ldg(p.entity_draw_words + 1u + 3u * (size_t)gid + 2u);
+                entity_index = draw_word(1u + 3u * (size_t)gid + 0u);
+                mesh_index = draw_word(1u + 3u * (size_t)gid + 1u);
+                vis_offset = draw_word(1u + 3u * (size_t)gid + 2u);
             }
         }
     }
-    const uint32_t count = min(__ldg(p.entity_draw_words), p.draw_end);
+    const uint32_t count = min(draw_word(0u), p.draw_end);
     ORBIT_TRACE_STAMP(p.scan.trace, 0, 1 + 0 * (count + epoch));
-    const uint32_t pass = ci.occlusion_pass;
+    const uint32_t pass = kDeferWait ? 2u : ci.occlusion_pass;
     const bool mocc = ci.meshlet_visibility_buffer != ORBIT_NO_BUFFER;
 
     uint32_t chunks = 0u, lod_off = 0u, lod_cnt = 0u;
     bool visible = false;
+    HizProbe probe;                    // kDeferWait: the occlusion test up to the texel loads
+    const uint32_t hiz_lw = hiz_log2(p.hiz.width), hiz_lh = hiz_log2(p.hiz.height);
+    bool keep = false;                 // kDeferWait: should_draw of a draw that passes the occlusion test
     const bool in_range = gid < count;
     if (in_range) {
         // every load that depends only on the draw words, issued back to back (ordered loads, orbit_device.cuh): what
@@ -110,28 +141,29 @@ __global__ void __launch_bounds__(kEcThreads) entity_cull_kernel(const __grid_co
         mv.scale = largest_scale(mv.m);
         Sphere s = transform_sphere(mv, sph.x, sph.y, sph.z, sph.w);
         if (visible) visible = frustum_test(ci, s);
-        if (pass == 2u && visible) visible = occlusion_test(ci, s, p.hiz);
-        bool should_draw = visible;
-        if (pass == 2u) should_draw = visible && (!vib || mocc);
-        if (should_draw) {
-            const float dx = sub(ci.lod_target_pos_view_space[0], s.x);
-            const float dy = sub(ci.lod_target_pos_view_space[1], s.y);
-            const float dz = sub(ci.lod_target_pos_view_space[2], s.z);
-            const float lod_distance = sub(fsqrt(dot3(dx, dy, dz, dx, dy, dz)), s.r);
-            const float f = fdiv(orbit_log2f(fdiv(fmaxf(lod_distance, 0.0f), ci.lod_base)), orbit_log2f(ci.lod_step));
-            uint32_t lod = f2u(fmaxf(add(f, 1.0f), 0.0f));
-            lod = min(max(lod, ci.min_mesh_lod), ci.max_mesh_lod);
-            const uint32_t lod_count = mi_hdr.z;
-            const uint32_t li = min(lod, lod_count - 1u) & 7u;
-            uint2 L = make_uint2(lods[0].x, lods[0].y);
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-                if (li == 2u * k) L = make_uint2(lods[k].x, lods[k].y);
-                if (li == 2u * k + 1u) L = make_uint2(lods[k].z, lods[k].w);
+        if (kDeferWait) {
+            if (visible) {
+                probe = occlusion_project(ci, s, p.hiz, hiz_lw, hiz_lh);
+                keep = !vib || mocc;
+                const uint2 L = select_lod(ci, s, mi_hdr, lods);
+                chunks = (L.y + 31u) >> 5;
+                lod_off = L.x; lod_cnt = L.y;
             }
-            chunks = (L.y + 31u) >> 5;
-            lod_off = L.x; lod_cnt = L.y;
+        } else {
+            if (pass == 2u && visible) visible = occlusion_test(ci, s, p.hiz);
+            bool should_draw = visible;
+            if (pass == 2u) should_draw = visible && (!vib || mocc);
+            if (should_draw) {
+                const uint2 L = select_lod(ci, s, mi_hdr, lods);
+                chunks = (L.y + 31u) >> 5;
+                lod_off = L.x; lod_cnt = L.y;
+            }
         }
+    }
+    if (kDeferWait) {
+        pdl_wait();                    // the Hi-Z build has completed: its texels are visible from here on
+        if (visible) visible = occlusion_sample(probe, p.hiz, hiz_lw, hiz_lh);
+        if (!(visible && keep)) chunks = lod_off = lod_cnt = 0u;
     }
     // pass 2: visibility word of these 32 draws (lanes past `count` contribute 0)
     const uint32_t vis_mask = __ballot_sync(0xFFFFFFFFu, visible);
@@ -410,10 +442,15 @@ __global__ void __launch_bounds__(kEcThreads) entity_cull_views_kernel(const __g
     ORBIT_TRACE_STAMP(p.scan.trace, 0, 7);
 }
 
-cudaError_t launch_entity_cull(const EntityCullParams& p, uint32_t n_draws, uint32_t coresident_ctas, cudaStream_t stream) {
+// defer_wait: entity_cull_kernel<., true>, for a pass-2 launch that directly follows this library's Hi-Z build on `stream`
+// (orbit_hiz_build_entity_cull_late); coresident_ctas from entity_cull_max_ctas_per_sm(defer_wait)
+cudaError_t launch_entity_cull(const EntityCullParams& p, uint32_t n_draws, uint32_t coresident_ctas, cudaStream_t stream, bool defer_wait) {
     uint32_t grid = (n_draws + kEcThreads - 1) / kEcThreads;
     if (grid == 0) grid = 1;
-    if (grid <= coresident_ctas) return launch_kernel(entity_cull_kernel<true>, dim3(grid), dim3(kEcThreads), 0, stream, p);
+    const bool flat = grid <= coresident_ctas;
+    if (defer_wait)
+        return launch_kernel(flat ? entity_cull_kernel<true, true> : entity_cull_kernel<false, true>, dim3(grid), dim3(kEcThreads), 0, stream, p);
+    if (flat) return launch_kernel(entity_cull_kernel<true>, dim3(grid), dim3(kEcThreads), 0, stream, p);
     return launch_kernel(entity_cull_kernel<false>, dim3(grid), dim3(kEcThreads), 0, stream, p);
 }
 
@@ -434,9 +471,10 @@ cudaError_t launch_entity_cull_views(const EntityViewsParams& pv, uint32_t n_dra
     return launch_entity_views_pass<0>(pv, grid, coresident_ctas, stream);
 }
 
-int entity_cull_max_ctas_per_sm() {
+int entity_cull_max_ctas_per_sm(bool defer_wait) {
     int n = 0;
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, entity_cull_kernel<true>, kEcThreads, 0);
+    if (defer_wait) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, entity_cull_kernel<true, true>, kEcThreads, 0);
+    else cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, entity_cull_kernel<true>, kEcThreads, 0);
     return n;
 }
 

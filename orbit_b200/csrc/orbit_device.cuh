@@ -138,18 +138,29 @@ ORBIT_DEV float hiz_sample(const HizDevice& hz, uint32_t lw0, uint32_t lh0, uint
     return fminf(fminf(a, b), fminf(c, d));
 }
 
-// Occlusion block shared by the entity and meshlet stages. In the perspective case s.z is negated in place
-// (the entity stage's LOD distance later reads the negated value, as in the reference).
+// Occlusion block of the entity stage, in two halves: occlusion_project computes everything up to the pyramid level and
+// the footprint's centre (no pyramid texel is read), occlusion_sample samples the level (hiz_sample) and compares. occlusion_test is the two
+// in a row. In the perspective case s.z is negated in place (the entity stage's LOD distance later reads the negated
+// value, as in the reference).
+struct HizProbe {
+    bool sample;     // false: visible without a texel (sphere not entirely beyond the near plane, unknown projection type)
+    float depth;     // the sphere's nearest depth
+    uint32_t lvl;    // pyramid level to sample
+    float u, v;      // footprint centre
+};
+
 // kProj: 0 perspective, 1 orthographic, -1 decided at run time from ci.projection_type.
 template <int kProj = -1>
-ORBIT_DEV bool occlusion_test(const OrbitCullInfo& ci, Sphere& s, const HizDevice& hz, const uint32_t hiz_lw, const uint32_t hiz_lh) {
+ORBIT_DEV HizProbe occlusion_project(const OrbitCullInfo& ci, Sphere& s, const HizDevice& hz, const uint32_t hiz_lw, const uint32_t hiz_lh) {
+    HizProbe q;
+    q.sample = false;
     float ax, ay, az, aw, depth;
     const uint32_t proj = kProj >= 0 ? (uint32_t)kProj : ci.projection_type;
     if (proj == 0u) {
         float zp = -s.z;
         s.z = zp;
         bool cullable = zp >= fma_(s.r_model, s.s, ci.z_near);
-        if (!cullable) return true;  // visible stays true; nothing below has side effects
+        if (!cullable) return q;  // visible stays true; nothing below has side effects
         float P00 = ci.p00_or_width_recip_x2, P11 = ci.p11_or_height_recip_x2;
         float r = s.r, nr = -s.r;
         float c0 = -s.x, c1 = -zp;
@@ -179,18 +190,29 @@ ORBIT_DEV bool occlusion_test(const OrbitCullInfo& ci, Sphere& s, const HizDevic
         float k = fdiv(1.0f, sub(ci.z_far, ci.z_near));
         depth = mul(k, add(fma_(s.r_model, s.s, s.z), ci.z_far));
     } else {
-        return true;
+        return q;
     }
     float W = mul(sub(az, ax), (float)hz.width);
     float H = mul(sub(aw, ay), (float)hz.height);
     float u = mul(add(ax, az), 0.5f), v = mul(add(ay, aw), 0.5f);
     uint32_t lvl = hiz_level(fmaxf(W, H), hz.levels);
-    float sampled = hiz_sample(hz, hiz_lw, hiz_lh, lvl, u, v);
-    return depth >= sampled;
+    q.sample = true;
+    q.depth = depth; q.lvl = lvl; q.u = u; q.v = v;
+    return q;
+}
+ORBIT_DEV bool occlusion_sample(const HizProbe& q, const HizDevice& hz, const uint32_t hiz_lw, const uint32_t hiz_lh) {
+    if (!q.sample) return true;
+    float sampled = hiz_sample(hz, hiz_lw, hiz_lh, q.lvl, q.u, q.v);
+    return q.depth >= sampled;
 }
 template <int kProj = -1>
+ORBIT_DEV bool occlusion_test(const OrbitCullInfo& ci, Sphere& s, const HizDevice& hz, const uint32_t hiz_lw, const uint32_t hiz_lh) {
+    return occlusion_sample(occlusion_project<kProj>(ci, s, hz, hiz_lw, hiz_lh), hz, hiz_lw, hiz_lh);
+}
+ORBIT_DEV uint32_t hiz_log2(uint32_t n) { return 31u - (uint32_t)__clz((int)max(n, 1u)); }   // of a level-0 side (a power of two)
+template <int kProj = -1>
 ORBIT_DEV bool occlusion_test(const OrbitCullInfo& ci, Sphere& s, const HizDevice& hz) {
-    return occlusion_test<kProj>(ci, s, hz, 31u - (uint32_t)__clz((int)max(hz.width, 1u)), 31u - (uint32_t)__clz((int)max(hz.height, 1u)));
+    return occlusion_test<kProj>(ci, s, hz, hiz_log2(hz.width), hiz_log2(hz.height));
 }
 
 // Loads that are issued where they are written. In the latency-bound kernels the order of the independent loads is

@@ -162,11 +162,11 @@ cudaError_t launch_record_masks_put(const uint4* src, const uint32_t* dispatch_w
 cudaError_t launch_meshlet_emit(const MeshletCullParams& p, int emit_grid, cudaStream_t s);
 cudaError_t launch_meshlet_emit_pair(const MeshletCullParams& a, const MeshletCullParams& b, int emit_grid, cudaStream_t s);
 cudaError_t launch_draws_from_masks(const MeshletCullParams& p, uint32_t* header, int grid, int emit_grid, cudaStream_t s);
-cudaError_t launch_entity_cull(const EntityCullParams&, uint32_t n_draws, uint32_t coresident_ctas, cudaStream_t);
+cudaError_t launch_entity_cull(const EntityCullParams&, uint32_t n_draws, uint32_t coresident_ctas, cudaStream_t, bool defer_wait = false);
 cudaError_t launch_entity_cull_views(const EntityViewsParams&, uint32_t n_draws, uint32_t coresident_ctas, cudaStream_t);
 cudaError_t launch_meshlet_cull_views(const MeshletViewsParams&, int grid, int emit_grid_per_view, cudaStream_t);
 int meshlet_cull_views_max_ctas_per_sm(const OrbitCullInfo&);
-int entity_cull_max_ctas_per_sm();
+int entity_cull_max_ctas_per_sm(bool defer_wait);
 int entity_cull_views_max_ctas_per_sm(uint32_t occlusion_pass);
 cudaError_t launch_hiz_build(const HizBuildParams&, cudaStream_t);
 cudaError_t launch_hiz_build_views(const HizBuildViewsParams&, cudaStream_t);

@@ -426,6 +426,18 @@ class PreparedFrame:
         if rc:
             raise RuntimeError("orbit_hiz_build: %d" % rc)
 
+    def hiz_entity_late(self, s=None):
+        """hiz() followed by entity(True) — with a fused frame, by entity_late_main() — as ONE call
+        (orbit_hiz_build_entity_cull_late): the same buffers, but the entity kernel's work that does not read the pyramid runs
+        under the build."""
+        C, lib, p = self._C, self._lib, self._ptr
+        g_main, main_dispatch = (C.byref(self.g_early), p(self.main_dispatch)) if self.fused else (None, None)
+        rc = lib.orbit_hiz_build_entity_cull_late(self.context._h, self.vstate.depth_pyramid._h, p(self.depth), self._hw[0], self._hw[1],
+                                                  C.byref(self.g_late), g_main, C.byref(self.sb_late), p(self.late_dispatch), main_dispatch,
+                                                  self.rcap, s or self._stream())
+        if rc:
+            raise RuntimeError("orbit_hiz_build_entity_cull_late: %d" % rc)
+
     def launch(self, overlap_main_entity=False):
         """The frame's stage calls in dependency order. `overlap_main_entity`: the MAIN pass's entity stage depends only on the
         entity visibility bits the LATE entity stage wrote, not on the late MESHLET stage, so it may be forked onto a side stream
@@ -434,11 +446,11 @@ class PreparedFrame:
         with a static tile split — ends 7 us later when 40 SMs start a third of their CTAs late, so the frame gains nothing
         (104.5 vs 104.2 us); off by default, kept because it is bit-identical and pays off when the late pass is small."""
         s = self._stream()
-        self.entity(False, s); self.meshlet(False, s); self.hiz(s)
+        self.entity(False, s); self.meshlet(False, s)
+        self.hiz_entity_late(s)
         if self.fused:
-            self.entity_late_main(s); self.meshlet_late_main(s)
+            self.meshlet_late_main(s)
             return
-        self.entity(True, s)
         if not self.main_pass:
             self.meshlet(True, s)
             return

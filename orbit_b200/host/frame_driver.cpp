@@ -92,15 +92,16 @@ int orbit_host_frame_loop(orbit_ctx* ctx, const OrbitHostFrame* frames, uint32_t
         OR_OK(orbit_entity_cull(ctx, &f.cull_early, &f.scene_early, nullptr, f.early_dispatch, f.capacity_records, s_comp));
         OR_OK(orbit_meshlet_cull(ctx, &f.cull_early, &f.scene_early, nullptr, f.early_dispatch, f.capacity_records, f.early_draws,
                                  f.capacity_draws, nullptr, s_comp));
-        OR_OK(orbit_hiz_build(ctx, f.hiz, f.depth, f.width, f.height, s_comp));
+        // Hi-Z build + LATE entity stage in one call (the entity kernel's pyramid-independent work runs under the build)
         if (orbit_cull_pair_compatible(&f.cull_late, &f.cull_early)) {
             // LATE + MAIN (= pass 1 again, the EARLY CullInfo) fused: one entity kernel, one test kernel, an emit kernel per list
-            OR_OK(orbit_entity_cull_late_main(ctx, &f.cull_late, &f.cull_early, &f.scene_late, f.hiz, f.late_dispatch, f.main_dispatch,
-                                              f.capacity_records, s_comp));
+            OR_OK(orbit_hiz_build_entity_cull_late(ctx, f.hiz, f.depth, f.width, f.height, &f.cull_late, &f.cull_early, &f.scene_late,
+                                                   f.late_dispatch, f.main_dispatch, f.capacity_records, s_comp));
             OR_OK(orbit_meshlet_cull_late_main(ctx, &f.cull_late, &f.cull_early, &f.scene_late, f.hiz, f.late_dispatch, f.capacity_records,
                                                f.late_draws, f.main_draws, f.capacity_draws, nullptr, nullptr, s_comp));
         } else {
-            OR_OK(orbit_entity_cull(ctx, &f.cull_late, &f.scene_late, f.hiz, f.late_dispatch, f.capacity_records, s_comp));
+            OR_OK(orbit_hiz_build_entity_cull_late(ctx, f.hiz, f.depth, f.width, f.height, &f.cull_late, nullptr, &f.scene_late,
+                                                   f.late_dispatch, nullptr, f.capacity_records, s_comp));
             OR_OK(orbit_meshlet_cull(ctx, &f.cull_late, &f.scene_late, f.hiz, f.late_dispatch, f.capacity_records, f.late_draws,
                                      f.capacity_draws, nullptr, s_comp));
             OR_OK(orbit_entity_cull(ctx, &f.cull_early, &f.scene_early, nullptr, f.main_dispatch, f.capacity_records, s_comp));   // MAIN = pass 1 again

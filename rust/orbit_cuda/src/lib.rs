@@ -147,6 +147,10 @@ extern "C" {
                                         hiz: *const orbit_hiz, late_dispatch_buffer: *const c_void, capacity_records: u64,
                                         late_draw_command_buffer: *mut c_void, main_draw_command_buffer: *mut c_void, capacity_draws: u64,
                                         late_task_payloads: *mut c_void, main_task_payloads: *mut c_void, stream: *mut c_void) -> c_int;
+    pub fn orbit_hiz_build_entity_cull_late(ctx: *mut orbit_ctx, hiz: *mut orbit_hiz, depth: *const f32, depth_width: u32, depth_height: u32,
+                                            late: *const OrbitCullInfo, main_pass: *const OrbitCullInfo, scene: *const OrbitSceneBuffers,
+                                            late_dispatch_buffer: *mut c_void, main_dispatch_buffer: *mut c_void, capacity_records: u64,
+                                            stream: *mut c_void) -> c_int;
     pub fn orbit_entity_cull_views(ctx: *mut orbit_ctx, culls: *const OrbitCullInfo, n_views: u32, scene: *const OrbitSceneBuffers,
                                    dispatch_buffers: *const *mut c_void, capacity_records: u64, stream: *mut c_void) -> c_int;
     pub fn orbit_meshlet_cull_views(ctx: *mut orbit_ctx, culls: *const OrbitCullInfo, n_views: u32, scene: *const OrbitSceneBuffers,
@@ -281,5 +285,17 @@ impl DepthPyramid {
         Ok(())
     }
     pub fn get_current(&self) -> *const orbit_hiz { self.hiz }
+    /// update() followed by the LATE cull's create_meshlet_dispatch_command (`late`: pass 2 against this pyramid) or, with
+    /// `main_pass`, by the entity half of create_late_and_main_commands, in one call: the same buffers, with the entity kernel's
+    /// pyramid-independent work under the build (orbit_hiz_build_entity_cull_late). `main_dispatch_buffer` is null without `main_pass`.
+    pub unsafe fn update_and_cull_late(&mut self, ctx: &Context, depth_buffer: *const f32, late: &OrbitCullInfo, main_pass: Option<&OrbitCullInfo>,
+                                       scene: &OrbitSceneBuffers, late_dispatch_buffer: *mut c_void, main_dispatch_buffer: *mut c_void,
+                                       capacity_records: u64, stream: *mut c_void) -> Result<(), Error> {
+        let main_ptr = main_pass.map_or(std::ptr::null(), |m| m as *const OrbitCullInfo);
+        check(orbit_hiz_build_entity_cull_late(ctx.0, self.hiz, depth_buffer, self.size[0], self.size[1], late, main_ptr, scene,
+                                               late_dispatch_buffer, main_dispatch_buffer, capacity_records, stream))?;
+        self.usable = true;
+        Ok(())
+    }
 }
 impl Drop for DepthPyramid { fn drop(&mut self) { unsafe { orbit_hiz_destroy(self.hiz) } } }
