@@ -285,6 +285,47 @@ int orbit_light_cluster(orbit_ctx* ctx, const OrbitClusterParams* params, const 
                         void* offset_count_image, void* light_index_list, uint64_t capacity_indices,
                         void* stream);
 
+/* ---- depth from an image (a depth attachment imported from Vulkan) ------------------------------------------------------
+ * An optimally tiled VkImage imported with cudaImportExternalMemory can only be mapped as a CUDA (mipmapped) array, not as a
+ * linear pointer. orbit_depth_image wraps such an array, so the depth-reading stages take it directly: no image-to-buffer
+ * copy pass per frame and camera. Each *_image call writes byte for byte what its linear twin writes for the same depth values.
+ *
+ * orbit_depth_image_wrap: `cuda_array` is a caller-owned cudaArray_t (passed as void*), e.g. level 0 of a mipmapped array
+ * mapped from an imported VkImage (cudaGetMipmappedArrayLevel(&a, mm, 0)), or one from cudaMallocArray. It must be 2-D
+ * (extent depth 0, not layered, not a cubemap), at least 1 x 1, with one 32-bit cudaChannelFormatKindFloat channel; the
+ * handle records its width and height. The call creates its own texture object on the array (unnormalised coordinates,
+ * point filtering, clamp addressing, element read mode) and allocates nothing on the device. Anything else, a NULL array
+ * included, and an array the context's device cannot query, is ORBIT_ERR_INVALID_ARGUMENT. The array stays the caller's.
+ * orbit_depth_image_destroy releases the texture object, never the array. Destroying an image, or freeing its array, while
+ * enqueued work or a captured CUDA graph still reads it is the caller's error (as with orbit_hiz_destroy).
+ *
+ * Stage calls: every argument rule of the linear twin applies, and the image's size must equal the depth size the pyramid was
+ * created for (orbit_light_cluster_image: params->info.screen_size). A refused call (ORBIT_ERR_INVALID_ARGUMENT) launches
+ * nothing. Concurrency and CUDA-graph rules are the twin's; the texture handle travels in the kernel parameters, so a
+ * replayed graph reads the array's contents at replay time, for as long as the image lives.
+ * Synchronisation: the calls read the array on `stream`. Ordering the renderer's writes of the image before them (an
+ * imported Vulkan semaphore waited on `stream` with cudaWaitExternalSemaphoresAsync) is the caller's job. */
+typedef struct orbit_depth_image orbit_depth_image;
+int  orbit_depth_image_wrap(orbit_ctx* ctx, void* cuda_array, orbit_depth_image** out);
+void orbit_depth_image_destroy(orbit_depth_image* image);
+/* The wrapped array's width and height in texels. */
+int  orbit_depth_image_size(const orbit_depth_image* image, uint32_t* width, uint32_t* height);
+/* orbit_hiz_build with the depth read from `image`. */
+int  orbit_hiz_build_image(orbit_ctx* ctx, orbit_hiz* hiz, const orbit_depth_image* image, void* stream);
+/* orbit_hiz_build_views with depths[v] read from images[v] (all of the pyramids' depth size; a NULL entry is refused). */
+int  orbit_hiz_build_views_image(orbit_ctx* ctx, orbit_hiz* const* hizs, const orbit_depth_image* const* images,
+                                 uint32_t n_views, void* stream);
+/* orbit_hiz_build_entity_cull_late with (depth, depth_width, depth_height) replaced by `image`. */
+int  orbit_hiz_build_image_entity_cull_late(orbit_ctx* ctx, orbit_hiz* hiz, const orbit_depth_image* image,
+                                            const OrbitCullInfo* late, const OrbitCullInfo* main_pass /* nullable */,
+                                            const OrbitSceneBuffers* scene, void* late_dispatch_buffer,
+                                            void* main_dispatch_buffer /* nullable */, uint64_t capacity_records, void* stream);
+/* orbit_light_cluster with `depth` replaced by `image`. */
+int  orbit_light_cluster_image(orbit_ctx* ctx, const OrbitClusterParams* params, const orbit_depth_image* image,
+                               const void* lights, void* tile_masks, void* depth_bounds, void* unique_clusters,
+                               void* offset_count_image, void* light_index_list, uint64_t capacity_indices,
+                               void* stream);
+
 /* ---- SceneData::update_scene (scene.rs:404-492), the per-frame producer of the entity buffers the culling path
  *      reads (SURVEY §8f item 3). For every entity with a mesh, in entity order: instance_index = running count,
  *      GpuEntityData {model_matrix = Mat4::from_scale_rotation_translation(scale, orientation, position),

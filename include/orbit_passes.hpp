@@ -161,6 +161,8 @@ public:
         check(orbit_hiz_create(ctx_, width, height, &hiz_), "DepthPyramid::resize"); w_ = width; h_ = height;
     }
     void update(const float* depth_buffer, void* stream) { check(orbit_hiz_build(ctx_, hiz_, depth_buffer, w_, h_, stream), "DepthPyramid::update"); usable = true; }
+    // the depth attachment as a wrapped CUDA array (orbit_depth_image_wrap), e.g. imported from Vulkan
+    void update(const orbit_depth_image* depth_image, void* stream) { check(orbit_hiz_build_image(ctx_, hiz_, depth_image, stream), "DepthPyramid::update"); usable = true; }
     orbit_hiz* get_current() const { return hiz_; }
     bool usable = false;
 private:

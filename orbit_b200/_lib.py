@@ -72,6 +72,15 @@ PROTOTYPES = {
     "orbit_peer_close": (C.c_int, [C.c_void_p, C.c_void_p]),
     "orbit_peer_free": (None, [C.c_void_p, C.c_void_p]),
     "orbit_device_copy": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p]),
+    "orbit_depth_image_wrap": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(C.c_void_p)]),
+    "orbit_depth_image_destroy": (None, [C.c_void_p]),
+    "orbit_depth_image_size": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint32), C.POINTER(C.c_uint32)]),
+    "orbit_hiz_build_image": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "orbit_hiz_build_views_image": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_uint32, C.c_void_p]),
+    "orbit_hiz_build_image_entity_cull_late": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(L.CullInfo), C.POINTER(L.CullInfo),
+                                                         C.POINTER(L.SceneBuffers), C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p]),
+    "orbit_light_cluster_image": (C.c_int, [C.c_void_p, C.POINTER(L.ClusterParams), C.c_void_p, C.c_void_p, C.c_void_p,
+                                            C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p]),
 }
 
 _lib = None

@@ -105,6 +105,13 @@ struct orbit_hiz {
     int device;
 };
 
+// A caller's 2-D float CUDA array behind the texture object the *_image stage calls read it through
+struct orbit_depth_image {
+    cudaTextureObject_t tex;
+    uint32_t width, height;
+    int device;
+};
+
 // Outgrown scratch is retired, not freed (see orbit_ctx::retired). With doubling capacities a context retires a handful of
 // buffers in its life; if the list ever fills up the oldest entries are freed after one device synchronisation.
 static int retire(orbit_ctx* c, void* p) {
@@ -408,12 +415,13 @@ int orbit_hiz_build(orbit_ctx* c, orbit_hiz* h, const float* depth, uint32_t dw,
 
 // Batched form: one launch, a row of CTAs per pyramid. Pyramid v's ticket is counter word 40 + v (words 40..55 are used by
 // nothing else and were zeroed with the rest at context creation; each row's last CTA re-zeroes its own).
-int orbit_hiz_build_views(orbit_ctx* c, orbit_hiz* const* hizs, const float* const* depths, uint32_t n_views, uint32_t dw, uint32_t dh,
-                          void* stream) {
-    if (!c || !hizs || !depths || n_views == 0u || n_views > ORBIT_MAX_BATCH_VIEWS) return ORBIT_ERR_INVALID_ARGUMENT;
+// Depth v comes from depths[v], or from images[v] when depths is NULL (images already checked, each dw x dh).
+static int hiz_build_views(orbit_ctx* c, orbit_hiz* const* hizs, const float* const* depths, const orbit_depth_image* const* images,
+                           uint32_t n_views, uint32_t dw, uint32_t dh, void* stream) {
+    if (!c || !hizs || n_views == 0u || n_views > ORBIT_MAX_BATCH_VIEWS) return ORBIT_ERR_INVALID_ARGUMENT;
     for (uint32_t v = 0; v < n_views; ++v) {
         const orbit_hiz* h = hizs[v];
-        if (!h || !depths[v] || dw != h->depth_w || dh != h->depth_h) return ORBIT_ERR_INVALID_ARGUMENT;
+        if (!h || (depths && !depths[v]) || dw != h->depth_w || dh != h->depth_h) return ORBIT_ERR_INVALID_ARGUMENT;
         for (uint32_t u = 0; u < v; ++u) if (hizs[u]->info.texels == h->info.texels) return ORBIT_ERR_INVALID_ARGUMENT;
     }
     GUARD(c);
@@ -422,15 +430,90 @@ int orbit_hiz_build_views(orbit_ctx* c, orbit_hiz* const* hizs, const float* con
     for (uint32_t v = 0; v < n_views; ++v) {
         const orbit_hiz* h = hizs[v];
         HizBuildParams& p = pv.view[v];
-        p.depth = depths[v]; p.texels = h->info.texels; p.depth_w = dw; p.depth_h = dh;
+        if (depths) p.depth = depths[v];
+        else p.depth_tex = images[v]->tex;
+        p.texels = h->info.texels; p.depth_w = dw; p.depth_h = dh;
         p.width = h->info.width; p.height = h->info.height; p.levels = h->info.levels;
         for (int i = 0; i < ORBIT_HIZ_MAX_LEVELS; ++i) p.level_offset[i] = h->info.level_offset[i];
         p.ticket = c->counters + 40 + v;
     }
     pv.view[0].trace = next_trace(c);
-    CK(launch_hiz_build_views(pv, (cudaStream_t)stream));
+    CK(launch_hiz_build_views(pv, (cudaStream_t)stream, depths == nullptr));
     c->launches += 1;
     return ORBIT_OK;
+}
+
+int orbit_hiz_build_views(orbit_ctx* c, orbit_hiz* const* hizs, const float* const* depths, uint32_t n_views, uint32_t dw, uint32_t dh,
+                          void* stream) {
+    if (!depths) return ORBIT_ERR_INVALID_ARGUMENT;
+    return hiz_build_views(c, hizs, depths, nullptr, n_views, dw, dh, stream);
+}
+
+// ---- depth images ------------------------------------------------------------------------------------------
+int orbit_depth_image_wrap(orbit_ctx* c, void* cuda_array, orbit_depth_image** out) {
+    if (!out) return ORBIT_ERR_INVALID_ARGUMENT;
+    *out = nullptr;
+    if (!c || !cuda_array) return ORBIT_ERR_INVALID_ARGUMENT;
+    GUARD(c);
+    const cudaArray_t a = static_cast<cudaArray_t>(cuda_array);
+    cudaChannelFormatDesc fmt{};
+    cudaExtent ext{};
+    unsigned int flags = 0;
+    cudaError_t e = cudaArrayGetInfo(&fmt, &ext, &flags, a);
+    if (e != cudaSuccess) { g_last_cuda_error = (int)e; cudaGetLastError(); return ORBIT_ERR_INVALID_ARGUMENT; }
+    if (fmt.f != cudaChannelFormatKindFloat || fmt.x != 32 || fmt.y != 0 || fmt.z != 0 || fmt.w != 0) return ORBIT_ERR_INVALID_ARGUMENT;
+    if (ext.depth != 0 || (flags & (cudaArrayLayered | cudaArrayCubemap)) != 0u) return ORBIT_ERR_INVALID_ARGUMENT;
+    if (ext.width == 0 || ext.height == 0 || ext.width > 0xFFFFFFFFull || ext.height > 0xFFFFFFFFull) return ORBIT_ERR_INVALID_ARGUMENT;
+    // the library owns the sampler, as the reference does: every setting that could change a fetched value is fixed here
+    cudaResourceDesc res{};
+    res.resType = cudaResourceTypeArray;
+    res.res.array.array = a;
+    cudaTextureDesc td{};
+    td.addressMode[0] = td.addressMode[1] = cudaAddressModeClamp;
+    td.filterMode = cudaFilterModePoint;
+    td.readMode = cudaReadModeElementType;
+    td.normalizedCoords = 0;
+    orbit_depth_image* img = new (std::nothrow) orbit_depth_image();
+    if (!img) return ORBIT_ERR_OUT_OF_MEMORY;
+    e = cudaCreateTextureObject(&img->tex, &res, &td, nullptr);
+    if (e != cudaSuccess) { g_last_cuda_error = (int)e; delete img; return ORBIT_ERR_CUDA; }
+    img->width = (uint32_t)ext.width; img->height = (uint32_t)ext.height; img->device = c->device;
+    *out = img;
+    return ORBIT_OK;
+}
+
+void orbit_depth_image_destroy(orbit_depth_image* img) {
+    if (!img) return;
+    { DeviceGuard guard(img->device); cudaDestroyTextureObject(img->tex); }
+    delete img;
+}
+
+int orbit_depth_image_size(const orbit_depth_image* img, uint32_t* w, uint32_t* h) {
+    if (!img || !w || !h) return ORBIT_ERR_INVALID_ARGUMENT;
+    *w = img->width; *h = img->height;
+    return ORBIT_OK;
+}
+
+static bool image_ok(const orbit_ctx* c, const orbit_depth_image* img, uint32_t w, uint32_t h) {
+    return img && img->device == c->device && img->width == w && img->height == h;
+}
+
+int orbit_hiz_build_image(orbit_ctx* c, orbit_hiz* h, const orbit_depth_image* img, void* stream) {
+    if (!c || !h || !image_ok(c, img, h->depth_w, h->depth_h)) return ORBIT_ERR_INVALID_ARGUMENT;
+    GUARD(c);
+    HizBuildParams p = hiz_build_params(c, h, nullptr, img->width, img->height);
+    p.depth_tex = img->tex;
+    CK(launch_hiz_build(p, (cudaStream_t)stream, true));
+    c->launches += 1;
+    return ORBIT_OK;
+}
+
+int orbit_hiz_build_views_image(orbit_ctx* c, orbit_hiz* const* hizs, const orbit_depth_image* const* images, uint32_t n_views,
+                                void* stream) {
+    if (!c || !hizs || !images || n_views == 0u || n_views > ORBIT_MAX_BATCH_VIEWS || !images[0]) return ORBIT_ERR_INVALID_ARGUMENT;
+    const uint32_t dw = images[0]->width, dh = images[0]->height;
+    for (uint32_t v = 0; v < n_views; ++v) if (!image_ok(c, images[v], dw, dh)) return ORBIT_ERR_INVALID_ARGUMENT;
+    return hiz_build_views(c, hizs, nullptr, images, n_views, dw, dh, stream);
 }
 
 // ---- entity stage ----------------------------------------------------------------------------------------
@@ -573,10 +656,12 @@ int orbit_entity_cull_late_main(orbit_ctx* c, const OrbitCullInfo* late, const O
 // made the C2 frame 1.3 us slower instead of 2.6 us faster (entity CTAs beside a running build slow both). Every argument is checked, and
 // the scan descriptors are grown (ensure_status may enqueue a memset), before the build is launched: a refused call launches
 // nothing, and nothing but the build sits between the two kernels on the stream.
-int orbit_hiz_build_entity_cull_late(orbit_ctx* c, orbit_hiz* h, const float* depth, uint32_t dw, uint32_t dh, const OrbitCullInfo* late,
-                                     const OrbitCullInfo* main_pass, const OrbitSceneBuffers* scene, void* late_dispatch_buffer,
-                                     void* main_dispatch_buffer, uint64_t capacity_records, void* stream) {
-    if (!hiz_build_args_ok(c, h, depth, dw, dh) || !late || late->occlusion_pass != 2u) return ORBIT_ERR_INVALID_ARGUMENT;
+// depth_ok: the depth source was checked against h (orbit_hiz_build's or orbit_hiz_build_image's rule); the build reads `image`
+// when it is not NULL, else `depth`.
+static int hiz_build_entity_late(orbit_ctx* c, orbit_hiz* h, bool depth_ok, const float* depth, const orbit_depth_image* image,
+                                 const OrbitCullInfo* late, const OrbitCullInfo* main_pass, const OrbitSceneBuffers* scene,
+                                 void* late_dispatch_buffer, void* main_dispatch_buffer, uint64_t capacity_records, void* stream) {
+    if (!depth_ok || !late || late->occlusion_pass != 2u) return ORBIT_ERR_INVALID_ARGUMENT;
     if (main_pass ? !late_main_args_ok(late, main_pass, late_dispatch_buffer, main_dispatch_buffer) : main_dispatch_buffer != nullptr)
         return ORBIT_ERR_INVALID_ARGUMENT;
     uint32_t begin, end;
@@ -585,9 +670,26 @@ int orbit_hiz_build_entity_cull_late(orbit_ctx* c, orbit_hiz* h, const float* de
     GUARD(c);
     rc = ensure_status(c, (size_t)(end - begin + 255u) / 256u + 1u, (cudaStream_t)stream);
     if (rc != ORBIT_OK) return rc;
-    CK(launch_hiz_build(hiz_build_params(c, h, depth, dw, dh), (cudaStream_t)stream));
+    HizBuildParams p = hiz_build_params(c, h, depth, h->depth_w, h->depth_h);
+    if (image) p.depth_tex = image->tex;
+    CK(launch_hiz_build(p, (cudaStream_t)stream, image != nullptr));
     c->launches += 1;
     return entity_launch(c, late, scene, h, late_dispatch_buffer, main_dispatch_buffer, capacity_records, begin, end, stream, true);
+}
+
+int orbit_hiz_build_entity_cull_late(orbit_ctx* c, orbit_hiz* h, const float* depth, uint32_t dw, uint32_t dh, const OrbitCullInfo* late,
+                                     const OrbitCullInfo* main_pass, const OrbitSceneBuffers* scene, void* late_dispatch_buffer,
+                                     void* main_dispatch_buffer, uint64_t capacity_records, void* stream) {
+    return hiz_build_entity_late(c, h, hiz_build_args_ok(c, h, depth, dw, dh), depth, nullptr, late, main_pass, scene, late_dispatch_buffer,
+                                 main_dispatch_buffer, capacity_records, stream);
+}
+
+int orbit_hiz_build_image_entity_cull_late(orbit_ctx* c, orbit_hiz* h, const orbit_depth_image* image, const OrbitCullInfo* late,
+                                           const OrbitCullInfo* main_pass, const OrbitSceneBuffers* scene, void* late_dispatch_buffer,
+                                           void* main_dispatch_buffer, uint64_t capacity_records, void* stream) {
+    const bool depth_ok = c && h && image_ok(c, image, h->depth_w, h->depth_h);
+    return hiz_build_entity_late(c, h, depth_ok, nullptr, image, late, main_pass, scene, late_dispatch_buffer, main_dispatch_buffer,
+                                 capacity_records, stream);
 }
 
 // ---- meshlet stage ---------------------------------------------------------------------------------------
@@ -969,12 +1071,14 @@ int orbit_meshlet_cull_views_occlusion(orbit_ctx* c, const OrbitCullInfo* culls,
 }
 
 // ---- clustered lights ------------------------------------------------------------------------------------
-int orbit_light_cluster(orbit_ctx* c, const OrbitClusterParams* params, const float* depth, const void* lights,
-                        void* tile_masks, void* depth_bounds, void* unique_clusters, void* offset_count_image,
-                        void* light_index_list, uint64_t capacity_indices, void* stream) {
-    if (!c || !params || !depth || !tile_masks || !depth_bounds || !unique_clusters || !offset_count_image || !light_index_list)
+// Depth from `image` when it is not NULL (orbit_light_cluster_image), else from `depth`.
+static int light_cluster(orbit_ctx* c, const OrbitClusterParams* params, const float* depth, const orbit_depth_image* image,
+                         const void* lights, void* tile_masks, void* depth_bounds, void* unique_clusters, void* offset_count_image,
+                         void* light_index_list, uint64_t capacity_indices, void* stream) {
+    if (!c || !params || !(depth || image) || !tile_masks || !depth_bounds || !unique_clusters || !offset_count_image || !light_index_list)
         return ORBIT_ERR_INVALID_ARGUMENT;
     const OrbitClusterCullInfo& ci = params->info;
+    if (image && !image_ok(c, image, ci.screen_size[0], ci.screen_size[1])) return ORBIT_ERR_INVALID_ARGUMENT;
     const uint64_t cx = ci.cluster_count[0], cy = ci.cluster_count[1], cz = ci.cluster_count[2];
     if (cx == 0 || cy == 0 || cz == 0 || cx * cy * cz > 0x7FFFFFFFull || ci.tile_size_px == 0) return ORBIT_ERR_INVALID_ARGUMENT;
     if (ci.screen_size[0] == 0 || ci.screen_size[1] == 0) return ORBIT_ERR_INVALID_ARGUMENT;
@@ -994,7 +1098,9 @@ int orbit_light_cluster(orbit_ctx* c, const OrbitClusterParams* params, const fl
     if (rc != ORBIT_OK) return rc;
     ClusterParams p{};
     p.info = ci; p.z_scale = params->z_scale; p.z_bias = params->z_bias;
-    p.depth = depth; p.lights = (const uint8_t*)lights; p.light_view = c->light_view;
+    if (image) p.depth_tex = image->tex;
+    else p.depth = depth;
+    p.lights = (const uint8_t*)lights; p.light_view = c->light_view;
     p.tile_masks = (uint32_t*)tile_masks; p.depth_bounds = (uint32_t*)depth_bounds;
     p.unique_clusters = (uint32_t*)unique_clusters; p.offset_count_image = (uint32_t*)offset_count_image;
     p.light_index_words = (uint32_t*)light_index_list; p.overflow_flag = &c->status_dev->light_index_overflow;
@@ -1010,7 +1116,7 @@ int orbit_light_cluster(orbit_ctx* c, const OrbitClusterParams* params, const fl
     uint64_t grid = (warps + 7u) / 8u;
     const uint64_t cap_grid = (uint64_t)c->sm_count * 8u;
     if (grid > cap_grid) grid = cap_grid;
-    CK(launch_mark_active(p, (int)grid, s));
+    CK(launch_mark_active(p, (int)grid, s, image != nullptr));
     p.scan = next_scan(c);
     CK(launch_compact_clusters(p, s));
     if (light_parallel) {
@@ -1033,6 +1139,22 @@ int orbit_light_cluster(orbit_ctx* c, const OrbitClusterParams* params, const fl
         c->launches += (L ? 4 : 3);
     }
     return ORBIT_OK;
+}
+
+int orbit_light_cluster(orbit_ctx* c, const OrbitClusterParams* params, const float* depth, const void* lights,
+                        void* tile_masks, void* depth_bounds, void* unique_clusters, void* offset_count_image,
+                        void* light_index_list, uint64_t capacity_indices, void* stream) {
+    if (!depth) return ORBIT_ERR_INVALID_ARGUMENT;
+    return light_cluster(c, params, depth, nullptr, lights, tile_masks, depth_bounds, unique_clusters, offset_count_image,
+                         light_index_list, capacity_indices, stream);
+}
+
+int orbit_light_cluster_image(orbit_ctx* c, const OrbitClusterParams* params, const orbit_depth_image* image, const void* lights,
+                              void* tile_masks, void* depth_bounds, void* unique_clusters, void* offset_count_image,
+                              void* light_index_list, uint64_t capacity_indices, void* stream) {
+    if (!image) return ORBIT_ERR_INVALID_ARGUMENT;
+    return light_cluster(c, params, nullptr, image, lights, tile_masks, depth_bounds, unique_clusters, offset_count_image,
+                         light_index_list, capacity_indices, stream);
 }
 
 int orbit_draws_scatter(orbit_ctx* c, const void* src, uint64_t src_capacity_draws, void* dst, uint32_t dst_first, uint32_t total_count,

@@ -13,6 +13,9 @@
 // owns two adjacent columns of each, so levels 1..3 are reduced in registers + warp shuffles, levels 4..6 by
 // one warp through a 8x8 shared-memory tile. The last CTA to finish (atomic ticket) reduces the remaining
 // small levels out of L2. Pyramids smaller than 64 in a dimension take the generic tail path only.
+//
+// Depth source: every kernel exists twice, for a linear buffer (HizBuildParams::depth) and for a depth image
+// (HizBuildParams::depth_tex, orbit_*_image). Only the level-0 loads differ; the footprint arithmetic is the same.
 #include "params.cuh"
 
 namespace orbit {
@@ -21,6 +24,7 @@ namespace orbit {
 __device__ __forceinline__ float ld_cg(const float* p) { return __ldcg(p); }
 
 // Generic level-by-level reduction of levels [first, levels) by ONE CTA (reads level first-1 from global / L2).
+template <bool kImage>
 __device__ void hiz_tail(const HizBuildParams& p, uint32_t first) {
     for (uint32_t l = first; l < p.levels; ++l) {
         const uint32_t w = max(p.width >> l, 1u), h = max(p.height >> l, 1u);
@@ -31,6 +35,11 @@ __device__ void hiz_tail(const HizBuildParams& p, uint32_t first) {
                 int x0, x1, y0, y1;
                 footprint(fdiv(add((float)x, 0.5f), (float)w), p.depth_w, x0, x1);
                 footprint(fdiv(add((float)y, 0.5f), (float)h), p.depth_h, y0, y1);
+                if constexpr (kImage) {
+                    const cudaTextureObject_t t = p.depth_tex;
+                    dst[i] = fminf(fminf(depth_texel(t, x0, y0), depth_texel(t, x1, y0)), fminf(depth_texel(t, x0, y1), depth_texel(t, x1, y1)));
+                    continue;
+                }
                 const float* r0 = p.depth + (size_t)y0 * p.depth_w;
                 const float* r1 = p.depth + (size_t)y1 * p.depth_w;
                 dst[i] = fminf(fminf(__ldg(r0 + x0), __ldg(r0 + x1)), fminf(__ldg(r1 + x0), __ldg(r1 + x1)));
@@ -79,10 +88,15 @@ __device__ void hiz_tail_smem(const HizBuildParams& p, uint32_t first, float* s_
 
 __global__ void __launch_bounds__(256) hiz_small_kernel(const __grid_constant__ HizBuildParams p) {
     pdl_wait();
-    hiz_tail(p, 0u);
+    hiz_tail<false>(p, 0u);
+}
+__global__ void __launch_bounds__(256) hiz_small_image_kernel(const __grid_constant__ HizBuildParams p) {
+    pdl_wait();
+    hiz_tail<true>(p, 0u);
 }
 
 // One pyramid, one CTA per 64x64 tile of level 0 (blockIdx.x); the batched kernel runs one row of the grid per pyramid.
+template <bool kImage>
 __device__ __forceinline__ void hiz_build_body(const HizBuildParams& p) {
     __shared__ float s_l3[8][8];
     __shared__ bool s_last;
@@ -100,7 +114,35 @@ __device__ __forceinline__ void hiz_build_body(const HizBuildParams& p) {
     footprint(fdiv(add((float)(x_a + 1u), 0.5f), (float)p.width), p.depth_w, xb0, xb1);
     const uint32_t y_base = ty * 64u + warp * 8u;
     float va[8], vb[8];
-    {
+    if constexpr (kImage) {
+        // The same 64 texels as below, fetched from the depth image. The rows of the eight footprints, in order y0[0], y1[0],
+        // y0[1], .. (warp-uniform), repeat the row before whenever the depth is barely taller than the level (1080 -> 1024
+        // rows: 9 distinct of 16): a repeated row is not fetched again (predicated off) but copied once every fetch has left.
+        int ys[16];
+#pragma unroll
+        for (int r = 0; r < 8; ++r) footprint(fdiv(add((float)(y_base + r), 0.5f), (float)p.height), p.depth_h, ys[2 * r], ys[2 * r + 1]);
+        const cudaTextureObject_t tex = p.depth_tex;
+        const int xs[4] = {xa0, xa1, xb0, xb1};
+        float t[16][4];
+#pragma unroll
+        for (int s = 0; s < 16; ++s) {
+            const bool fresh = s == 0 || ys[s] != ys[s - 1];
+#pragma unroll
+            for (int c = 0; c < 4; ++c) t[s][c] = depth_texel_if(tex, xs[c], ys[s], fresh);
+        }
+#pragma unroll
+        for (int s = 1; s < 16; ++s) {
+            if (ys[s] == ys[s - 1]) {
+#pragma unroll
+                for (int c = 0; c < 4; ++c) t[s][c] = t[s - 1][c];
+            }
+        }
+#pragma unroll
+        for (int r = 0; r < 8; ++r) {
+            va[r] = fminf(fminf(t[2 * r][0], t[2 * r][1]), fminf(t[2 * r + 1][0], t[2 * r + 1][1]));
+            vb[r] = fminf(fminf(t[2 * r][2], t[2 * r][3]), fminf(t[2 * r + 1][2], t[2 * r + 1][3]));
+        }
+    } else {
         // All 64 texel loads of the thread leave back to back, before any of them is consumed: left to the compiler, the loads of
         // a row were issued only when the row before had been reduced (two rows in flight: four to five dependent DRAM round
         // trips for the tile, "level0 loaded" 4.9 us into an 8 us kernel). `asm volatile` keeps the loads in program order.
@@ -198,34 +240,42 @@ __device__ __forceinline__ void hiz_build_body(const HizBuildParams& p) {
     if (!s_last) return;
     __threadfence();
     if ((p.width >> 6) * (p.height >> 6) <= 4096u) hiz_tail_smem(p, 7u, s_top_a, s_top_b);
-    else hiz_tail(p, 7u);
+    else hiz_tail<kImage>(p, 7u);
     ORBIT_TRACE_STAMP(p.trace, 4, 4);
 }
 
-__global__ void __launch_bounds__(256) hiz_build_kernel(const __grid_constant__ HizBuildParams p) { hiz_build_body(p); }
+__global__ void __launch_bounds__(256) hiz_build_kernel(const __grid_constant__ HizBuildParams p) { hiz_build_body<false>(p); }
+__global__ void __launch_bounds__(256) hiz_build_image_kernel(const __grid_constant__ HizBuildParams p) { hiz_build_body<true>(p); }
 
 // orbit_hiz_build_views: pyramid blockIdx.y; each has its own ticket, so each row's last CTA reduces that pyramid's top levels
-__global__ void __launch_bounds__(256) hiz_build_views_kernel(const __grid_constant__ HizBuildViewsParams pv) { hiz_build_body(pv.view[blockIdx.y]); }
+__global__ void __launch_bounds__(256) hiz_build_views_kernel(const __grid_constant__ HizBuildViewsParams pv) { hiz_build_body<false>(pv.view[blockIdx.y]); }
 __global__ void __launch_bounds__(256) hiz_small_views_kernel(const __grid_constant__ HizBuildViewsParams pv) {
     pdl_wait();
-    hiz_tail(pv.view[blockIdx.y], 0u);
+    hiz_tail<false>(pv.view[blockIdx.y], 0u);
+}
+__global__ void __launch_bounds__(256) hiz_build_views_image_kernel(const __grid_constant__ HizBuildViewsParams pv) { hiz_build_body<true>(pv.view[blockIdx.y]); }
+__global__ void __launch_bounds__(256) hiz_small_views_image_kernel(const __grid_constant__ HizBuildViewsParams pv) {
+    pdl_wait();
+    hiz_tail<true>(pv.view[blockIdx.y], 0u);
 }
 
-cudaError_t launch_hiz_build(const HizBuildParams& p, cudaStream_t stream) {
+// image: level 0 is read from p.depth_tex (a depth image) instead of p.depth
+cudaError_t launch_hiz_build(const HizBuildParams& p, cudaStream_t stream, bool image) {
     if (p.width >= 64u && p.height >= 64u && p.levels >= 7u) {
         const uint32_t grid = (p.width >> 6) * (p.height >> 6);
-        return launch_kernel(hiz_build_kernel, dim3(grid), dim3(256), 0, stream, p);
+        return launch_kernel(image ? hiz_build_image_kernel : hiz_build_kernel, dim3(grid), dim3(256), 0, stream, p);
     } else {
-        return launch_kernel(hiz_small_kernel, dim3(1), dim3(256), 0, stream, p);
+        return launch_kernel(image ? hiz_small_image_kernel : hiz_small_kernel, dim3(1), dim3(256), 0, stream, p);
     }
     return cudaGetLastError();
 }
 
-cudaError_t launch_hiz_build_views(const HizBuildViewsParams& pv, cudaStream_t stream) {
+cudaError_t launch_hiz_build_views(const HizBuildViewsParams& pv, cudaStream_t stream, bool image) {
     const HizBuildParams& p = pv.view[0];   // every pyramid of the call has this geometry
     if (p.width >= 64u && p.height >= 64u && p.levels >= 7u)
-        return launch_kernel(hiz_build_views_kernel, dim3((p.width >> 6) * (p.height >> 6), pv.n_views), dim3(256), 0, stream, pv);
-    return launch_kernel(hiz_small_views_kernel, dim3(1, pv.n_views), dim3(256), 0, stream, pv);
+        return launch_kernel(image ? hiz_build_views_image_kernel : hiz_build_views_kernel, dim3((p.width >> 6) * (p.height >> 6), pv.n_views),
+                             dim3(256), 0, stream, pv);
+    return launch_kernel(image ? hiz_small_views_image_kernel : hiz_small_views_kernel, dim3(1, pv.n_views), dim3(256), 0, stream, pv);
 }
 
 }  // namespace orbit

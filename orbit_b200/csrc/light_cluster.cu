@@ -30,7 +30,9 @@ namespace orbit {
 // lanes of one key at a time.
 constexpr uint32_t kNoKey = 0xFFFFFFFFu;
 
-__global__ void __launch_bounds__(256) mark_active_kernel(const __grid_constant__ ClusterParams p) {
+// kImage: depth from p.depth_tex (a depth image, orbit_light_cluster_image) instead of the linear buffer p.depth
+template <bool kImage>
+__device__ __forceinline__ void mark_active_body(const ClusterParams& p) {
     const OrbitClusterCullInfo& ci = p.info;
     const uint32_t W = ci.screen_size[0], H = ci.screen_size[1];
     const uint32_t cx = ci.cluster_count[0], cy = ci.cluster_count[1], cz = ci.cluster_count[2];
@@ -48,7 +50,10 @@ __global__ void __launch_bounds__(256) mark_active_kernel(const __grid_constant_
         const uint32_t x = x0 + lane;
         float dv[kRows];
 #pragma unroll
-        for (uint32_t k = 0; k < kRows; ++k) dv[k] = (x < W && y0 + k < H) ? __ldg(p.depth + (size_t)(y0 + k) * W + x) : 0.0f;
+        for (uint32_t k = 0; k < kRows; ++k) {
+            if constexpr (kImage) dv[k] = (x < W && y0 + k < H) ? depth_texel(p.depth_tex, (int)x, (int)(y0 + k)) : 0.0f;
+            else dv[k] = (x < W && y0 + k < H) ? __ldg(p.depth + (size_t)(y0 + k) * W + x) : 0.0f;
+        }
         // tile column of this lane: one (warp-uniform) integer division per step instead of one per pixel
         uint32_t tx = x0 / tile_px;
         {
@@ -121,6 +126,9 @@ __global__ void __launch_bounds__(256) mark_active_kernel(const __grid_constant_
         }
     }
 }
+
+__global__ void __launch_bounds__(256) mark_active_kernel(const __grid_constant__ ClusterParams p) { mark_active_body<false>(p); }
+__global__ void __launch_bounds__(256) mark_active_image_kernel(const __grid_constant__ ClusterParams p) { mark_active_body<true>(p); }
 
 struct Aabb3 { float lo[3], hi[3]; };
 
@@ -584,8 +592,9 @@ cudaError_t launch_light_lists(const ClusterParams& p, const uint32_t* hits, con
     return cudaGetLastError();
 }
 
-cudaError_t launch_mark_active(const ClusterParams& p, int grid, cudaStream_t s) {
-    mark_active_kernel<<<grid, 256, 0, s>>>(p);
+cudaError_t launch_mark_active(const ClusterParams& p, int grid, cudaStream_t s, bool image) {
+    if (image) mark_active_image_kernel<<<grid, 256, 0, s>>>(p);
+    else mark_active_kernel<<<grid, 256, 0, s>>>(p);
     return cudaGetLastError();
 }
 cudaError_t launch_compact_clusters(const ClusterParams& p, cudaStream_t s) {

@@ -123,6 +123,22 @@ ORBIT_DEV void footprint(float u, float wf, int hi, int& i0, int& i1) {
 
 ORBIT_DEV void footprint(float u, uint32_t w, int& i0, int& i1) { footprint(u, (float)w, (int)w - 1, i0, i1); }   // any size (depth buffer)
 
+// Depth texel (x, y) of a depth image (orbit_depth_image_wrap's texture: unnormalised, point, clamp, element type): an
+// unfiltered integer-coordinate load (TLD.LZ, the texelFetch analogue). tex2D<float> at texel centres would be a filtered
+// TEX instead. `volatile` keeps a run of these fetches in program order, like the level-0 loads of the linear source.
+ORBIT_DEV float depth_texel(cudaTextureObject_t t, int x, int y) {
+    float4 v;   // one channel: .y .z .w are not read
+    asm volatile("tex.2d.v4.f32.s32 {%0, %1, %2, %3}, [%4, {%5, %6}];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(t), "r"(x), "r"(y));
+    return v.x;
+}
+// depth_texel when `fetch` is set (a predicated load), else 0
+ORBIT_DEV float depth_texel_if(cudaTextureObject_t t, int x, int y, bool fetch) {
+    float4 v = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+    asm volatile("{ .reg .pred q; setp.ne.b32 q, %7, 0; @q tex.2d.v4.f32.s32 {%0, %1, %2, %3}, [%4, {%5, %6}]; }"
+                 : "+f"(v.x), "+f"(v.y), "+f"(v.z), "+f"(v.w) : "l"(t), "r"(x), "r"(y), "r"((int)fetch));
+    return v.x;
+}
+
 // ReduceMin sampler (device.rs:1404-1420) on level `lvl`: min of the 2x2 bilinear footprint, read through the
 // non-coherent (texture / L1) path with 32-bit texel indices.
 ORBIT_DEV float hiz_sample(const HizDevice& hz, uint32_t lw0, uint32_t lh0, uint32_t lvl, float u, float v) {

@@ -118,7 +118,10 @@ struct MeshBoundsParams {
 };
 
 struct HizBuildParams {
-    const float* depth;
+    union {                            // the kernel's template parameter picks the member (same 8 bytes, same offset)
+        const float* depth;            // linear source: depth_w x depth_h floats, row-major
+        cudaTextureObject_t depth_tex; // image source (orbit_depth_image): read with depth_texel
+    };
     float* texels;
     uint32_t depth_w, depth_h;
     uint32_t width, height, levels;
@@ -135,7 +138,10 @@ struct HizBuildViewsParams {
 struct ClusterParams {
     OrbitClusterCullInfo info;
     float z_scale, z_bias;
-    const float* depth;
+    union {                            // as in HizBuildParams: linear buffer or depth image, picked by the mark_active kernel
+        const float* depth;
+        cudaTextureObject_t depth_tex;
+    };
     const uint8_t* lights;            // OrbitLightData[]
     float4* light_view;               // scratch: (view xyz, outer_radius or +inf for non-point lights)
     float4* cluster_boxes;            // scratch (light-parallel path, else nullptr): view-space box lo / hi per compacted-list slot
@@ -168,12 +174,12 @@ cudaError_t launch_meshlet_cull_views(const MeshletViewsParams&, int grid, int e
 int meshlet_cull_views_max_ctas_per_sm(const OrbitCullInfo&);
 int entity_cull_max_ctas_per_sm(bool defer_wait);
 int entity_cull_views_max_ctas_per_sm(uint32_t occlusion_pass);
-cudaError_t launch_hiz_build(const HizBuildParams&, cudaStream_t);
-cudaError_t launch_hiz_build_views(const HizBuildViewsParams&, cudaStream_t);
+cudaError_t launch_hiz_build(const HizBuildParams&, cudaStream_t, bool image = false);
+cudaError_t launch_hiz_build_views(const HizBuildViewsParams&, cudaStream_t, bool image = false);
 cudaError_t launch_meshlet_bounds(const MeshletBoundsParams&, int grid, cudaStream_t);
 cudaError_t launch_mesh_bounds(const MeshBoundsParams&, int grid, cudaStream_t);
 cudaError_t launch_scene_update(const SceneUpdateParams&, cudaStream_t);
-cudaError_t launch_mark_active(const ClusterParams&, int grid, cudaStream_t);
+cudaError_t launch_mark_active(const ClusterParams&, int grid, cudaStream_t, bool image = false);
 cudaError_t launch_compact_clusters(const ClusterParams&, cudaStream_t);
 cudaError_t launch_light_view(const ClusterParams&, cudaStream_t);
 cudaError_t launch_light_culling(const ClusterParams&, int grid, cudaStream_t);

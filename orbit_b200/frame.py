@@ -16,7 +16,7 @@ import numpy as np
 import torch
 
 from . import layouts as L
-from .passes import (AssetGraphData, Context, CullInfo, DepthPyramid, OcclusionCullInfo, Projection, SceneGraphData,
+from .passes import (AssetGraphData, Context, CullInfo, DepthImage, DepthPyramid, OcclusionCullInfo, Projection, SceneGraphData,
                      _stream, create_meshlet_dispatch_command, create_meshlet_draw_commands)
 
 
@@ -192,24 +192,33 @@ class _ViewsPass:
 
 
 class _HizViews:
-    """orbit_hiz_build_views for the pyramids of up to MAX_BATCH_VIEWS views (one depth buffer each, all of one size)."""
+    """orbit_hiz_build_views for the pyramids of up to MAX_BATCH_VIEWS views (one depth buffer each, all of one size), or
+    orbit_hiz_build_views_image when the depth buffers are DepthImages."""
 
     def __init__(self, context, pyramids, depth_buffers):
         import ctypes as C
         from . import _lib
         self.context, self._lib, self.pyramids = context, _lib.lib(), list(pyramids)
         n = self.n = len(self.pyramids)
+        self.depths = list(depth_buffers)
+        self.hizs = (C.c_void_p * n)(*[p._h.value for p in self.pyramids])
+        self.image = all(isinstance(d, DepthImage) for d in self.depths)
+        if self.image:
+            assert len({d.size for d in self.depths}) == 1, "every depth image of a batch has the same size"
+            self.dptrs = (C.c_void_p * n)(*[d._h.value for d in self.depths])
+            return
         shapes = {tuple(d.shape) for d in depth_buffers}
         assert len(shapes) == 1, "every depth buffer of a batch has the same size"
         self.h, self.w = shapes.pop()
         assert all(d.dtype == torch.float32 and d.is_contiguous() for d in depth_buffers)
-        self.depths = list(depth_buffers)
-        self.hizs = (C.c_void_p * n)(*[p._h.value for p in self.pyramids])
         self.dptrs = (C.c_void_p * n)(*[d.data_ptr() for d in self.depths])
 
     def launch(self, s):
         from . import _lib
-        _lib.check(self._lib.orbit_hiz_build_views(self.context._h, self.hizs, self.dptrs, self.n, self.w, self.h, s), "orbit_hiz_build_views")
+        if self.image:
+            _lib.check(self._lib.orbit_hiz_build_views_image(self.context._h, self.hizs, self.dptrs, self.n, s), "orbit_hiz_build_views_image")
+        else:
+            _lib.check(self._lib.orbit_hiz_build_views(self.context._h, self.hizs, self.dptrs, self.n, self.w, self.h, s), "orbit_hiz_build_views")
         for p in self.pyramids:
             p.usable = True
 
@@ -264,7 +273,7 @@ class PreparedViews:
     """PreparedFrame for several cameras over one scene: EARLY -> Hi-Z -> LATE (and, with `main_pass`, MAIN) of every camera,
     every argument packed once, 3 + 1 + 3 (+ 3) launches per group of up to MAX_BATCH_VIEWS cameras instead of 7 (10) per
     camera. `capture()` / `replay()` put the whole multi-camera frame into one CUDA graph. `outputs[v]`: camera v's
-    {"early", "late"[, "main"]} -> (dispatch_buffer, draw_buffer)."""
+    {"early", "late"[, "main"]} -> (dispatch_buffer, draw_buffer). `depth_buffers`: tensors, or DepthImages (all of one kind)."""
 
     def __init__(self, context, dscene, vstates, views, depth_buffers, meshlet_occlusion=True, name="views", main_pass=True):
         self.context = context
@@ -330,13 +339,17 @@ class PreparedFrame:
 
     The reference re-declares the passes each frame on its render graph; the packed form is the CUDA analogue:
     asynchronous stage calls on one stream, optionally captured into a CUDA graph (`capture()` / `replay()`) so
-    a frame costs one graph launch. Safe to replay: the scan epoch and tickets live in device memory."""
+    a frame costs one graph launch. Safe to replay: the scan epoch and tickets live in device memory.
+
+    `depth_buffer` is a float32 device tensor [H, W] or a DepthImage; with an image, hiz() and hiz_entity_late() (so launch())
+    call the *_image entry points, which write the same bytes."""
 
     def __init__(self, context, dscene, vstate, view, depth_buffer, meshlet_occlusion=True, name="forward_depth_prepass", main_pass=False,
                  fuse_late_main=True):
         import ctypes as C
         from . import _lib
         from .passes import _ptr, _scene_buffers
+        self.image = isinstance(depth_buffer, DepthImage)
         self.context, self.dscene, self.vstate, self.view, self.depth = context, dscene, vstate, view, depth_buffer
         self._lib, self._C, self._ptr = _lib.lib(), C, _ptr
         mvis = vstate.meshlet_visibility if meshlet_occlusion else None
@@ -362,11 +375,20 @@ class PreparedFrame:
         # LATE + MAIN fused (one entity kernel, one test kernel, an emit kernel per list) whenever the pair allows it
         self.fused = bool(main_pass and fuse_late_main and self._lib.orbit_cull_pair_compatible(C.byref(self.g_late), C.byref(self.g_early)))
         self.graph = None
-        h, w = depth_buffer.shape
-        self._hw = (w, h)
+        if self.image:
+            self._hw = depth_buffer.size
+            self._hiz_build, self._hiz_entity_late = self._lib.orbit_hiz_build_image, self._lib.orbit_hiz_build_image_entity_cull_late
+        else:
+            h, w = depth_buffer.shape
+            self._hw = (w, h)
+            self._hiz_build, self._hiz_entity_late = self._lib.orbit_hiz_build, self._lib.orbit_hiz_build_entity_cull_late
 
     def _stream(self):
         return self._C.c_void_p(torch.cuda.current_stream(self.context.device).cuda_stream)
+
+    def _depth_args(self):
+        """The depth arguments of the build calls chosen at construction: (image) or (depth, width, height)."""
+        return (self.depth._h,) if self.image else (self._ptr(self.depth), self._hw[0], self._hw[1])
 
     def entity(self, late, s=None):
         C, lib, p = self._C, self._lib, self._ptr
@@ -422,9 +444,9 @@ class PreparedFrame:
 
     def hiz(self, s=None):
         s = s or self._stream()
-        rc = self._lib.orbit_hiz_build(self.context._h, self.vstate.depth_pyramid._h, self._ptr(self.depth), self._hw[0], self._hw[1], s)
+        rc = self._hiz_build(self.context._h, self.vstate.depth_pyramid._h, *self._depth_args(), s)
         if rc:
-            raise RuntimeError("orbit_hiz_build: %d" % rc)
+            raise RuntimeError("%s: %d" % (self._hiz_build.__name__, rc))
 
     def hiz_entity_late(self, s=None):
         """hiz() followed by entity(True) — with a fused frame, by entity_late_main() — as ONE call
@@ -432,11 +454,11 @@ class PreparedFrame:
         under the build."""
         C, lib, p = self._C, self._lib, self._ptr
         g_main, main_dispatch = (C.byref(self.g_early), p(self.main_dispatch)) if self.fused else (None, None)
-        rc = lib.orbit_hiz_build_entity_cull_late(self.context._h, self.vstate.depth_pyramid._h, p(self.depth), self._hw[0], self._hw[1],
-                                                  C.byref(self.g_late), g_main, C.byref(self.sb_late), p(self.late_dispatch), main_dispatch,
-                                                  self.rcap, s or self._stream())
+        rc = self._hiz_entity_late(self.context._h, self.vstate.depth_pyramid._h, *self._depth_args(),
+                                   C.byref(self.g_late), g_main, C.byref(self.sb_late), p(self.late_dispatch), main_dispatch,
+                                   self.rcap, s or self._stream())
         if rc:
-            raise RuntimeError("orbit_hiz_build_entity_cull_late: %d" % rc)
+            raise RuntimeError("%s: %d" % (self._hiz_entity_late.__name__, rc))
 
     def launch(self, overlap_main_entity=False):
         """The frame's stage calls in dependency order. `overlap_main_entity`: the MAIN pass's entity stage depends only on the
@@ -491,6 +513,7 @@ def host_frame_loop(context, prepared, scene_datas, h_transforms, h_depth, h_cou
     import ctypes as C
     from . import _lib
     n = len(prepared)
+    assert not any(pf.image for pf in prepared), "the host frame driver reads depth from a linear buffer"
     frames = (L.HostFrame * n)()
     for f, pf, sd in zip(frames, prepared, scene_datas):
         sd.update_scene(pf.dscene.assets)       # packs sd._packed (and keeps the ranges allocated)

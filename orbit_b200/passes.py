@@ -214,6 +214,33 @@ def _scene_buffers(assets, scene, cull):
     return sb
 
 
+class DepthImage:
+    """A depth buffer held in a 2-D single-channel float32 CUDA array (orbit_depth_image_wrap): the form a depth attachment
+    imported from Vulkan takes (cudaExternalMemoryGetMappedMipmappedArray, level 0). `cuda_array` is the cudaArray_t as an
+    integer; the array stays the caller's and must outlive this object and every enqueued or captured call that reads it.
+    DepthPyramid.update, compute_clusters and the frame classes take one wherever they take a depth tensor."""
+
+    def __init__(self, context, cuda_array):
+        self.context = context
+        self._h = C.c_void_p()
+        _lib.check(_lib.lib().orbit_depth_image_wrap(context._h, C.c_void_p(int(cuda_array)), C.byref(self._h)), "orbit_depth_image_wrap")
+        self.cuda_array = int(cuda_array)
+        w, h = C.c_uint32(), C.c_uint32()
+        _lib.check(_lib.lib().orbit_depth_image_size(self._h, C.byref(w), C.byref(h)), "orbit_depth_image_size")
+        self.size = (w.value, h.value)
+
+    def close(self):
+        if self._h:
+            _lib.lib().orbit_depth_image_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
 class DepthPyramid:
     """draw_gen.rs:451-567. One linear f32 allocation holding all mips back to back."""
 
@@ -260,7 +287,13 @@ class DepthPyramid:
         self.usable = False
 
     def update(self, depth_buffer):
-        """depth_buffer: float32 device tensor [H, W] (reverse-Z)."""
+        """depth_buffer: float32 device tensor [H, W] (reverse-Z), or a DepthImage of the same size."""
+        if isinstance(depth_buffer, DepthImage):
+            assert depth_buffer.size == self.size
+            _lib.check(_lib.lib().orbit_hiz_build_image(self.context._h, self._h, depth_buffer._h, _stream(self.context)),
+                       "orbit_hiz_build_image")
+            self.usable = True
+            return
         h, w = depth_buffer.shape
         assert (w, h) == self.size and depth_buffer.dtype == torch.float32 and depth_buffer.is_contiguous()
         _lib.check(_lib.lib().orbit_hiz_build(self.context._h, self._h, _ptr(depth_buffer), w, h, _stream(self.context)), "orbit_hiz_build")
@@ -360,8 +393,10 @@ class GraphClusterInfo:
 
 def compute_clusters(context, settings, view_matrix, projection_matrix, near, depth_buffer, scene, name="clusters"):
     """cluster.rs:368-397 = mark_active_clusters + compact_active_clusters + cluster_light_assignment.
-    view_matrix / projection_matrix: 4x4 math convention (Camera in the reference)."""
-    h, w = depth_buffer.shape
+    view_matrix / projection_matrix: 4x4 math convention (Camera in the reference).
+    depth_buffer: float32 device tensor [H, W], or a DepthImage."""
+    image = isinstance(depth_buffer, DepthImage)
+    w, h = depth_buffer.size if image else (depth_buffer.shape[1], depth_buffer.shape[0])
     assert (w, h) == tuple(settings.screen_resolution)
     cx, cy, cz = settings.cluster_counts()
     n = cx * cy * cz
@@ -377,10 +412,11 @@ def compute_clusters(context, settings, view_matrix, projection_matrix, near, de
     masks = context.create_transient(name + "_tile_depth_slice_mask", 4 * cx * cy)
     bounds = context.create_transient(name + "_cluster_depth_bounds", 8 * n)
     unique = context.create_transient(name + "_unique_cluster_buffer", 16 + 4 * n)
-    image = context.create_transient(name + "_cluster_offset_image", 8 * n)
+    offsets = context.create_transient(name + "_cluster_offset_image", 8 * n)
     cap = L.MAX_LIGHTS_PER_CLUSTER * n          # MAX_LIGHT_INDEX_COUNT in the reference is a fixed constant
     index = context.create_transient(name + "_light_index_buffer", 4 + 4 * cap)
-    _lib.check(_lib.lib().orbit_light_cluster(context._h, C.byref(p), _ptr(depth_buffer), _ptr(scene.light_data_buffer),
-                                              _ptr(masks), _ptr(bounds), _ptr(unique), _ptr(image), _ptr(index), cap,
-                                              _stream(context)), "orbit_light_cluster")
-    return GraphClusterInfo(image, index, masks, bounds, unique, (cx, cy), cz, p.z_scale, p.z_bias, settings.tile_px_size()), p
+    fn, name_ = ((_lib.lib().orbit_light_cluster_image, "orbit_light_cluster_image") if image
+                 else (_lib.lib().orbit_light_cluster, "orbit_light_cluster"))
+    _lib.check(fn(context._h, C.byref(p), depth_buffer._h if image else _ptr(depth_buffer), _ptr(scene.light_data_buffer),
+                  _ptr(masks), _ptr(bounds), _ptr(unique), _ptr(offsets), _ptr(index), cap, _stream(context)), name_)
+    return GraphClusterInfo(offsets, index, masks, bounds, unique, (cx, cy), cz, p.z_scale, p.z_bias, settings.tile_px_size()), p

@@ -14,6 +14,7 @@ pub const ORBIT_HIZ_MAX_LEVELS: usize = 16;
 
 #[repr(C)] pub struct orbit_ctx { _p: [u8; 0] }
 #[repr(C)] pub struct orbit_hiz { _p: [u8; 0] }
+#[repr(C)] pub struct orbit_depth_image { _p: [u8; 0] }
 
 /// = `GpuCullInfo` (draw_gen.rs:208-237), 400 bytes.
 #[repr(C)]
@@ -181,6 +182,20 @@ extern "C" {
                              n_meshes: u32, stream: *mut c_void) -> i32;
     pub fn orbit_draws_scatter(ctx: *mut orbit_ctx, src_draw_buffer: *const c_void, src_capacity_draws: u64, dst_draw_buffer: *mut c_void,
                                dst_first: u32, total_count: u32, dst_capacity_draws: u64, stream: *mut c_void) -> i32;
+    pub fn orbit_depth_image_wrap(ctx: *mut orbit_ctx, cuda_array: *mut c_void, out: *mut *mut orbit_depth_image) -> c_int;
+    pub fn orbit_depth_image_destroy(image: *mut orbit_depth_image);
+    pub fn orbit_depth_image_size(image: *const orbit_depth_image, width: *mut u32, height: *mut u32) -> c_int;
+    pub fn orbit_hiz_build_image(ctx: *mut orbit_ctx, hiz: *mut orbit_hiz, image: *const orbit_depth_image, stream: *mut c_void) -> c_int;
+    pub fn orbit_hiz_build_views_image(ctx: *mut orbit_ctx, hizs: *const *mut orbit_hiz, images: *const *const orbit_depth_image, n_views: u32,
+                                       stream: *mut c_void) -> c_int;
+    pub fn orbit_hiz_build_image_entity_cull_late(ctx: *mut orbit_ctx, hiz: *mut orbit_hiz, image: *const orbit_depth_image,
+                                                  late: *const OrbitCullInfo, main_pass: *const OrbitCullInfo, scene: *const OrbitSceneBuffers,
+                                                  late_dispatch_buffer: *mut c_void, main_dispatch_buffer: *mut c_void, capacity_records: u64,
+                                                  stream: *mut c_void) -> c_int;
+    pub fn orbit_light_cluster_image(ctx: *mut orbit_ctx, params: *const OrbitClusterParams, image: *const orbit_depth_image, lights: *const c_void,
+                                     tile_masks: *mut c_void, depth_bounds: *mut c_void, unique_clusters: *mut c_void,
+                                     offset_count_image: *mut c_void, light_index_list: *mut c_void, capacity_indices: u64,
+                                     stream: *mut c_void) -> c_int;
 }
 
 /// Safe-ish wrappers shaped like the reference entry points (draw_gen.rs:327-389, 456-566).
@@ -299,3 +314,62 @@ impl DepthPyramid {
     }
 }
 impl Drop for DepthPyramid { fn drop(&mut self) { unsafe { orbit_hiz_destroy(self.hiz) } } }
+
+/// The depth attachment as a CUDA array (orbit_depth_image_wrap): level 0 of the mipmapped array that
+/// cudaExternalMemoryGetMappedMipmappedArray maps from an imported VkImage, with one 32-bit float channel. The array stays the
+/// caller's; it, and this handle, must outlive every enqueued call and captured graph that reads them. Ordering the renderer's
+/// writes of the image before the calls (an imported semaphore waited on the stream) is the caller's job.
+pub struct DepthImage { image: *mut orbit_depth_image, size: [u32; 2] }
+impl DepthImage {
+    pub unsafe fn wrap(ctx: &Context, cuda_array: *mut c_void) -> Result<Self, Error> {
+        let mut p = std::ptr::null_mut();
+        check(orbit_depth_image_wrap(ctx.0, cuda_array, &mut p))?;
+        let (mut w, mut h) = (0u32, 0u32);
+        check(orbit_depth_image_size(p, &mut w, &mut h))?;
+        Ok(Self { image: p, size: [w, h] })
+    }
+    pub fn size(&self) -> [u32; 2] { self.size }
+    pub fn as_ptr(&self) -> *const orbit_depth_image { self.image }
+}
+impl Drop for DepthImage { fn drop(&mut self) { unsafe { orbit_depth_image_destroy(self.image) } } }
+
+impl DepthPyramid {
+    /// update() with the depth read from `image` (orbit_hiz_build_image): the same texels.
+    pub unsafe fn update_from_image(&mut self, ctx: &Context, image: &DepthImage, stream: *mut c_void) -> Result<(), Error> {
+        check(orbit_hiz_build_image(ctx.0, self.hiz, image.image, stream))?;
+        self.usable = true;
+        Ok(())
+    }
+    /// update_and_cull_late() with the depth read from `image` (orbit_hiz_build_image_entity_cull_late).
+    pub unsafe fn update_from_image_and_cull_late(&mut self, ctx: &Context, image: &DepthImage, late: &OrbitCullInfo,
+                                                  main_pass: Option<&OrbitCullInfo>, scene: &OrbitSceneBuffers, late_dispatch_buffer: *mut c_void,
+                                                  main_dispatch_buffer: *mut c_void, capacity_records: u64, stream: *mut c_void) -> Result<(), Error> {
+        let main_ptr = main_pass.map_or(std::ptr::null(), |m| m as *const OrbitCullInfo);
+        check(orbit_hiz_build_image_entity_cull_late(ctx.0, self.hiz, image.image, late, main_ptr, scene, late_dispatch_buffer,
+                                                     main_dispatch_buffer, capacity_records, stream))?;
+        self.usable = true;
+        Ok(())
+    }
+}
+
+impl Context {
+    /// update_depth_pyramids() with depth v read from images[v] (orbit_hiz_build_views_image).
+    pub unsafe fn update_depth_pyramids_from_images(&self, pyramids: &mut [DepthPyramid], images: &[&DepthImage], stream: *mut c_void) -> Result<(), Error> {
+        if pyramids.is_empty() || pyramids.len() > ORBIT_MAX_BATCH_VIEWS as usize || images.len() != pyramids.len() {
+            return Err(Error(ORBIT_ERR_INVALID_ARGUMENT));
+        }
+        let hizs: Vec<*mut orbit_hiz> = pyramids.iter().map(|p| p.hiz).collect();
+        let imgs: Vec<*const orbit_depth_image> = images.iter().map(|i| i.image as *const orbit_depth_image).collect();
+        check(orbit_hiz_build_views_image(self.0, hizs.as_ptr(), imgs.as_ptr(), pyramids.len() as u32, stream))?;
+        for p in pyramids.iter_mut() { p.usable = true; }
+        Ok(())
+    }
+    /// compute_clusters (cluster.rs:368-591) with the depth read from `image` (orbit_light_cluster_image).
+    pub unsafe fn compute_clusters_from_image(&self, params: &OrbitClusterParams, image: &DepthImage, lights: *const c_void,
+                                              tile_masks: *mut c_void, depth_bounds: *mut c_void, unique_clusters: *mut c_void,
+                                              offset_count_image: *mut c_void, light_index_list: *mut c_void, capacity_indices: u64,
+                                              stream: *mut c_void) -> Result<(), Error> {
+        check(orbit_light_cluster_image(self.0, params, image.image, lights, tile_masks, depth_bounds, unique_clusters, offset_count_image,
+                                        light_index_list, capacity_indices, stream))
+    }
+}
