@@ -5,6 +5,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <initializer_list>
 #include <new>
 #include "params.cuh"
 
@@ -24,8 +25,54 @@ bool pdl_enabled() {
 }  // namespace orbit
 
 static thread_local int g_last_cuda_error = 0;
-static constexpr size_t kViewChunkWords = 2u * 2048u;   // per view: two parities of chunk counts
-static constexpr size_t kViewCounterWords = ORBIT_MAX_BATCH_VIEWS * (kViewChunkWords + 4u);
+
+// ---- the context's device words ------------------------------------------------------------------------------------------
+// Every word and region of orbit_ctx::counters, chunk_counts and view_counters, in 32-bit words. Each block is zeroed when it
+// is allocated (then kScanEpoch set to 1). A captured CUDA graph keeps these addresses in its kernel parameters: no offset may
+// move. A meshlet-stage list has kListWords (survivor totals per parity, then parity words A, B) and kChunkWords (per-chunk
+// survivor counts, two parities of 2048 chunks).
+struct Region { uint32_t at, words; };
+constexpr uint32_t kListWords = 4u, kChunkWords = 2u * 2048u;
+// orbit_ctx::counters
+constexpr Region kScanTicket{0, 1};            // scans (entity stage, light clusters): next tile to hand out
+constexpr Region kScanDone{1, 1};              // scans: CTAs that have finished
+constexpr Region kHizTicket{2, 1};             // orbit_hiz_build: last-CTA ticket
+constexpr Region kScanEpoch{3, 1};             // scans: launch epoch, device-advanced
+constexpr Region kMeshletWords{4, kListWords}; // orbit_meshlet_cull, orbit_draws_from_masks
+constexpr Region kCursorSnapshot{8, 1};        // orbit_scene_update: visibility cursor at the start of the update
+constexpr Region kTestWords{10, kListWords};   // orbit_meshlet_test: never read; apart, so none leaks into kMeshletWords
+constexpr Region kDrawsHeader{16, 3};          // orbit_draws_from_masks: dispatch header written by the recount kernel
+constexpr Region kMainWords{20, kListWords};   // fused MAIN pass (orbit_meshlet_cull_late_main)
+constexpr Region kPeerDone{24, 16};            // orbit_peer_put: CTAs that have finished, per transfer (self-resetting)
+constexpr Region kHizViewTickets{40, ORBIT_MAX_BATCH_VIEWS};   // orbit_hiz_build_views: pyramid v's last-CTA ticket
+constexpr uint32_t kCounterWords = 64;
+// orbit_ctx::chunk_counts
+constexpr Region kMeshletChunks{0, kChunkWords};                // orbit_meshlet_cull, orbit_draws_from_masks
+constexpr Region kTestChunks{kChunkWords, kChunkWords};         // orbit_meshlet_test
+constexpr Region kMainChunks{2u * kChunkWords, kChunkWords};    // fused MAIN pass
+constexpr uint32_t kChunkCountWords = 3u * kChunkWords;
+// orbit_ctx::view_counters (batched meshlet stage): view v's chunk counts at kViewChunks.at + v * kChunkWords, its list words
+// at kViewWords.at + v * kListWords
+constexpr Region kViewChunks{0, ORBIT_MAX_BATCH_VIEWS * kChunkWords};
+constexpr Region kViewWords{kViewChunks.words, ORBIT_MAX_BATCH_VIEWS * kListWords};
+constexpr uint32_t kViewCounterWords = kViewWords.at + kViewWords.words;
+
+// no two regions overlap and all lie in [0, total)
+constexpr bool disjoint_within(std::initializer_list<Region> regions, uint32_t total) {
+    for (const Region* a = regions.begin(); a != regions.end(); ++a) {
+        if (a->at + a->words > total) return false;
+        for (const Region* b = regions.begin(); b != a; ++b)
+            if (a->at < b->at + b->words && b->at < a->at + a->words) return false;
+    }
+    return true;
+}
+static_assert(disjoint_within({kScanTicket, kScanDone, kHizTicket, kScanEpoch, kMeshletWords, kCursorSnapshot, kTestWords, kDrawsHeader,
+                               kMainWords, kPeerDone, kHizViewTickets}, kCounterWords), "orbit_ctx::counters: regions overlap or overrun the allocation");
+static_assert(disjoint_within({kMeshletChunks, kTestChunks, kMainChunks}, kChunkCountWords),
+              "orbit_ctx::chunk_counts: regions overlap or overrun the allocation");
+static_assert(disjoint_within({kViewChunks, kViewWords}, kViewCounterWords),
+              "orbit_ctx::view_counters: regions overlap or overrun the allocation");
+
 #define CK(expr)                                                       \
     do {                                                               \
         cudaError_t e_ = (expr);                                       \
@@ -54,15 +101,12 @@ struct orbit_ctx {
     size_t status_capacity = 0;       // descriptors
     uint4* main_masks = nullptr;      // record entries of the fused MAIN pass
     size_t main_mask_capacity = 0;
-    unsigned int* counters = nullptr; // 32 words: [0] ticket, [1] done, [2] hiz ticket, [3] scan epoch (device-advanced), [4,5] meshlet survivor
-                                      // totals per parity, [6,7] parity words A/B of the meshlet stage, [8] scene-update cursor snapshot,
-                                      // [10..13] the same four words for test-only calls, [16..18] dispatch header of orbit_draws_from_masks
+    unsigned int* counters = nullptr; // kCounterWords words (layout at the top of this file)
     // device-written status, pinned + mapped
     OrbitStatus* status_host = nullptr;
     OrbitStatus* status_dev = nullptr;
-    uint32_t* chunk_counts = nullptr; // 2 x 2048 per-chunk survivor counts
-    uint32_t* view_counters = nullptr;// batched views (orbit_meshlet_cull_views): 16 x 2 x 2048 chunk counts, then 16 x {survivor totals
-                                      // per parity, parity words A/B} — apart from the single-view words, so both forms may interleave.
+    uint32_t* chunk_counts = nullptr; // kChunkCountWords words
+    uint32_t* view_counters = nullptr;// kViewCounterWords words, apart from the single-view words, so both forms may interleave.
                                       // Allocated by the first batched call, never in orbit_ctx_create: an allocation there moves the
                                       // buffers created after it (the scan descriptors the entity kernel polls), and the single-view
                                       // entity stage measured ~1 us slower on C2 with its descriptors at the shifted address
@@ -125,55 +169,42 @@ static int retire(orbit_ctx* c, void* p) {
     return ORBIT_OK;
 }
 
+// Grows scratch to hold `count` elements: `initial`, doubled as often as needed, is the capacity of every one of `arrays` (a
+// pointer and its bytes per element). All are retired first, then each is allocated in order and zeroed on *zero_on if given.
+struct ScratchArray { void** ptr; size_t elem_bytes; };
+static int grow(orbit_ctx* c, size_t* capacity, uint64_t count, size_t initial, std::initializer_list<ScratchArray> arrays,
+                const cudaStream_t* zero_on = nullptr) {
+    if (count <= *capacity) return ORBIT_OK;
+    size_t cap = initial; while (cap < count) cap *= 2;
+    for (const ScratchArray& a : arrays) {
+        int rc = retire(c, *a.ptr);
+        if (rc != ORBIT_OK) return rc;
+    }
+    for (const ScratchArray& a : arrays) *a.ptr = nullptr;
+    *capacity = 0;
+    for (const ScratchArray& a : arrays) {
+        CK(cudaMalloc(a.ptr, cap * a.elem_bytes));
+        if (zero_on) CK(cudaMemsetAsync(*a.ptr, 0, cap * a.elem_bytes, *zero_on));
+    }
+    *capacity = cap;
+    return ORBIT_OK;
+}
+
 // Scan descriptors; a fresh array is zeroed on `stream` (epoch 0 never matches a launch: epochs start at 1).
 static int ensure_status(orbit_ctx* c, size_t tiles, cudaStream_t stream) {
-    if (tiles <= c->status_capacity) return ORBIT_OK;
-    size_t cap = c->status_capacity ? c->status_capacity : 4096;
-    while (cap < tiles) cap *= 2;
-    int rc = retire(c, c->status);
-    if (rc != ORBIT_OK) return rc;
-    c->status = nullptr; c->status_capacity = 0;
-    CK(cudaMalloc(&c->status, cap * sizeof(unsigned long long)));
-    CK(cudaMemsetAsync(c->status, 0, cap * sizeof(unsigned long long), stream));
-    c->status_capacity = cap;
-    return ORBIT_OK;
+    return grow(c, &c->status_capacity, tiles, 4096, {{(void**)&c->status, sizeof(unsigned long long)}}, &stream);
 }
-
 static int ensure_tile_sums(orbit_ctx* c, size_t tiles) {
-    if (tiles <= c->tile_sums_capacity) return ORBIT_OK;
-    size_t cap = c->tile_sums_capacity ? c->tile_sums_capacity : 1024;
-    while (cap < tiles) cap *= 2;
-    int rc = retire(c, c->tile_sums);
-    if (rc != ORBIT_OK) return rc;
-    c->tile_sums = nullptr; c->tile_sums_capacity = 0;
-    CK(cudaMalloc(&c->tile_sums, cap * sizeof(unsigned long long)));
-    c->tile_sums_capacity = cap;
-    return ORBIT_OK;
+    return grow(c, &c->tile_sums_capacity, tiles, 1024, {{(void**)&c->tile_sums, sizeof(unsigned long long)}});
 }
-
 // record entries of the fused MAIN pass (orbit_meshlet_cull_late_main)
 static int ensure_main_masks(orbit_ctx* c, uint64_t max_records) {
-    if (max_records <= c->main_mask_capacity) return ORBIT_OK;
-    int rc = retire(c, c->main_masks);
-    if (rc != ORBIT_OK) return rc;
-    c->main_masks = nullptr; c->main_mask_capacity = 0;
-    size_t cap = 65536; while (cap < max_records) cap *= 2;
-    CK(cudaMalloc(&c->main_masks, cap * sizeof(uint4)));
-    c->main_mask_capacity = cap;
-    return ORBIT_OK;
+    return grow(c, &c->main_mask_capacity, max_records, 65536, {{(void**)&c->main_masks, sizeof(uint4)}});
 }
-
+// record entries and side words of the meshlet stage, one of each per dispatch record / (record, lane)
 static int ensure_record_scratch(orbit_ctx* c, uint64_t max_records) {
-    if (max_records <= c->draw_mask_capacity) return ORBIT_OK;
-    int rc = retire(c, c->draw_masks);
-    if (rc == ORBIT_OK) rc = retire(c, c->cmd_side);
-    if (rc != ORBIT_OK) return rc;
-    c->draw_masks = nullptr; c->cmd_side = nullptr; c->draw_mask_capacity = 0;
-    size_t cap = 65536; while (cap < max_records) cap *= 2;
-    CK(cudaMalloc(&c->draw_masks, cap * sizeof(uint4)));
-    CK(cudaMalloc(&c->cmd_side, cap * 32u * sizeof(uint4)));
-    c->draw_mask_capacity = cap;
-    return ORBIT_OK;
+    return grow(c, &c->draw_mask_capacity, max_records, 65536,
+                {{(void**)&c->draw_masks, sizeof(uint4)}, {(void**)&c->cmd_side, 32u * sizeof(uint4)}});
 }
 
 // The light-parallel culling path keeps one hit bit per (cluster, light); grids whose matrix would exceed this budget (the
@@ -184,25 +215,10 @@ static uint64_t light_hits_words_needed(uint64_t clusters, uint64_t n_lights) { 
 }
 
 static int ensure_light_hits(orbit_ctx* c, uint64_t words) {
-    if (words <= c->light_hits_words) return ORBIT_OK;
-    int rc = retire(c, c->light_hits);
-    if (rc != ORBIT_OK) return rc;
-    c->light_hits = nullptr; c->light_hits_words = 0;
-    size_t cap = 1u << 16; while (cap < words) cap *= 2;
-    CK(cudaMalloc(&c->light_hits, cap * sizeof(uint32_t)));
-    c->light_hits_words = cap;
-    return ORBIT_OK;
+    return grow(c, &c->light_hits_words, words, 1u << 16, {{(void**)&c->light_hits, sizeof(uint32_t)}});
 }
-
 static int ensure_lights(orbit_ctx* c, uint64_t n_lights) {
-    if (n_lights <= c->light_capacity) return ORBIT_OK;
-    int rc = retire(c, c->light_view);
-    if (rc != ORBIT_OK) return rc;
-    c->light_view = nullptr; c->light_capacity = 0;
-    size_t cap = 1024; while (cap < n_lights) cap *= 2;
-    CK(cudaMalloc(&c->light_view, cap * sizeof(float4)));
-    c->light_capacity = cap;
-    return ORBIT_OK;
+    return grow(c, &c->light_capacity, n_lights, 1024, {{(void**)&c->light_view, sizeof(float4)}});
 }
 
 // block of the timeline buffer for the next kernel launch (development builds), else nullptr
@@ -212,19 +228,44 @@ static unsigned long long* next_trace(orbit_ctx* c) {
 }
 
 static ScanState next_scan(orbit_ctx* c) {
-    return ScanState{next_trace(c), c->status, c->counters + 0, c->counters + 1, c->counters + 3};
+    return ScanState{next_trace(c), c->status, c->counters + kScanTicket.at, c->counters + kScanDone.at, c->counters + kScanEpoch.at};
+}
+
+// Pyramid geometry of h into a parameter block that reads it (HizDevice) or builds it (HizBuildParams)
+template <typename P>
+static void set_pyramid(P& p, const orbit_hiz* h) {
+    p.texels = h->info.texels; p.width = h->info.width; p.height = h->info.height; p.levels = h->info.levels;
+    for (int i = 0; i < ORBIT_HIZ_MAX_LEVELS; ++i) p.level_offset[i] = h->info.level_offset[i];
 }
 
 static HizDevice hiz_device(const orbit_hiz* h) {
     HizDevice d{};
-    if (h) {
-        d.texels = h->info.texels; d.width = h->info.width; d.height = h->info.height; d.levels = h->info.levels;
-        for (int i = 0; i < ORBIT_HIZ_MAX_LEVELS; ++i) d.level_offset[i] = h->info.level_offset[i];
-    }
+    if (h) set_pyramid(d, h);
     return d;
 }
 
+// hizs[v] shares its texels with none of hizs[0..v)
+static bool pyramid_distinct(const orbit_hiz* const* hizs, uint32_t v) {
+    for (uint32_t u = 0; u < v; ++u) if (hizs[u]->info.texels == hizs[v]->info.texels) return false;
+    return true;
+}
+
 static uint32_t npot(uint32_t v) { uint32_t p = 1; while (p < v) p <<= 1; return p; }
+
+// A kernel's CTAs per SM, cached in `occ` (`query` asks the runtime on first use); at least 1
+template <typename Query>
+static int occupancy(int& occ, Query query) {
+    if (occ <= 0) occ = query();
+    return occ > 0 ? occ : 1;
+}
+
+// Meshlet test-kernel grid: persistent warps, cyclic tiles, no inter-CTA dependency -> one full wave of CTAs. `occ` caches the
+// kernel variant's occupancy; ORBIT_MC_CTAS_PER_SM overrides it.
+template <typename Query>
+static uint64_t test_grid(orbit_ctx* c, int& occ, Query query) {
+    const int per_sm = occupancy(occ, query);
+    return (uint64_t)c->sm_count * (uint64_t)(c->mc_ctas_per_sm > 0 ? c->mc_ctas_per_sm : per_sm);
+}
 
 extern "C" {
 
@@ -259,11 +300,11 @@ int orbit_ctx_create(int device, orbit_ctx** out) {
     cudaDeviceProp prop;
     CK(cudaGetDeviceProperties(&prop, device));
     c->sm_count = prop.multiProcessorCount;
-    CK(cudaMalloc(&c->counters, 64 * sizeof(unsigned int)));
-    CK(cudaMemset(c->counters, 0, 64 * sizeof(unsigned int)));
-    { const unsigned int one = 1u; CK(cudaMemcpy(c->counters + 3, &one, sizeof(one), cudaMemcpyHostToDevice)); }
-    CK(cudaMalloc(&c->chunk_counts, 6 * 2048 * sizeof(uint32_t)));   // two parities for orbit_meshlet_cull + two (never read) for orbit_meshlet_test + two for the fused MAIN pass
-    CK(cudaMemset(c->chunk_counts, 0, 6 * 2048 * sizeof(uint32_t)));
+    CK(cudaMalloc(&c->counters, kCounterWords * sizeof(unsigned int)));
+    CK(cudaMemset(c->counters, 0, kCounterWords * sizeof(unsigned int)));
+    { const unsigned int one = 1u; CK(cudaMemcpy(c->counters + kScanEpoch.at, &one, sizeof(one), cudaMemcpyHostToDevice)); }
+    CK(cudaMalloc(&c->chunk_counts, kChunkCountWords * sizeof(uint32_t)));
+    CK(cudaMemset(c->chunk_counts, 0, kChunkCountWords * sizeof(uint32_t)));
     CK(cudaHostAlloc(&c->status_host, sizeof(OrbitStatus), cudaHostAllocMapped));
     std::memset(c->status_host, 0, sizeof(OrbitStatus));
     CK(cudaHostGetDevicePointer(&c->status_dev, c->status_host, 0));
@@ -395,47 +436,46 @@ static bool hiz_build_args_ok(orbit_ctx* c, orbit_hiz* h, const float* depth, ui
     return c && h && depth && dw == h->depth_w && dh == h->depth_h;
 }
 
-static HizBuildParams hiz_build_params(orbit_ctx* c, orbit_hiz* h, const float* depth, uint32_t dw, uint32_t dh) {
+// One build of h, from `image` when it is not NULL, else from `depth`; arguments already checked (the source has h's depth
+// size), device already current.
+static int hiz_build_launch(orbit_ctx* c, const orbit_hiz* h, const float* depth, const orbit_depth_image* image, void* stream) {
     HizBuildParams p{};
-    p.depth = depth; p.texels = h->info.texels; p.depth_w = dw; p.depth_h = dh;
-    p.width = h->info.width; p.height = h->info.height; p.levels = h->info.levels;
-    for (int i = 0; i < ORBIT_HIZ_MAX_LEVELS; ++i) p.level_offset[i] = h->info.level_offset[i];
-    p.ticket = c->counters + 2;
+    if (image) p.depth_tex = image->tex;
+    else p.depth = depth;
+    p.depth_w = h->depth_w; p.depth_h = h->depth_h;
+    set_pyramid(p, h);
+    p.ticket = c->counters + kHizTicket.at;
     p.trace = next_trace(c);
-    return p;
+    CK(launch_hiz_build(p, (cudaStream_t)stream, image != nullptr));
+    c->launches += 1;
+    return ORBIT_OK;
 }
 
 int orbit_hiz_build(orbit_ctx* c, orbit_hiz* h, const float* depth, uint32_t dw, uint32_t dh, void* stream) {
     if (!hiz_build_args_ok(c, h, depth, dw, dh)) return ORBIT_ERR_INVALID_ARGUMENT;
     GUARD(c);
-    CK(launch_hiz_build(hiz_build_params(c, h, depth, dw, dh), (cudaStream_t)stream));
-    c->launches += 1;
-    return ORBIT_OK;
+    return hiz_build_launch(c, h, depth, nullptr, stream);
 }
 
-// Batched form: one launch, a row of CTAs per pyramid. Pyramid v's ticket is counter word 40 + v (words 40..55 are used by
-// nothing else and were zeroed with the rest at context creation; each row's last CTA re-zeroes its own).
-// Depth v comes from depths[v], or from images[v] when depths is NULL (images already checked, each dw x dh).
+// Batched form: one launch, a row of CTAs per pyramid, each row with its own ticket (kHizViewTickets; each row's last CTA
+// re-zeroes its own). Depth v comes from depths[v], or from images[v] when depths is NULL (images already checked, each dw x dh).
 static int hiz_build_views(orbit_ctx* c, orbit_hiz* const* hizs, const float* const* depths, const orbit_depth_image* const* images,
                            uint32_t n_views, uint32_t dw, uint32_t dh, void* stream) {
     if (!c || !hizs || n_views == 0u || n_views > ORBIT_MAX_BATCH_VIEWS) return ORBIT_ERR_INVALID_ARGUMENT;
     for (uint32_t v = 0; v < n_views; ++v) {
         const orbit_hiz* h = hizs[v];
-        if (!h || (depths && !depths[v]) || dw != h->depth_w || dh != h->depth_h) return ORBIT_ERR_INVALID_ARGUMENT;
-        for (uint32_t u = 0; u < v; ++u) if (hizs[u]->info.texels == h->info.texels) return ORBIT_ERR_INVALID_ARGUMENT;
+        if (!h || (depths && !depths[v]) || dw != h->depth_w || dh != h->depth_h || !pyramid_distinct(hizs, v)) return ORBIT_ERR_INVALID_ARGUMENT;
     }
     GUARD(c);
     HizBuildViewsParams pv{};
     pv.n_views = n_views;
     for (uint32_t v = 0; v < n_views; ++v) {
-        const orbit_hiz* h = hizs[v];
         HizBuildParams& p = pv.view[v];
         if (depths) p.depth = depths[v];
         else p.depth_tex = images[v]->tex;
-        p.texels = h->info.texels; p.depth_w = dw; p.depth_h = dh;
-        p.width = h->info.width; p.height = h->info.height; p.levels = h->info.levels;
-        for (int i = 0; i < ORBIT_HIZ_MAX_LEVELS; ++i) p.level_offset[i] = h->info.level_offset[i];
-        p.ticket = c->counters + 40 + v;
+        p.depth_w = dw; p.depth_h = dh;
+        set_pyramid(p, hizs[v]);
+        p.ticket = c->counters + kHizViewTickets.at + v;
     }
     pv.view[0].trace = next_trace(c);
     CK(launch_hiz_build_views(pv, (cudaStream_t)stream, depths == nullptr));
@@ -501,11 +541,7 @@ static bool image_ok(const orbit_ctx* c, const orbit_depth_image* img, uint32_t 
 int orbit_hiz_build_image(orbit_ctx* c, orbit_hiz* h, const orbit_depth_image* img, void* stream) {
     if (!c || !h || !image_ok(c, img, h->depth_w, h->depth_h)) return ORBIT_ERR_INVALID_ARGUMENT;
     GUARD(c);
-    HizBuildParams p = hiz_build_params(c, h, nullptr, img->width, img->height);
-    p.depth_tex = img->tex;
-    CK(launch_hiz_build(p, (cudaStream_t)stream, true));
-    c->launches += 1;
-    return ORBIT_OK;
+    return hiz_build_launch(c, h, nullptr, img, stream);
 }
 
 int orbit_hiz_build_views_image(orbit_ctx* c, orbit_hiz* const* hizs, const orbit_depth_image* const* images, uint32_t n_views,
@@ -561,18 +597,6 @@ static EntityCullParams entity_params(orbit_ctx* c, const OrbitCullInfo* cull, c
     return p;
 }
 
-static uint32_t entity_coresident_ctas(orbit_ctx* c, bool defer_wait) {
-    int& occ = c->entity_occupancy[defer_wait ? 1 : 0];
-    if (occ <= 0) occ = entity_cull_max_ctas_per_sm(defer_wait);
-    return (uint32_t)(c->sm_count * (occ > 0 ? occ : 1));
-}
-
-static uint32_t entity_views_coresident_ctas(orbit_ctx* c, uint32_t pass) {
-    int& occ = c->entity_views_occupancy[pass];
-    if (occ <= 0) occ = entity_cull_views_max_ctas_per_sm(pass);
-    return (uint32_t)(c->sm_count * (occ > 0 ? occ : 1));
-}
-
 // Every argument rule of one entity-stage call; on success, the draw range it covers. Launches nothing.
 static int entity_stage_args(orbit_ctx* c, const OrbitCullInfo* cull, const OrbitSceneBuffers* scene, const orbit_hiz* hiz,
                              void* meshlet_dispatch_buffer, uint32_t* begin, uint32_t* end) {
@@ -590,7 +614,8 @@ static int entity_launch(orbit_ctx* c, const OrbitCullInfo* cull, const OrbitSce
     EntityCullParams p = entity_params(c, cull, scene, hiz, meshlet_dispatch_buffer, capacity_records, begin, end);
     p.dispatch_mirror = (uint32_t*)mirror_dispatch_buffer;
     p.scan = next_scan(c);
-    CK(launch_entity_cull(p, end - begin, entity_coresident_ctas(c, defer_wait), (cudaStream_t)stream, defer_wait));
+    const int per_sm = occupancy(c->entity_occupancy[defer_wait ? 1 : 0], [&] { return entity_cull_max_ctas_per_sm(defer_wait); });
+    CK(launch_entity_cull(p, end - begin, (uint32_t)(c->sm_count * per_sm), (cudaStream_t)stream, defer_wait));
     c->launches += 1;
     return ORBIT_OK;
 }
@@ -670,10 +695,8 @@ static int hiz_build_entity_late(orbit_ctx* c, orbit_hiz* h, bool depth_ok, cons
     GUARD(c);
     rc = ensure_status(c, (size_t)(end - begin + 255u) / 256u + 1u, (cudaStream_t)stream);
     if (rc != ORBIT_OK) return rc;
-    HizBuildParams p = hiz_build_params(c, h, depth, h->depth_w, h->depth_h);
-    if (image) p.depth_tex = image->tex;
-    CK(launch_hiz_build(p, (cudaStream_t)stream, image != nullptr));
-    c->launches += 1;
+    rc = hiz_build_launch(c, h, depth, image, stream);
+    if (rc != ORBIT_OK) return rc;
     return entity_launch(c, late, scene, h, late_dispatch_buffer, main_dispatch_buffer, capacity_records, begin, end, stream, true);
 }
 
@@ -704,14 +727,17 @@ static void set_cull(MeshletCullParams& p, const OrbitCullInfo* cull) {
     }
 }
 
+// Emit-kernel CTAs per SM: as many as fit, at most 4
+static int emit_ctas_per_sm(orbit_ctx* c) {
+    const int per_sm = occupancy(c->emit_occupancy, meshlet_emit_max_ctas_per_sm);
+    return per_sm > 4 ? 4 : per_sm;
+}
+
 // Emit grid for a dispatch buffer of max_records records; *small_grid = the CTAs that take part when the list is short.
 static uint64_t emit_grids(orbit_ctx* c, uint64_t max_records, uint32_t* small_grid) {
-    // emit kernel: two CTAs per SM (every CTA repeats the 2048-entry chunk scan; more CTAs only add to that)
-    if (c->emit_occupancy <= 0) c->emit_occupancy = meshlet_emit_max_ctas_per_sm();
-    // emit kernel: as many CTAs per SM as fit (3) for long lists; two per SM take part when the list is short (decided on the
-    // device from the survivor count, see meshlet_emit_body)
-    int emit_per_sm = c->emit_occupancy > 0 ? c->emit_occupancy : 1;
-    if (emit_per_sm > 4) emit_per_sm = 4;
+    // as many CTAs per SM as fit (3) for long lists; two per SM take part when the list is short (decided on the device from
+    // the survivor count, see meshlet_emit_body): every CTA repeats the 2048-entry chunk scan, more CTAs only add to that
+    int emit_per_sm = emit_ctas_per_sm(c);
     // even CTAs that leave at once cost launch time (C2 frame: +1.6 us over its three emit launches), so a dispatch buffer too
     // small for a long list (capacity below 2^18 records = 8 M meshlets) gets the two per SM of the short case outright
     if (max_records < (1u << 18) && emit_per_sm > 2) emit_per_sm = 2;
@@ -719,6 +745,35 @@ static uint64_t emit_grids(orbit_ctx* c, uint64_t max_records, uint32_t* small_g
     if (c->emit_ctas_per_sm >= 1 && c->emit_ctas_per_sm <= c->emit_occupancy) emit_per_sm = emit_small_per_sm = c->emit_ctas_per_sm;   // tuning knob
     *small_grid = (uint32_t)(c->sm_count * emit_small_per_sm);
     return (uint64_t)c->sm_count * (uint64_t)emit_per_sm;
+}
+
+// One list's slice of context scratch: record entries, their side words (nullptr: the entries carry flag 1 and whoever emits
+// reads the meshlet itself), list words and chunk counts
+struct MeshletScratch { uint4* draw_masks; uint4* cmd_side; uint32_t* words; uint32_t* chunk_counts; };
+
+// The fields every meshlet-stage launch fills. cull == nullptr: an emit-only launch (orbit_draws_from_masks), which reads no
+// CullInfo, pyramid, entity, material or visibility data.
+static MeshletCullParams meshlet_params(orbit_ctx* c, const OrbitCullInfo* cull, const OrbitSceneBuffers* scene, const orbit_hiz* hiz,
+                                        const void* dispatch_buffer, uint64_t capacity_records, void* draw_command_buffer,
+                                        uint64_t capacity_draws, void* task_payloads, const MeshletScratch& s) {
+    MeshletCullParams p{};
+    if (cull) {
+        set_cull(p, cull);
+        p.hiz = hiz_device(hiz);
+        p.entities = (const float4*)scene->entities;
+        p.materials = (const uint8_t*)scene->materials;
+        p.meshlet_visibility = scene->meshlet_visibility;
+    }
+    p.meshlets = (const uint4*)scene->meshlets;
+    p.dispatch_words = (const uint32_t*)dispatch_buffer;
+    p.draw_words = (uint32_t*)draw_command_buffer;
+    p.task_payloads = (uint32_t*)task_payloads;
+    p.overflow_flag = &c->status_dev->draw_overflow;
+    p.draw_masks = s.draw_masks; p.cmd_side = s.cmd_side;
+    p.draw_total = s.words; p.chunk_parity = s.words + 2; p.chunk_counts = s.chunk_counts;
+    p.capacity_records = capacity_records;
+    p.capacity_draws = capacity_draws;
+    return p;
 }
 
 // mode 0: test + emit (orbit_meshlet_cull); mode 1: test only, record entries into `record_masks` (orbit_meshlet_test)
@@ -747,50 +802,21 @@ static int meshlet_stage(orbit_ctx* c, const OrbitCullInfo* cull, const OrbitSce
         rc = ensure_main_masks(c, max_records);
         if (rc != ORBIT_OK) return rc;
     }
-    MeshletCullParams p{};
-    p.hiz = hiz_device(hiz);
-    p.dispatch_words = (const uint32_t*)meshlet_dispatch_buffer;
-    p.meshlets = (const uint4*)scene->meshlets;
-    p.entities = (const float4*)scene->entities;
-    p.materials = (const uint8_t*)scene->materials;
-    p.meshlet_visibility = scene->meshlet_visibility;
-    p.draw_words = (uint32_t*)draw_command_buffer;
-    p.task_payloads = (uint32_t*)task_payloads;
-    p.overflow_flag = &c->status_dev->draw_overflow;
-    if (!test_only) {
-        p.draw_masks = c->draw_masks;
-        p.cmd_side = c->cmd_side;
-        p.draw_total = c->counters + 4;     // [4],[5]
-        p.chunk_parity = c->counters + 6;   // [6] word A, [7] word B
-        p.chunk_counts = c->chunk_counts;
-    } else {
-        // the survivor counters of a test-only call are never read: they go to a second set of scratch words, so that
-        // they cannot leak into a later orbit_meshlet_cull / orbit_draws_from_masks of this context
-        p.draw_masks = (uint4*)record_masks;
-        p.cmd_side = nullptr;               // entries carry flag 1: whoever emits reads the meshlet itself
-        p.draw_total = c->counters + 10;    // [10],[11]
-        p.chunk_parity = c->counters + 12;  // [12],[13]
-        p.chunk_counts = c->chunk_counts + 2 * 2048;
-    }
+    const MeshletScratch s = test_only
+        ? MeshletScratch{(uint4*)record_masks, nullptr, c->counters + kTestWords.at, c->chunk_counts + kTestChunks.at}
+        : MeshletScratch{c->draw_masks, c->cmd_side, c->counters + kMeshletWords.at, c->chunk_counts + kMeshletChunks.at};
+    MeshletCullParams p = meshlet_params(c, cull, scene, hiz, meshlet_dispatch_buffer, max_records, draw_command_buffer, capacity_draws,
+                                         task_payloads, s);
     if (fused_main) {
         p.main_masks = c->main_masks;
-        p.main_chunk_counts = c->chunk_counts + 4 * 2048;
-        p.main_chunk_parity = c->counters + 22;   // [22] word A, [23] word B
-        p.main_draw_total = c->counters + 20;     // [20],[21]
+        p.main_chunk_counts = c->chunk_counts + kMainChunks.at;
+        p.main_draw_total = c->counters + kMainWords.at;
+        p.main_chunk_parity = p.main_draw_total + 2;
         p.main_alpha_mode_flags = fused_main->cull->alpha_mode_flags;
     }
-    p.capacity_records = max_records;
-    p.capacity_draws = capacity_draws;
     p.scan.trace = next_trace(c);
     p.trace_emit = next_trace(c);
-    set_cull(p, cull);
-    // test kernel: persistent warps, cyclic tiles, no inter-CTA dependency -> one full wave of CTAs
-    int& occ_slot = c->mc_occupancy[meshlet_cull_variant_index(*cull)];
-    if (occ_slot <= 0) occ_slot = meshlet_cull_max_ctas_per_sm(p);
-    const int occ = occ_slot;
-    int per_sm = c->mc_ctas_per_sm;
-    if (per_sm <= 0) per_sm = occ > 0 ? occ : 1;
-    const uint64_t grid = (uint64_t)c->sm_count * (uint64_t)per_sm;
+    const uint64_t grid = test_grid(c, c->mc_occupancy[meshlet_cull_variant_index(*cull)], [&] { return meshlet_cull_max_ctas_per_sm(p); });
     uint32_t emit_small_grid;
     const uint64_t emit_grid = emit_grids(c, max_records, &emit_small_grid);
     p.emit_small_grid = emit_small_grid;
@@ -856,25 +882,16 @@ int orbit_draws_from_masks(orbit_ctx* c, const OrbitSceneBuffers* scene, const v
     if (((uintptr_t)record_masks & 15u) || ((uintptr_t)draw_command_buffer & 3u) || ((uintptr_t)scene->meshlets & 15u)) return ORBIT_ERR_INVALID_ARGUMENT;
     if (region_stride_records > 0xFFFFFFFFull) return ORBIT_ERR_INVALID_ARGUMENT;
     GUARD(c);
-    MeshletCullParams p{};
-    p.meshlets = (const uint4*)scene->meshlets;
-    p.draw_words = (uint32_t*)draw_command_buffer;
-    p.overflow_flag = &c->status_dev->draw_overflow;
-    p.draw_masks = (uint4*)record_masks;      // read only on this path
-    p.cmd_side = nullptr;
-    p.draw_total = c->counters + 4;
-    p.chunk_parity = c->counters + 6;
-    p.chunk_counts = c->chunk_counts;
-    p.capacity_records = 0xFFFFFFFFull;
-    p.capacity_draws = capacity_draws;
-    p.dispatch_words = c->counters + 16;      // a 3-word dispatch header written by the recount kernel
+    uint32_t* const header = c->counters + kDrawsHeader.at;
+    // record_masks is read only on this path; the survivors are counted in orbit_meshlet_cull's list words and chunk counts
+    MeshletCullParams p = meshlet_params(c, nullptr, scene, nullptr, header, 0xFFFFFFFFull, draw_command_buffer, capacity_draws, nullptr,
+                                         MeshletScratch{(uint4*)record_masks, nullptr, c->counters + kMeshletWords.at,
+                                                        c->chunk_counts + kMeshletChunks.at});
     p.region_counts = region_counts; p.region_stride = region_stride_records; p.n_regions = n_regions;
     p.trace_emit = next_trace(c);
-    if (c->emit_occupancy <= 0) c->emit_occupancy = meshlet_emit_max_ctas_per_sm();
-    int emit_per_sm = c->emit_occupancy > 0 ? c->emit_occupancy : 1;
-    if (emit_per_sm > 4) emit_per_sm = 4;
+    const int emit_per_sm = emit_ctas_per_sm(c);
     p.emit_small_grid = (uint32_t)(c->sm_count * (emit_per_sm < 2 ? emit_per_sm : 2));
-    CK(launch_draws_from_masks(p, c->counters + 16, c->sm_count * 4, c->sm_count * emit_per_sm, (cudaStream_t)stream));
+    CK(launch_draws_from_masks(p, header, c->sm_count * 4, c->sm_count * emit_per_sm, (cudaStream_t)stream));
     c->launches += 2;
     return ORBIT_OK;
 }
@@ -903,13 +920,12 @@ static int check_views(const OrbitCullInfo* culls, uint32_t n_views, const Orbit
     return check_view_buffers(buffers, n_views);
 }
 
-int orbit_entity_cull_views(orbit_ctx* c, const OrbitCullInfo* culls, uint32_t n_views, const OrbitSceneBuffers* scene,
-                            void* const* dispatch_buffers, uint64_t capacity_records, void* stream) {
-    if (!c) return ORBIT_ERR_INVALID_ARGUMENT;
-    int rc = check_views(culls, n_views, scene, (const void* const*)dispatch_buffers, false);
-    if (rc != ORBIT_OK) return rc;
+// The entity stage of both batched forms, after their own checks: view v reads scenes[v] (per_view_scene) or scenes[0], and
+// the pyramid hizs[v] (pass 2; NULL otherwise).
+static int entity_views_stage(orbit_ctx* c, const OrbitCullInfo* culls, uint32_t n_views, const OrbitSceneBuffers* scenes, bool per_view_scene,
+                              const orbit_hiz* const* hizs, void* const* dispatch_buffers, uint64_t capacity_records, void* stream) {
     uint32_t begin, end;
-    rc = draw_range(scene, &begin, &end);
+    int rc = draw_range(scenes, &begin, &end);
     if (rc != ORBIT_OK) return rc;
     const uint32_t n = end - begin;
     GUARD(c);
@@ -917,11 +933,23 @@ int orbit_entity_cull_views(orbit_ctx* c, const OrbitCullInfo* culls, uint32_t n
     if (rc != ORBIT_OK) return rc;
     EntityViewsParams pv{};
     pv.n_views = n_views;
-    for (uint32_t v = 0; v < n_views; ++v) pv.view[v] = entity_params(c, &culls[v], scene, nullptr, dispatch_buffers[v], capacity_records, begin, end);
+    for (uint32_t v = 0; v < n_views; ++v)
+        pv.view[v] = entity_params(c, &culls[v], per_view_scene ? &scenes[v] : scenes, hizs ? hizs[v] : nullptr, dispatch_buffers[v],
+                                   capacity_records, begin, end);
     pv.view[0].scan = next_scan(c);
-    CK(launch_entity_cull_views(pv, n, entity_views_coresident_ctas(c, 0u), (cudaStream_t)stream));
+    const uint32_t pass = culls[0].occlusion_pass;
+    const int per_sm = occupancy(c->entity_views_occupancy[pass], [&] { return entity_cull_views_max_ctas_per_sm(pass); });
+    CK(launch_entity_cull_views(pv, n, (uint32_t)(c->sm_count * per_sm), (cudaStream_t)stream));
     c->launches += 1;
     return ORBIT_OK;
+}
+
+int orbit_entity_cull_views(orbit_ctx* c, const OrbitCullInfo* culls, uint32_t n_views, const OrbitSceneBuffers* scene,
+                            void* const* dispatch_buffers, uint64_t capacity_records, void* stream) {
+    if (!c) return ORBIT_ERR_INVALID_ARGUMENT;
+    int rc = check_views(culls, n_views, scene, (const void* const*)dispatch_buffers, false);
+    if (rc != ORBIT_OK) return rc;
+    return entity_views_stage(c, culls, n_views, scene, false, nullptr, dispatch_buffers, capacity_records, stream);
 }
 
 // The meshlet stage of both batched forms, after their own checks: view v reads scenes[v] (per_view_scene) or scenes[0], and
@@ -960,34 +988,17 @@ static int meshlet_views_stage(orbit_ctx* c, const OrbitCullInfo* culls, uint32_
     MeshletViewsParams pv{};
     pv.n_views = n_views;
     for (uint32_t v = 0; v < n_views; ++v) {
-        MeshletCullParams& p = pv.view[v];
-        const OrbitSceneBuffers* scene = per_view_scene ? &scenes[v] : scenes;
-        set_cull(p, &culls[v]);
-        p.hiz = hiz_device(hizs ? hizs[v] : nullptr);
-        p.dispatch_words = (const uint32_t*)dispatch_buffers[v];
-        p.meshlets = (const uint4*)scene->meshlets;
-        p.entities = (const float4*)scene->entities;
-        p.materials = (const uint8_t*)scene->materials;
-        p.meshlet_visibility = scene->meshlet_visibility;
-        p.draw_words = (uint32_t*)draw_command_buffers[v];
-        p.task_payloads = task_payloads ? (uint32_t*)task_payloads[v] : nullptr;
-        p.overflow_flag = &c->status_dev->draw_overflow;
-        p.draw_masks = c->draw_masks + (size_t)v * capacity_records;
-        p.cmd_side = c->cmd_side + (size_t)v * capacity_records * 32u;
-        p.chunk_counts = c->view_counters + v * kViewChunkWords;
-        p.draw_total = c->view_counters + ORBIT_MAX_BATCH_VIEWS * kViewChunkWords + 4u * v;   // [0],[1]
-        p.chunk_parity = p.draw_total + 2;                                                   // [2] word A, [3] word B
-        p.capacity_records = capacity_records;
-        p.capacity_draws = capacity_draws;
-        p.emit_small_grid = small_per_view;
+        const MeshletScratch s{c->draw_masks + (size_t)v * capacity_records, c->cmd_side + (size_t)v * capacity_records * 32u,
+                               c->view_counters + kViewWords.at + v * kListWords, c->view_counters + kViewChunks.at + v * kChunkWords};
+        pv.view[v] = meshlet_params(c, &culls[v], per_view_scene ? &scenes[v] : scenes, hizs ? hizs[v] : nullptr, dispatch_buffers[v],
+                                    capacity_records, draw_command_buffers[v], capacity_draws, task_payloads ? task_payloads[v] : nullptr, s);
+        pv.view[v].emit_small_grid = small_per_view;
     }
     pv.view[0].scan.trace = next_trace(c);
     pv.view[0].trace_emit = next_trace(c);
-    int& occ_slot = c->views_occupancy[meshlet_cull_variant_index(culls[0])];
-    if (occ_slot <= 0) occ_slot = meshlet_cull_views_max_ctas_per_sm(culls[0]);
-    int per_sm = c->mc_ctas_per_sm;
-    if (per_sm <= 0) per_sm = occ_slot > 0 ? occ_slot : 1;
-    CK(launch_meshlet_cull_views(pv, c->sm_count * per_sm, (int)emit_per_view, (cudaStream_t)stream));
+    const uint64_t grid = test_grid(c, c->views_occupancy[meshlet_cull_variant_index(culls[0])],
+                                    [&] { return meshlet_cull_views_max_ctas_per_sm(culls[0]); });
+    CK(launch_meshlet_cull_views(pv, (int)grid, (int)emit_per_view, (cudaStream_t)stream));
     c->launches += 2;
     return ORBIT_OK;
 }
@@ -1022,7 +1033,7 @@ static int check_views_occlusion(const OrbitCullInfo* culls, uint32_t n_views, c
         if (pass == 2u) {
             if (!h || h->info.width != hizs[0]->info.width || h->info.height != hizs[0]->info.height || h->info.levels != hizs[0]->info.levels)
                 return ORBIT_ERR_INVALID_ARGUMENT;
-            for (uint32_t u = 0; u < v; ++u) if (hizs[u]->info.texels == h->info.texels) return ORBIT_ERR_INVALID_ARGUMENT;
+            if (!pyramid_distinct(hizs, v)) return ORBIT_ERR_INVALID_ARGUMENT;
         }
         int rc = check_cull(&ci, &scenes[v], h, meshlet_stage);
         if (rc != ORBIT_OK) return rc;
@@ -1042,21 +1053,8 @@ int orbit_entity_cull_views_occlusion(orbit_ctx* c, const OrbitCullInfo* culls, 
     if (!c) return ORBIT_ERR_INVALID_ARGUMENT;
     int rc = check_views_occlusion(culls, n_views, scenes, hizs, (const void* const*)dispatch_buffers, false);
     if (rc != ORBIT_OK) return rc;
-    uint32_t begin, end;
-    rc = draw_range(&scenes[0], &begin, &end);
-    if (rc != ORBIT_OK) return rc;
-    const uint32_t n = end - begin, pass = culls[0].occlusion_pass;
-    GUARD(c);
-    rc = ensure_status(c, (size_t)n_views * ((n + 255u) / 256u + 1u), (cudaStream_t)stream);   // one descriptor block per view
-    if (rc != ORBIT_OK) return rc;
-    EntityViewsParams pv{};
-    pv.n_views = n_views;
-    for (uint32_t v = 0; v < n_views; ++v)
-        pv.view[v] = entity_params(c, &culls[v], &scenes[v], pass == 2u ? hizs[v] : nullptr, dispatch_buffers[v], capacity_records, begin, end);
-    pv.view[0].scan = next_scan(c);
-    CK(launch_entity_cull_views(pv, n, entity_views_coresident_ctas(c, pass), (cudaStream_t)stream));
-    c->launches += 1;
-    return ORBIT_OK;
+    return entity_views_stage(c, culls, n_views, scenes, true, culls[0].occlusion_pass == 2u ? hizs : nullptr, dispatch_buffers,
+                              capacity_records, stream);
 }
 
 int orbit_meshlet_cull_views_occlusion(orbit_ctx* c, const OrbitCullInfo* culls, uint32_t n_views, const OrbitSceneBuffers* scenes,
@@ -1194,7 +1192,7 @@ int orbit_scene_update(orbit_ctx* c, const OrbitSceneUpdate* u, void* stream) {
     SceneUpdateParams p{};
     p.transforms = (const uint8_t*)u->transforms; p.mesh_slots = u->mesh_slots; p.visibility_offsets = u->visibility_offsets;
     p.mesh_infos = (const uint8_t*)u->mesh_infos; p.visibility_cursor = u->visibility_cursor;
-    p.cursor_snapshot = c->counters + 8; p.tile_sums = c->tile_sums;
+    p.cursor_snapshot = c->counters + kCursorSnapshot.at; p.tile_sums = c->tile_sums;
     p.entity_data = (float4*)u->entity_data; p.entity_draw_words = (uint32_t*)u->entity_draws;
     p.overflow_flag = &c->status_dev->visibility_overflow;
     p.n_entities = u->n_entities; p.visibility_capacity_words = u->visibility_capacity_words;
@@ -1407,7 +1405,7 @@ int orbit_peer_put(orbit_ctx* c, const OrbitPeerPut* puts, uint32_t n_puts, uint
         if (p.n16[i] > largest) largest = p.n16[i];
     }
     p.flag_value = flag_value;
-    p.done = c->counters + 24;                 // [24..39]: CTAs that have finished, per transfer (self-resetting)
+    p.done = c->counters + kPeerDone.at;
     GUARD(c);
     uint64_t gx = (largest + 1023u) / 1024u;   // four 16-byte stores per thread
     const uint64_t cap = (uint64_t)c->sm_count * 8u / n_puts;
