@@ -326,6 +326,50 @@ int  orbit_light_cluster_image(orbit_ctx* ctx, const OrbitClusterParams* params,
                                void* offset_count_image, void* light_index_list, uint64_t capacity_indices,
                                void* stream);
 
+/* ---- outputs into images (the depth pyramid and the cluster grid imported from Vulkan) -------------------------------------
+ * The reference keeps the depth pyramid in an R32_SFLOAT image with one mip per level (draw_gen.rs:451-567), which its task
+ * shaders and Hi-Z viewer sample, and the cluster offset/count grid in a 3-D R32G32_UINT image (cluster.rs:532-544), which
+ * forward.frag reads. Imported into CUDA they are (mipmapped) arrays; these calls write them directly, so no buffer-to-image
+ * copy pass per frame and camera is needed.
+ *
+ * orbit_hiz_attach_image: `cuda_mipmapped_array` is a caller-owned cudaMipmappedArray_t (passed as void*), e.g. one mapped from
+ * an imported VkImage with cudaExternalMemoryGetMappedMipmappedArray. From then on every build of `hiz` also stores each level
+ * l into level l of the array, byte for byte the linear level: orbit_hiz_build, orbit_hiz_build_image, orbit_hiz_build_views
+ * (_image) and orbit_hiz_build(_image)_entity_cull_late. The linear pyramid is still written and stays what every culling
+ * call reads (and what orbit_peer_put moves); the array is a write-only mirror that no call reads back.
+ *   - refused with ORBIT_ERR_INVALID_ARGUMENT, leaving no CUDA error behind: a NULL argument, a pyramid of another device, a
+ *     second attach to the same pyramid (there is no detach: the mirror lives as long as the pyramid), and an array that is
+ *     not exactly the pyramid: level l < info.levels must exist with extent max(width>>l,1) x max(height>>l,1) (depth 0), one
+ *     32-bit cudaChannelFormatKindFloat channel, created with cudaArraySurfaceLoadStore, neither layered nor a cubemap;
+ *   - the call creates one surface object per level and allocates nothing on the device. orbit_hiz_destroy releases them,
+ *     never the array. Destroying the pyramid, or freeing the array, while enqueued work or a captured CUDA graph still
+ *     writes it is the caller's error;
+ *   - batched builds: each pyramid mirrors only if it has an array of its own (mixed batches are fine); two pyramids of one
+ *     call with the same array are refused;
+ *   - calls enqueued before the attach do not write the mirror. The surface handles travel in the kernel parameters: a
+ *     captured graph writes the array that was attached at capture time;
+ *   - a pyramid that arrives by orbit_peer_put (the ranks of a sharded view) is not rebuilt there, so its mirror is not written;
+ *   - synchronisation: the mirror is written on the build's stream; ordering the renderer's reads after it (an imported
+ *     Vulkan semaphore signalled on that stream with cudaSignalExternalSemaphoresAsync) is the caller's job.
+ *
+ * orbit_cluster_grid_wrap: `cuda_array` is a caller-owned 3-D cudaArray_t (extent depth >= 1) with two 32-bit
+ * cudaChannelFormatKindUnsigned channels (x = y = 32, z = w = 0), created with cudaArraySurfaceLoadStore, neither layered nor
+ * a cubemap; anything else, NULL included, is ORBIT_ERR_INVALID_ARGUMENT. The call creates one surface object and allocates
+ * nothing on the device; orbit_cluster_grid_destroy releases it, never the array (lifetime rules as above).
+ * orbit_light_cluster_image_grid: orbit_light_cluster_image with the offset/count grid written into `grid` instead of a
+ * linear buffer. Texel (x, y, z), idx = (z*cy + y)*cx + x, holds exactly the two words orbit_light_cluster_image writes at
+ * idx; inactive clusters hold (0, 0). Every texel is written by every call, so nothing of a previous frame survives. Every
+ * argument rule of orbit_light_cluster_image applies, and the grid's extent must equal params->info.cluster_count; a refused
+ * call launches nothing. Counts as an orbit_light_cluster call (concurrency rules at the top). */
+int  orbit_hiz_attach_image(orbit_ctx* ctx, orbit_hiz* hiz, void* cuda_mipmapped_array);
+typedef struct orbit_cluster_grid orbit_cluster_grid;
+int  orbit_cluster_grid_wrap(orbit_ctx* ctx, void* cuda_array, orbit_cluster_grid** out);
+void orbit_cluster_grid_destroy(orbit_cluster_grid* grid);
+int  orbit_light_cluster_image_grid(orbit_ctx* ctx, const OrbitClusterParams* params, const orbit_depth_image* image,
+                                    const void* lights, void* tile_masks, void* depth_bounds, void* unique_clusters,
+                                    const orbit_cluster_grid* grid, void* light_index_list, uint64_t capacity_indices,
+                                    void* stream);
+
 /* ---- SceneData::update_scene (scene.rs:404-492), the per-frame producer of the entity buffers the culling path
  *      reads (SURVEY §8f item 3). For every entity with a mesh, in entity order: instance_index = running count,
  *      GpuEntityData {model_matrix = Mat4::from_scale_rotation_translation(scale, orientation, position),

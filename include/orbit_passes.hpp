@@ -163,6 +163,9 @@ public:
     void update(const float* depth_buffer, void* stream) { check(orbit_hiz_build(ctx_, hiz_, depth_buffer, w_, h_, stream), "DepthPyramid::update"); usable = true; }
     // the depth attachment as a wrapped CUDA array (orbit_depth_image_wrap), e.g. imported from Vulkan
     void update(const orbit_depth_image* depth_image, void* stream) { check(orbit_hiz_build_image(ctx_, hiz_, depth_image, stream), "DepthPyramid::update"); usable = true; }
+    // mirror every later build into a caller-owned cudaMipmappedArray_t (orbit_hiz_attach_image), e.g. the renderer's pyramid
+    // image imported from Vulkan; resize() creates a new pyramid without one (attach the new size's array then)
+    void attach_image(void* cuda_mipmapped_array) { check(orbit_hiz_attach_image(ctx_, hiz_, cuda_mipmapped_array), "DepthPyramid::attach_image"); }
     orbit_hiz* get_current() const { return hiz_; }
     bool usable = false;
 private:
@@ -194,5 +197,14 @@ struct ClusterSettings {
         z_bias = -(((float)z_slice_count * std::log2(near_)) / log_f_n);
     }
 };
+
+// compute_clusters, cluster.rs:368-397, with the depth attachment and the cluster offset/count image as wrapped CUDA arrays
+// (orbit_depth_image_wrap, orbit_cluster_grid_wrap), e.g. both imported from Vulkan: orbit_light_cluster_image_grid
+inline void compute_clusters(orbit_ctx* ctx, const OrbitClusterParams& params, const orbit_depth_image* depth_image, const void* lights,
+                             void* tile_masks, void* depth_bounds, void* unique_clusters, const orbit_cluster_grid* light_offset_image,
+                             void* light_index_list, uint64_t capacity_indices, void* stream) {
+    check(orbit_light_cluster_image_grid(ctx, &params, depth_image, lights, tile_masks, depth_bounds, unique_clusters, light_offset_image,
+                                         light_index_list, capacity_indices, stream), "compute_clusters");
+}
 
 }  // namespace orbit_host

@@ -81,6 +81,11 @@ PROTOTYPES = {
                                                          C.POINTER(L.SceneBuffers), C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p]),
     "orbit_light_cluster_image": (C.c_int, [C.c_void_p, C.POINTER(L.ClusterParams), C.c_void_p, C.c_void_p, C.c_void_p,
                                             C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p]),
+    "orbit_hiz_attach_image": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
+    "orbit_cluster_grid_wrap": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(C.c_void_p)]),
+    "orbit_cluster_grid_destroy": (None, [C.c_void_p]),
+    "orbit_light_cluster_image_grid": (C.c_int, [C.c_void_p, C.POINTER(L.ClusterParams), C.c_void_p, C.c_void_p, C.c_void_p,
+                                                 C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p]),
 }
 
 _lib = None

@@ -14,7 +14,7 @@ LIB_PATH = os.path.join(LIB_DIR, "liborbit_b200.so")
 SOURCES = ["api.cu", "hiz_build.cu", "entity_cull.cu", "meshlet_cull.cu", "light_cluster.cu", "scene_update.cu", "asset_bounds.cu"]
 HOST_LIB_PATH = os.path.join(LIB_DIR, "liborbit_host.so")   # compiled host-side frame driver above the C ABI
 HOST_SOURCES = [os.path.join(HERE, "host", "frame_driver.cpp")]
-HEADERS = ["orbit_device.cuh", "scan.cuh", "params.cuh", "../../include/orbit_cuda.h", "../../include/orbit_layouts.h"]
+HEADERS = ["orbit_device.cuh", "scan.cuh", "params.cuh", "light_culling_kernel.cuh", "../../include/orbit_cuda.h", "../../include/orbit_layouts.h"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo",
     "--fmad=false", "--prec-div=true", "--prec-sqrt=true", "--ftz=false",

@@ -147,6 +147,16 @@ struct orbit_hiz {
     uint32_t depth_w, depth_h;
     bool owns;
     int device;
+    // orbit_hiz_attach_image: the caller's mipmapped array (never freed here) and a surface per level, else NULL
+    cudaMipmappedArray_t mirror_array = nullptr;
+    HizMirror mirror{};
+};
+
+// A caller's 3-D R32G32_UINT CUDA array behind the surface object orbit_light_cluster_image_grid writes the grid through
+struct orbit_cluster_grid {
+    cudaSurfaceObject_t surf;
+    uint32_t width, height, depth;
+    int device;
 };
 
 // A caller's 2-D float CUDA array behind the texture object the *_image stage calls read it through
@@ -247,6 +257,13 @@ static HizDevice hiz_device(const orbit_hiz* h) {
 // hizs[v] shares its texels with none of hizs[0..v)
 static bool pyramid_distinct(const orbit_hiz* const* hizs, uint32_t v) {
     for (uint32_t u = 0; u < v; ++u) if (hizs[u]->info.texels == hizs[v]->info.texels) return false;
+    return true;
+}
+
+// hizs[v] shares its mirror array (if it has one) with none of hizs[0..v): a build writes it
+static bool mirror_distinct(const orbit_hiz* const* hizs, uint32_t v) {
+    if (!hizs[v]->mirror_array) return true;
+    for (uint32_t u = 0; u < v; ++u) if (hizs[u]->mirror_array == hizs[v]->mirror_array) return false;
     return true;
 }
 
@@ -420,10 +437,60 @@ static int hiz_make(orbit_ctx* c, uint32_t dw, uint32_t dh, float* texels, bool 
 int orbit_hiz_create(orbit_ctx* c, uint32_t dw, uint32_t dh, orbit_hiz** out) { return hiz_make(c, dw, dh, nullptr, true, out); }
 int orbit_hiz_wrap(orbit_ctx* c, uint32_t dw, uint32_t dh, float* texels, orbit_hiz** out) { return hiz_make(c, dw, dh, texels, false, out); }
 
+static void destroy_surfaces(const HizMirror& m, uint32_t levels) {
+    for (uint32_t l = 0; l < levels; ++l) cudaDestroySurfaceObject(m.level[l]);
+}
+
 void orbit_hiz_destroy(orbit_hiz* h) {
     if (!h) return;
-    if (h->owns) { DeviceGuard guard(h->device); cudaFree(h->info.texels); }
+    if (h->owns || h->mirror_array) {
+        DeviceGuard guard(h->device);
+        if (h->owns) cudaFree(h->info.texels);
+        if (h->mirror_array) destroy_surfaces(h->mirror, h->info.levels);   // the array stays the caller's
+    }
     delete h;
+}
+
+// True for an array whose first channel is 32 bits of `kind`, whose second has `y` bits (0 or 32) and which has no others,
+// created with surface load/store and neither layered nor a cubemap; *ext is its extent. Clears the non-sticky error a failed
+// query sets.
+static bool array_info(cudaArray_t a, cudaChannelFormatKind kind, int y, cudaExtent* ext) {
+    cudaChannelFormatDesc fmt{};
+    unsigned int flags = 0;
+    const cudaError_t e = cudaArrayGetInfo(&fmt, ext, &flags, a);
+    if (e != cudaSuccess) { g_last_cuda_error = (int)e; cudaGetLastError(); return false; }
+    if (fmt.f != kind || fmt.x != 32 || fmt.y != y || fmt.z != 0 || fmt.w != 0) return false;
+    return (flags & cudaArraySurfaceLoadStore) != 0u && (flags & (cudaArrayLayered | cudaArrayCubemap)) == 0u;
+}
+
+static cudaError_t make_surface(cudaArray_t a, cudaSurfaceObject_t* out) {
+    cudaResourceDesc res{};
+    res.resType = cudaResourceTypeArray;
+    res.res.array.array = a;
+    return cudaCreateSurfaceObject(out, &res);
+}
+
+int orbit_hiz_attach_image(orbit_ctx* c, orbit_hiz* h, void* cuda_mipmapped_array) {
+    if (!c || !h || !cuda_mipmapped_array || h->device != c->device || h->mirror_array) return ORBIT_ERR_INVALID_ARGUMENT;
+    GUARD(c);
+    const cudaMipmappedArray_t mm = static_cast<cudaMipmappedArray_t>(cuda_mipmapped_array);
+    cudaArray_t level[ORBIT_HIZ_MAX_LEVELS] = {};
+    for (uint32_t l = 0; l < h->info.levels; ++l) {
+        const cudaError_t e = cudaGetMipmappedArrayLevel(&level[l], mm, l);
+        if (e != cudaSuccess) { g_last_cuda_error = (int)e; cudaGetLastError(); return ORBIT_ERR_INVALID_ARGUMENT; }
+        cudaExtent ext{};
+        if (!array_info(level[l], cudaChannelFormatKindFloat, 0, &ext)) return ORBIT_ERR_INVALID_ARGUMENT;
+        const uint32_t w = h->info.width >> l, hh = h->info.height >> l;
+        if (ext.width != (w ? w : 1u) || ext.height != (hh ? hh : 1u) || ext.depth != 0) return ORBIT_ERR_INVALID_ARGUMENT;
+    }
+    HizMirror m{};
+    for (uint32_t l = 0; l < h->info.levels; ++l) {
+        const cudaError_t e = make_surface(level[l], &m.level[l]);
+        if (e != cudaSuccess) { g_last_cuda_error = (int)e; destroy_surfaces(m, l); return ORBIT_ERR_CUDA; }
+    }
+    h->mirror = m;
+    h->mirror_array = mm;
+    return ORBIT_OK;
 }
 
 int orbit_hiz_info(const orbit_hiz* h, OrbitHizInfo* out) {
@@ -446,7 +513,7 @@ static int hiz_build_launch(orbit_ctx* c, const orbit_hiz* h, const float* depth
     set_pyramid(p, h);
     p.ticket = c->counters + kHizTicket.at;
     p.trace = next_trace(c);
-    CK(launch_hiz_build(p, (cudaStream_t)stream, image != nullptr));
+    CK(launch_hiz_build(p, (cudaStream_t)stream, image != nullptr, h->mirror_array ? &h->mirror : nullptr));
     c->launches += 1;
     return ORBIT_OK;
 }
@@ -465,9 +532,11 @@ static int hiz_build_views(orbit_ctx* c, orbit_hiz* const* hizs, const float* co
     for (uint32_t v = 0; v < n_views; ++v) {
         const orbit_hiz* h = hizs[v];
         if (!h || (depths && !depths[v]) || dw != h->depth_w || dh != h->depth_h || !pyramid_distinct(hizs, v)) return ORBIT_ERR_INVALID_ARGUMENT;
+        if (!mirror_distinct(hizs, v)) return ORBIT_ERR_INVALID_ARGUMENT;
     }
     GUARD(c);
     HizBuildViewsParams pv{};
+    HizMirrorViews mv{};
     pv.n_views = n_views;
     for (uint32_t v = 0; v < n_views; ++v) {
         HizBuildParams& p = pv.view[v];
@@ -476,9 +545,10 @@ static int hiz_build_views(orbit_ctx* c, orbit_hiz* const* hizs, const float* co
         p.depth_w = dw; p.depth_h = dh;
         set_pyramid(p, hizs[v]);
         p.ticket = c->counters + kHizViewTickets.at + v;
+        if (hizs[v]->mirror_array) { mv.view[v] = hizs[v]->mirror; mv.mirrored |= 1u << v; }
     }
     pv.view[0].trace = next_trace(c);
-    CK(launch_hiz_build_views(pv, (cudaStream_t)stream, depths == nullptr));
+    CK(launch_hiz_build_views(pv, (cudaStream_t)stream, depths == nullptr, mv.mirrored ? &mv : nullptr));
     c->launches += 1;
     return ORBIT_OK;
 }
@@ -1069,15 +1139,17 @@ int orbit_meshlet_cull_views_occlusion(orbit_ctx* c, const OrbitCullInfo* culls,
 }
 
 // ---- clustered lights ------------------------------------------------------------------------------------
-// Depth from `image` when it is not NULL (orbit_light_cluster_image), else from `depth`.
+// Depth from `image` when it is not NULL (orbit_light_cluster_image), else from `depth`. The offset / count grid goes to
+// `out_grid` when it is not NULL (orbit_light_cluster_image_grid), else to `offset_count_image`.
 static int light_cluster(orbit_ctx* c, const OrbitClusterParams* params, const float* depth, const orbit_depth_image* image,
                          const void* lights, void* tile_masks, void* depth_bounds, void* unique_clusters, void* offset_count_image,
-                         void* light_index_list, uint64_t capacity_indices, void* stream) {
-    if (!c || !params || !(depth || image) || !tile_masks || !depth_bounds || !unique_clusters || !offset_count_image || !light_index_list)
+                         const orbit_cluster_grid* out_grid, void* light_index_list, uint64_t capacity_indices, void* stream) {
+    if (!c || !params || !(depth || image) || !tile_masks || !depth_bounds || !unique_clusters || !(offset_count_image || out_grid) || !light_index_list)
         return ORBIT_ERR_INVALID_ARGUMENT;
     const OrbitClusterCullInfo& ci = params->info;
     if (image && !image_ok(c, image, ci.screen_size[0], ci.screen_size[1])) return ORBIT_ERR_INVALID_ARGUMENT;
     const uint64_t cx = ci.cluster_count[0], cy = ci.cluster_count[1], cz = ci.cluster_count[2];
+    if (out_grid && (out_grid->device != c->device || out_grid->width != cx || out_grid->height != cy || out_grid->depth != cz)) return ORBIT_ERR_INVALID_ARGUMENT;
     if (cx == 0 || cy == 0 || cz == 0 || cx * cy * cz > 0x7FFFFFFFull || ci.tile_size_px == 0) return ORBIT_ERR_INVALID_ARGUMENT;
     if (ci.screen_size[0] == 0 || ci.screen_size[1] == 0) return ORBIT_ERR_INVALID_ARGUMENT;
     // every pixel must map to a tile inside the grid (cluster.rs:41-43 derives counts with div_ceil)
@@ -1100,7 +1172,9 @@ static int light_cluster(orbit_ctx* c, const OrbitClusterParams* params, const f
     else p.depth = depth;
     p.lights = (const uint8_t*)lights; p.light_view = c->light_view;
     p.tile_masks = (uint32_t*)tile_masks; p.depth_bounds = (uint32_t*)depth_bounds;
-    p.unique_clusters = (uint32_t*)unique_clusters; p.offset_count_image = (uint32_t*)offset_count_image;
+    p.unique_clusters = (uint32_t*)unique_clusters;
+    if (out_grid) p.offset_count_surf = out_grid->surf;
+    else p.offset_count_image = (uint32_t*)offset_count_image;
     p.light_index_words = (uint32_t*)light_index_list; p.overflow_flag = &c->status_dev->light_index_overflow;
     p.capacity_indices = capacity_indices;
     // scratch of the light-parallel path: [boxes: 8 words per cluster][bit matrix][block counts][hit totals: 1 word per cluster]
@@ -1109,14 +1183,14 @@ static int light_cluster(orbit_ctx* c, const OrbitClusterParams* params, const f
     // fill_buffer(.., 0) of masks and bounds: cluster.rs:447-450; inactive image texels are zeroed (unspecified in the reference)
     CK(cudaMemsetAsync(tile_masks, 0, cx * cy * 4u, s));
     CK(cudaMemsetAsync(depth_bounds, 0, clusters * 8u, s));
-    CK(cudaMemsetAsync(offset_count_image, 0, clusters * 8u, s));
+    if (!out_grid) CK(cudaMemsetAsync(offset_count_image, 0, clusters * 8u, s));   // the grid's inactive texels: the compaction kernel
     const uint64_t warps = (uint64_t)((ci.screen_size[0] + 31u) / 32u) * ((ci.screen_size[1] + 3u) / 4u);
     uint64_t grid = (warps + 7u) / 8u;
     const uint64_t cap_grid = (uint64_t)c->sm_count * 8u;
     if (grid > cap_grid) grid = cap_grid;
     CK(launch_mark_active(p, (int)grid, s, image != nullptr));
     p.scan = next_scan(c);
-    CK(launch_compact_clusters(p, s));
+    CK(launch_compact_clusters(p, s, out_grid != nullptr));
     if (light_parallel) {
         const uint32_t wpc = light_hits_blocks(L) * 16u;   // row stride of the bit matrix (64-byte aligned rows)
         uint32_t* const hit_rows = c->light_hits + clusters * 8u;
@@ -1125,7 +1199,7 @@ static int light_cluster(orbit_ctx* c, const OrbitClusterParams* params, const f
         uint64_t lgrid = (clusters + 31u) / 32u;     // a warp per active cluster, 32 per CTA, persistent over tiles
         const uint64_t lcap = (uint64_t)c->sm_count * 2u;
         if (lgrid > lcap) lgrid = lcap;
-        CK(launch_light_lists(p, hit_rows, block_counts, wpc, (int)lgrid, s));
+        CK(launch_light_lists(p, hit_rows, block_counts, wpc, (int)lgrid, s, out_grid != nullptr));
         c->launches += 4;
     } else {
         CK(launch_light_view(p, s));
@@ -1133,7 +1207,7 @@ static int light_cluster(orbit_ctx* c, const OrbitClusterParams* params, const f
         uint64_t lgrid = clusters;                   // one CTA per active cluster, persistent: at most 2 x 1024 threads per SM
         const uint64_t lcap = (uint64_t)c->sm_count * 2u;
         if (lgrid > lcap) lgrid = lcap;
-        CK(launch_light_culling(p, (int)lgrid, s));
+        CK(launch_light_culling(p, (int)lgrid, s, out_grid != nullptr));
         c->launches += (L ? 4 : 3);
     }
     return ORBIT_OK;
@@ -1143,7 +1217,7 @@ int orbit_light_cluster(orbit_ctx* c, const OrbitClusterParams* params, const fl
                         void* tile_masks, void* depth_bounds, void* unique_clusters, void* offset_count_image,
                         void* light_index_list, uint64_t capacity_indices, void* stream) {
     if (!depth) return ORBIT_ERR_INVALID_ARGUMENT;
-    return light_cluster(c, params, depth, nullptr, lights, tile_masks, depth_bounds, unique_clusters, offset_count_image,
+    return light_cluster(c, params, depth, nullptr, lights, tile_masks, depth_bounds, unique_clusters, offset_count_image, nullptr,
                          light_index_list, capacity_indices, stream);
 }
 
@@ -1151,7 +1225,41 @@ int orbit_light_cluster_image(orbit_ctx* c, const OrbitClusterParams* params, co
                               void* tile_masks, void* depth_bounds, void* unique_clusters, void* offset_count_image,
                               void* light_index_list, uint64_t capacity_indices, void* stream) {
     if (!image) return ORBIT_ERR_INVALID_ARGUMENT;
-    return light_cluster(c, params, nullptr, image, lights, tile_masks, depth_bounds, unique_clusters, offset_count_image,
+    return light_cluster(c, params, nullptr, image, lights, tile_masks, depth_bounds, unique_clusters, offset_count_image, nullptr,
+                         light_index_list, capacity_indices, stream);
+}
+
+// ---- the cluster grid in a 3-D CUDA array (the reference's R32G32_UINT cluster image imported from Vulkan) -------------
+int orbit_cluster_grid_wrap(orbit_ctx* c, void* cuda_array, orbit_cluster_grid** out) {
+    if (!out) return ORBIT_ERR_INVALID_ARGUMENT;
+    *out = nullptr;
+    if (!c || !cuda_array) return ORBIT_ERR_INVALID_ARGUMENT;
+    GUARD(c);
+    const cudaArray_t a = static_cast<cudaArray_t>(cuda_array);
+    cudaExtent ext{};
+    if (!array_info(a, cudaChannelFormatKindUnsigned, 32, &ext)) return ORBIT_ERR_INVALID_ARGUMENT;
+    if (ext.width == 0 || ext.height == 0 || ext.depth == 0 || ext.width > 0xFFFFFFFFull || ext.height > 0xFFFFFFFFull || ext.depth > 0xFFFFFFFFull)
+        return ORBIT_ERR_INVALID_ARGUMENT;
+    orbit_cluster_grid* g = new (std::nothrow) orbit_cluster_grid();
+    if (!g) return ORBIT_ERR_OUT_OF_MEMORY;
+    const cudaError_t e = make_surface(a, &g->surf);
+    if (e != cudaSuccess) { g_last_cuda_error = (int)e; delete g; return ORBIT_ERR_CUDA; }
+    g->width = (uint32_t)ext.width; g->height = (uint32_t)ext.height; g->depth = (uint32_t)ext.depth; g->device = c->device;
+    *out = g;
+    return ORBIT_OK;
+}
+
+void orbit_cluster_grid_destroy(orbit_cluster_grid* g) {
+    if (!g) return;
+    { DeviceGuard guard(g->device); cudaDestroySurfaceObject(g->surf); }
+    delete g;
+}
+
+int orbit_light_cluster_image_grid(orbit_ctx* c, const OrbitClusterParams* params, const orbit_depth_image* image, const void* lights,
+                                   void* tile_masks, void* depth_bounds, void* unique_clusters, const orbit_cluster_grid* grid,
+                                   void* light_index_list, uint64_t capacity_indices, void* stream) {
+    if (!image || !grid) return ORBIT_ERR_INVALID_ARGUMENT;
+    return light_cluster(c, params, nullptr, image, lights, tile_masks, depth_bounds, unique_clusters, nullptr, grid,
                          light_index_list, capacity_indices, stream);
 }
 

@@ -16,6 +16,11 @@
 //
 // Depth source: every kernel exists twice, for a linear buffer (HizBuildParams::depth) and for a depth image
 // (HizBuildParams::depth_tex, orbit_*_image). Only the level-0 loads differ; the footprint arithmetic is the same.
+//
+// Mirror (orbit_hiz_attach_image): each of those kernels has a kMirror twin that takes a second parameter block (HizMirror:
+// one surface per level of the caller's mipmapped array) and, next to every store of a texel to p.texels, writes the same
+// value to that level's surface. The linear pyramid is still written and stays what every culling kernel reads; the array
+// is never read back.
 #include "params.cuh"
 
 namespace orbit {
@@ -23,9 +28,18 @@ namespace orbit {
 
 __device__ __forceinline__ float ld_cg(const float* p) { return __ldcg(p); }
 
+// texel (x, y) of level l into the mirror, when the build has one (m: NULL for an unmirrored pyramid of a mixed batch).
+// Coordinates are in range by construction; zero boundary mode keeps a stray one from faulting.
+template <bool kMirror>
+__device__ __forceinline__ void mirror_store(const HizMirror* m, uint32_t l, uint32_t x, uint32_t y, float v) {
+    if constexpr (kMirror) {
+        if (m) surf2Dwrite(v, m->level[l], (int)(x * 4u), (int)y, cudaBoundaryModeZero);
+    }
+}
+
 // Generic level-by-level reduction of levels [first, levels) by ONE CTA (reads level first-1 from global / L2).
-template <bool kImage>
-__device__ void hiz_tail(const HizBuildParams& p, uint32_t first) {
+template <bool kImage, bool kMirror = false>
+__device__ void hiz_tail(const HizBuildParams& p, uint32_t first, const HizMirror* m = nullptr) {
     for (uint32_t l = first; l < p.levels; ++l) {
         const uint32_t w = max(p.width >> l, 1u), h = max(p.height >> l, 1u);
         float* dst = p.texels + p.level_offset[l];
@@ -38,11 +52,13 @@ __device__ void hiz_tail(const HizBuildParams& p, uint32_t first) {
                 if constexpr (kImage) {
                     const cudaTextureObject_t t = p.depth_tex;
                     dst[i] = fminf(fminf(depth_texel(t, x0, y0), depth_texel(t, x1, y0)), fminf(depth_texel(t, x0, y1), depth_texel(t, x1, y1)));
+                    mirror_store<kMirror>(m, 0u, x, y, dst[i]);
                     continue;
                 }
                 const float* r0 = p.depth + (size_t)y0 * p.depth_w;
                 const float* r1 = p.depth + (size_t)y1 * p.depth_w;
                 dst[i] = fminf(fminf(__ldg(r0 + x0), __ldg(r0 + x1)), fminf(__ldg(r1 + x0), __ldg(r1 + x1)));
+                mirror_store<kMirror>(m, 0u, x, y, dst[i]);
             }
         } else {
             const uint32_t sw = max(p.width >> (l - 1u), 1u), sh = max(p.height >> (l - 1u), 1u);
@@ -53,6 +69,7 @@ __device__ void hiz_tail(const HizBuildParams& p, uint32_t first) {
                 const uint32_t y0 = min(2u * y, sh - 1u), y1 = min(2u * y + 1u, sh - 1u);
                 dst[i] = fminf(fminf(ld_cg(src + (size_t)y0 * sw + x0), ld_cg(src + (size_t)y0 * sw + x1)),
                                fminf(ld_cg(src + (size_t)y1 * sw + x0), ld_cg(src + (size_t)y1 * sw + x1)));
+                mirror_store<kMirror>(m, l, x, y, dst[i]);
             }
         }
         __threadfence_block();
@@ -62,7 +79,8 @@ __device__ void hiz_tail(const HizBuildParams& p, uint32_t first) {
 
 // Top of the pyramid by the last CTA: level `first-1` (at most 4096 texels) is pulled into shared memory with one
 // round of L2 loads, then every remaining level is reduced out of shared memory (no global round trip per level).
-__device__ void hiz_tail_smem(const HizBuildParams& p, uint32_t first, float* s_a, float* s_b) {
+template <bool kMirror = false>
+__device__ void hiz_tail_smem(const HizBuildParams& p, uint32_t first, float* s_a, float* s_b, const HizMirror* m = nullptr) {
     uint32_t sw = max(p.width >> (first - 1u), 1u), sh = max(p.height >> (first - 1u), 1u);
     const float* src_g = p.texels + p.level_offset[first - 1u];
     for (uint32_t i = threadIdx.x; i < sw * sh; i += blockDim.x) s_a[i] = ld_cg(src_g + i);
@@ -79,6 +97,7 @@ __device__ void hiz_tail_smem(const HizBuildParams& p, uint32_t first, float* s_
             const float v = fminf(fminf(src[y0 * sw + x0], src[y0 * sw + x1]), fminf(src[y1 * sw + x0], src[y1 * sw + x1]));
             dst[i] = v;
             out[i] = v;
+            mirror_store<kMirror>(m, l, x, y, v);
         }
         __syncthreads();
         float* t = src; src = dst; dst = t;
@@ -94,10 +113,19 @@ __global__ void __launch_bounds__(256) hiz_small_image_kernel(const __grid_const
     pdl_wait();
     hiz_tail<true>(p, 0u);
 }
+__global__ void __launch_bounds__(256) hiz_small_mirror_kernel(const __grid_constant__ HizBuildParams p, const __grid_constant__ HizMirror m) {
+    pdl_wait();
+    hiz_tail<false, true>(p, 0u, &m);
+}
+__global__ void __launch_bounds__(256) hiz_small_image_mirror_kernel(const __grid_constant__ HizBuildParams p, const __grid_constant__ HizMirror m) {
+    pdl_wait();
+    hiz_tail<true, true>(p, 0u, &m);
+}
 
 // One pyramid, one CTA per 64x64 tile of level 0 (blockIdx.x); the batched kernel runs one row of the grid per pyramid.
-template <bool kImage>
-__device__ __forceinline__ void hiz_build_body(const HizBuildParams& p) {
+// m: the mirror of the kMirror variants (NULL: this pyramid of a batch has none)
+template <bool kImage, bool kMirror = false>
+__device__ __forceinline__ void hiz_build_body(const HizBuildParams& p, const HizMirror* m = nullptr) {
     __shared__ float s_l3[8][8];
     __shared__ bool s_last;
     __shared__ float s_top_a[4096], s_top_b[1024];
@@ -172,8 +200,11 @@ __device__ __forceinline__ void hiz_build_body(const HizBuildParams& p) {
     {
         float* l0 = p.texels + p.level_offset[0];
 #pragma unroll
-        for (int r = 0; r < 8; ++r)
+        for (int r = 0; r < 8; ++r) {
             *reinterpret_cast<float2*>(l0 + (size_t)(y_base + r) * p.width + x_a) = make_float2(va[r], vb[r]);
+            mirror_store<kMirror>(m, 0u, x_a, y_base + r, va[r]);
+            mirror_store<kMirror>(m, 0u, x_a + 1u, y_base + r, vb[r]);
+        }
     }
     // ---- level 1: 4 rows x 32 columns per warp, one texel per lane per row
     float l1[4];
@@ -184,6 +215,7 @@ __device__ __forceinline__ void hiz_build_body(const HizBuildParams& p) {
         for (int r = 0; r < 4; ++r) {
             l1[r] = fminf(fminf(va[2 * r], vb[2 * r]), fminf(va[2 * r + 1], vb[2 * r + 1]));
             d[(size_t)((y_base >> 1) + r) * w1 + (tx * 32u + lane)] = l1[r];
+            mirror_store<kMirror>(m, 1u, tx * 32u + lane, (y_base >> 1) + r, l1[r]);
         }
     }
     // ---- level 2: 2 rows x 16 columns per warp (even lanes hold the result)
@@ -195,7 +227,10 @@ __device__ __forceinline__ void hiz_build_body(const HizBuildParams& p) {
         for (int r = 0; r < 2; ++r) {
             float v = fminf(l1[2 * r], l1[2 * r + 1]);
             l2[r] = fminf(v, __shfl_xor_sync(0xFFFFFFFFu, v, 1));
-            if ((lane & 1u) == 0u) d[(size_t)((y_base >> 2) + r) * w2 + (tx * 16u + (lane >> 1))] = l2[r];
+            if ((lane & 1u) == 0u) {
+                d[(size_t)((y_base >> 2) + r) * w2 + (tx * 16u + (lane >> 1))] = l2[r];
+                mirror_store<kMirror>(m, 2u, tx * 16u + (lane >> 1), (y_base >> 2) + r, l2[r]);
+            }
         }
     }
     // ---- level 3: 1 row x 8 columns per warp (lanes 0,4,8,.. hold the result)
@@ -207,6 +242,7 @@ __device__ __forceinline__ void hiz_build_body(const HizBuildParams& p) {
         if ((lane & 3u) == 0u) {
             p.texels[p.level_offset[3] + (size_t)(y_base >> 3) * w3 + (tx * 8u + (lane >> 2))] = l3;
             s_l3[warp][lane >> 2] = l3;
+            mirror_store<kMirror>(m, 3u, tx * 8u + (lane >> 2), y_base >> 3, l3);
         }
     }
     __syncthreads();
@@ -214,15 +250,23 @@ __device__ __forceinline__ void hiz_build_body(const HizBuildParams& p) {
     if (warp == 0u) {
         const uint32_t x4 = lane & 3u, y4 = (lane >> 2) & 3u;  // lanes 0..15 meaningful
         float v4 = fminf(fminf(s_l3[2 * y4][2 * x4], s_l3[2 * y4][2 * x4 + 1]), fminf(s_l3[2 * y4 + 1][2 * x4], s_l3[2 * y4 + 1][2 * x4 + 1]));
-        if (lane < 16u) p.texels[p.level_offset[4] + (size_t)(ty * 4u + y4) * (p.width >> 4) + (tx * 4u + x4)] = v4;
+        if (lane < 16u) {
+            p.texels[p.level_offset[4] + (size_t)(ty * 4u + y4) * (p.width >> 4) + (tx * 4u + x4)] = v4;
+            mirror_store<kMirror>(m, 4u, tx * 4u + x4, ty * 4u + y4, v4);
+        }
         // level 5: combine x pairs (xor 1) and y pairs (xor 4)
         float v5 = fminf(v4, __shfl_xor_sync(0xFFFFFFFFu, v4, 1));
         v5 = fminf(v5, __shfl_xor_sync(0xFFFFFFFFu, v5, 4));
-        if (lane < 16u && (lane & 5u) == 0u)
+        if (lane < 16u && (lane & 5u) == 0u) {
             p.texels[p.level_offset[5] + (size_t)(ty * 2u + (y4 >> 1)) * (p.width >> 5) + (tx * 2u + (x4 >> 1))] = v5;
+            mirror_store<kMirror>(m, 5u, tx * 2u + (x4 >> 1), ty * 2u + (y4 >> 1), v5);
+        }
         float v6 = fminf(v5, __shfl_xor_sync(0xFFFFFFFFu, v5, 2));
         v6 = fminf(v6, __shfl_xor_sync(0xFFFFFFFFu, v6, 8));
-        if (lane == 0u) p.texels[p.level_offset[6] + (size_t)ty * (p.width >> 6) + tx] = v6;
+        if (lane == 0u) {
+            p.texels[p.level_offset[6] + (size_t)ty * (p.width >> 6) + tx] = v6;
+            mirror_store<kMirror>(m, 6u, tx, ty, v6);
+        }
     }
     ORBIT_TRACE_STAMP(p.trace, 4, 2);
     pdl_launch_dependents();
@@ -239,13 +283,19 @@ __device__ __forceinline__ void hiz_build_body(const HizBuildParams& p) {
     ORBIT_TRACE_STAMP(p.trace, 4, 3);
     if (!s_last) return;
     __threadfence();
-    if ((p.width >> 6) * (p.height >> 6) <= 4096u) hiz_tail_smem(p, 7u, s_top_a, s_top_b);
-    else hiz_tail<kImage>(p, 7u);
+    if ((p.width >> 6) * (p.height >> 6) <= 4096u) hiz_tail_smem<kMirror>(p, 7u, s_top_a, s_top_b, m);
+    else hiz_tail<kImage, kMirror>(p, 7u, m);
     ORBIT_TRACE_STAMP(p.trace, 4, 4);
 }
 
 __global__ void __launch_bounds__(256) hiz_build_kernel(const __grid_constant__ HizBuildParams p) { hiz_build_body<false>(p); }
 __global__ void __launch_bounds__(256) hiz_build_image_kernel(const __grid_constant__ HizBuildParams p) { hiz_build_body<true>(p); }
+__global__ void __launch_bounds__(256) hiz_build_mirror_kernel(const __grid_constant__ HizBuildParams p, const __grid_constant__ HizMirror m) {
+    hiz_build_body<false, true>(p, &m);
+}
+__global__ void __launch_bounds__(256) hiz_build_image_mirror_kernel(const __grid_constant__ HizBuildParams p, const __grid_constant__ HizMirror m) {
+    hiz_build_body<true, true>(p, &m);
+}
 
 // orbit_hiz_build_views: pyramid blockIdx.y; each has its own ticket, so each row's last CTA reduces that pyramid's top levels
 __global__ void __launch_bounds__(256) hiz_build_views_kernel(const __grid_constant__ HizBuildViewsParams pv) { hiz_build_body<false>(pv.view[blockIdx.y]); }
@@ -258,24 +308,52 @@ __global__ void __launch_bounds__(256) hiz_small_views_image_kernel(const __grid
     pdl_wait();
     hiz_tail<true>(pv.view[blockIdx.y], 0u);
 }
-
-// image: level 0 is read from p.depth_tex (a depth image) instead of p.depth
-cudaError_t launch_hiz_build(const HizBuildParams& p, cudaStream_t stream, bool image) {
-    if (p.width >= 64u && p.height >= 64u && p.levels >= 7u) {
-        const uint32_t grid = (p.width >> 6) * (p.height >> 6);
-        return launch_kernel(image ? hiz_build_image_kernel : hiz_build_kernel, dim3(grid), dim3(256), 0, stream, p);
-    } else {
-        return launch_kernel(image ? hiz_small_image_kernel : hiz_small_kernel, dim3(1), dim3(256), 0, stream, p);
-    }
-    return cudaGetLastError();
+// mixed batches: a row whose pyramid has no mirror passes NULL
+__device__ __forceinline__ const HizMirror* view_mirror(const HizMirrorViews& mv) {
+    return ((mv.mirrored >> blockIdx.y) & 1u) ? &mv.view[blockIdx.y] : nullptr;
+}
+__global__ void __launch_bounds__(256) hiz_build_views_mirror_kernel(const __grid_constant__ HizBuildViewsParams pv,
+                                                                     const __grid_constant__ HizMirrorViews mv) {
+    hiz_build_body<false, true>(pv.view[blockIdx.y], view_mirror(mv));
+}
+__global__ void __launch_bounds__(256) hiz_small_views_mirror_kernel(const __grid_constant__ HizBuildViewsParams pv,
+                                                                     const __grid_constant__ HizMirrorViews mv) {
+    pdl_wait();
+    hiz_tail<false, true>(pv.view[blockIdx.y], 0u, view_mirror(mv));
+}
+__global__ void __launch_bounds__(256) hiz_build_views_image_mirror_kernel(const __grid_constant__ HizBuildViewsParams pv,
+                                                                           const __grid_constant__ HizMirrorViews mv) {
+    hiz_build_body<true, true>(pv.view[blockIdx.y], view_mirror(mv));
+}
+__global__ void __launch_bounds__(256) hiz_small_views_image_mirror_kernel(const __grid_constant__ HizBuildViewsParams pv,
+                                                                           const __grid_constant__ HizMirrorViews mv) {
+    pdl_wait();
+    hiz_tail<true, true>(pv.view[blockIdx.y], 0u, view_mirror(mv));
 }
 
-cudaError_t launch_hiz_build_views(const HizBuildViewsParams& pv, cudaStream_t stream, bool image) {
+// image: level 0 is read from p.depth_tex (a depth image) instead of p.depth; mirror (nullable): the pyramid's mirror surfaces
+cudaError_t launch_hiz_build(const HizBuildParams& p, cudaStream_t stream, bool image, const HizMirror* mirror) {
+    const bool tiled = p.width >= 64u && p.height >= 64u && p.levels >= 7u;
+    const dim3 grid(tiled ? (p.width >> 6) * (p.height >> 6) : 1u);
+    if (mirror) {
+        if (tiled) return launch_kernel(image ? hiz_build_image_mirror_kernel : hiz_build_mirror_kernel, grid, dim3(256), 0, stream, p, *mirror);
+        return launch_kernel(image ? hiz_small_image_mirror_kernel : hiz_small_mirror_kernel, grid, dim3(256), 0, stream, p, *mirror);
+    }
+    if (tiled) return launch_kernel(image ? hiz_build_image_kernel : hiz_build_kernel, grid, dim3(256), 0, stream, p);
+    return launch_kernel(image ? hiz_small_image_kernel : hiz_small_kernel, grid, dim3(256), 0, stream, p);
+}
+
+// mirror (nullable): the batch's mirror surfaces, when at least one of its pyramids has a mirror
+cudaError_t launch_hiz_build_views(const HizBuildViewsParams& pv, cudaStream_t stream, bool image, const HizMirrorViews* mirror) {
     const HizBuildParams& p = pv.view[0];   // every pyramid of the call has this geometry
-    if (p.width >= 64u && p.height >= 64u && p.levels >= 7u)
-        return launch_kernel(image ? hiz_build_views_image_kernel : hiz_build_views_kernel, dim3((p.width >> 6) * (p.height >> 6), pv.n_views),
-                             dim3(256), 0, stream, pv);
-    return launch_kernel(image ? hiz_small_views_image_kernel : hiz_small_views_kernel, dim3(1, pv.n_views), dim3(256), 0, stream, pv);
+    const bool tiled = p.width >= 64u && p.height >= 64u && p.levels >= 7u;
+    const dim3 grid(tiled ? (p.width >> 6) * (p.height >> 6) : 1u, pv.n_views);
+    if (mirror) {
+        if (tiled) return launch_kernel(image ? hiz_build_views_image_mirror_kernel : hiz_build_views_mirror_kernel, grid, dim3(256), 0, stream, pv, *mirror);
+        return launch_kernel(image ? hiz_small_views_image_mirror_kernel : hiz_small_views_mirror_kernel, grid, dim3(256), 0, stream, pv, *mirror);
+    }
+    if (tiled) return launch_kernel(image ? hiz_build_views_image_kernel : hiz_build_views_kernel, grid, dim3(256), 0, stream, pv);
+    return launch_kernel(image ? hiz_small_views_image_kernel : hiz_small_views_kernel, grid, dim3(256), 0, stream, pv);
 }
 
 }  // namespace orbit

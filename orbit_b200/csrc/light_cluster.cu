@@ -176,8 +176,19 @@ __device__ __forceinline__ Aabb3 cluster_volume(const ClusterParams& p, uint32_t
     return a;
 }
 
+// The offset / count grid as a 3-D R32G32_UINT array (orbit_light_cluster_image_grid): each storing kernel has a kGrid twin
+// that writes texel (x, y, z) of p.offset_count_surf where the linear form writes words 2 idx, 2 idx + 1. An array cannot be
+// cleared with cudaMemsetAsync, so the compaction kernel's twin writes (0, 0) to every inactive cluster and the list kernels
+// write every active one: each call writes every texel once.
+__device__ __forceinline__ void grid_store(const ClusterParams& p, uint32_t idx, uint32_t off, uint32_t count) {
+    const uint32_t cx = p.info.cluster_count[0], cy = p.info.cluster_count[1];
+    const uint32_t z = idx / (cx * cy), t = idx - z * cx * cy, y = t / cx, x = t - y * cx;
+    surf3Dwrite(make_uint2(off, count), p.offset_count_surf, (int)(x * 8u), (int)y, (int)z, cudaBoundaryModeZero);
+}
+
 // ---------------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) compact_clusters_kernel(const __grid_constant__ ClusterParams p) {
+template <bool kGrid>
+__device__ __forceinline__ void compact_clusters_body(const ClusterParams& p) {
     __shared__ uint32_t s_warp[8];
     __shared__ uint32_t s_tile, s_base;
     const OrbitClusterCullInfo& ci = p.info;
@@ -227,8 +238,14 @@ __global__ void __launch_bounds__(256) compact_clusters_kernel(const __grid_cons
             p.cluster_boxes[2u * (size_t)slot + 1u] = make_float4(b.hi[0], b.hi[1], b.hi[2], 0.0f);
         }
     }
+    if constexpr (kGrid) {
+        if (idx < total && !active) grid_store(p, idx, 0u, 0u);
+    }
     if (tid == 0) scan_cta_exit(p.scan, epoch);
 }
+
+__global__ void __launch_bounds__(256) compact_clusters_kernel(const __grid_constant__ ClusterParams p) { compact_clusters_body<false>(p); }
+__global__ void __launch_bounds__(256) compact_clusters_grid_kernel(const __grid_constant__ ClusterParams p) { compact_clusters_body<true>(p); }
 
 // ---------------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) light_view_kernel(const __grid_constant__ ClusterParams p) {
@@ -255,91 +272,18 @@ constexpr int kLcWarps = 32;
 // concatenated in warp order up to the reference's cap of 256, and the cluster's range in the global list comes
 // from a look-back scan over clusters in compacted-list order. With few active clusters (typical: ~100 of 3456)
 // this spreads each cluster's L tests over 1024 threads instead of one warp (measured 716 us -> see profiles/).
-__global__ void __launch_bounds__(kLcWarps * 32) light_culling_kernel(const __grid_constant__ ClusterParams p) {
-    extern __shared__ uint32_t s_dyn[];                       // kLcWarps x 256 hit lists
-    __shared__ uint32_t s_warp[kLcWarps];
-    __shared__ uint32_t s_tile, s_off;
-    const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
-    uint32_t* const my_list = s_dyn + warp * ORBIT_MAX_LIGHTS_PER_CLUSTER;
-    const unsigned int epoch = scan_epoch(p.scan);
-    const uint32_t nactive = __ldcg(p.unique_clusters + 3);
-    const uint32_t L = p.info.global_light_count;
-    const uint32_t per = (L + kLcWarps - 1) / kLcWarps;
-    const uint32_t j_begin = min(warp * per, L), j_end = min(j_begin + per, L);
-    while (true) {
-        __syncthreads();
-        if (tid == 0) s_tile = atomicAdd(p.scan.ticket, 1u);
-        __syncthreads();
-        const uint32_t tile = s_tile;
-        if (tile >= nactive) {
-            if (tile == 0u && tid == 0) p.light_index_words[0] = 0u;
-            break;
-        }
-        const uint32_t idx = __ldcg(p.unique_clusters + 4u + tile);
-        const Aabb3 box = cluster_volume(p, idx);
-        uint32_t count = 0u;   // hits of this warp's stripe (uncapped)
-        for (uint32_t j0 = j_begin; j0 < j_end; j0 += 128u) {
-            float4 sv[4];
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {   // four independent 512-byte loads in flight per warp
-                const uint32_t j = j0 + (uint32_t)u * 32u + lane;
-                sv[u] = j < j_end ? __ldg(p.light_view + j) : make_float4(0.f, 0.f, 0.f, -1.f);
-            }
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-                const uint32_t j = j0 + (uint32_t)u * 32u + lane;
-                bool hit = false;
-                if (j < j_end) {
-                    const float4 s = sv[u];
-                    float acc = 0.0f;
-                    const float c[3] = {s.x, s.y, s.z};
-#pragma unroll
-                    for (int k = 0; k < 3; ++k) {
-                        // lo <= hi, so at most one of the reference's two branches adds a term; d is that term's
-                        // base (or 0, and fma(0,0,acc) == acc): same value, no divergence
-                        const float v = c[k];
-                        const float d = fmaxf(fmaxf(sub(box.lo[k], v), sub(v, box.hi[k])), 0.0f);
-                        acc = fma_(d, d, acc);
-                    }
-                    hit = acc <= mul(s.w, s.w);
-                }
-                const uint32_t bal = __ballot_sync(0xFFFFFFFFu, hit);
-                if (hit) {
-                    const uint32_t r = count + __popc(bal & ((1u << lane) - 1u));
-                    if (r < ORBIT_MAX_LIGHTS_PER_CLUSTER) my_list[r] = j;
-                }
-                count += __popc(bal);
-            }
-        }
-        if (lane == 0u) s_warp[warp] = min(count, ORBIT_MAX_LIGHTS_PER_CLUSTER);
-        __syncthreads();
-        // exclusive prefix of the (capped) stripe counts in warp order; everything past 256 is dropped
-        uint32_t before = 0u, total = 0u;
-#pragma unroll
-        for (int w = 0; w < kLcWarps; ++w) { const uint32_t v = s_warp[w]; if ((uint32_t)w < warp) before += v; total += v; }
-        total = min(total, ORBIT_MAX_LIGHTS_PER_CLUSTER);
-        if (warp == 0u) {
-            const uint32_t off = lookback_exclusive(p.scan, epoch, tile, total);
-            if (lane == 0u) {
-                s_off = off;
-                p.offset_count_image[2u * (size_t)idx] = off;
-                p.offset_count_image[2u * (size_t)idx + 1u] = total;
-                if (tile == nactive - 1u) {
-                    p.light_index_words[0] = off + total;
-                    if ((uint64_t)off + total > p.capacity_indices) *p.overflow_flag = 1u;
-                }
-            }
-        }
-        __syncthreads();
-        const uint32_t off = s_off;
-        const uint32_t mine = min(count, ORBIT_MAX_LIGHTS_PER_CLUSTER);
-        for (uint32_t k = lane; k < mine; k += 32u) {
-            const uint32_t r = before + k;
-            if (r < ORBIT_MAX_LIGHTS_PER_CLUSTER && (uint64_t)off + r < p.capacity_indices) p.light_index_words[1u + off + r] = my_list[k];
-        }
-    }
-    if (tid == 0) scan_cta_exit(p.scan, epoch);
-}
+// The kernel is in light_culling_kernel.cuh, compiled twice: light_culling_kernel (linear offset / count buffer) and
+// light_culling_grid_kernel (grid array, see grid_store).
+#define ORBIT_LC_KERNEL light_culling_kernel
+#define ORBIT_LC_GRID 0
+#include "light_culling_kernel.cuh"
+#undef ORBIT_LC_KERNEL
+#undef ORBIT_LC_GRID
+#define ORBIT_LC_KERNEL light_culling_grid_kernel
+#define ORBIT_LC_GRID 1
+#include "light_culling_kernel.cuh"
+#undef ORBIT_LC_KERNEL
+#undef ORBIT_LC_GRID
 
 // ---------------------------------------------------------------------------------------------------------
 // Light-parallel formulation of light_culling.comp:121-151 (the path taken whenever its bit matrix fits the scratch budget;
@@ -489,8 +433,9 @@ __global__ void __launch_bounds__(256) light_hits_kernel(const __grid_constant__
 // round of 64-byte row reads for up to 32 hit blocks, wherever in the light range they lie (block by block in 32-block steps
 // took one dependent round trip per step).
 constexpr int kLlWarps = 32;
-__global__ void __launch_bounds__(kLlWarps * 32) light_lists_kernel(const __grid_constant__ ClusterParams p, const uint32_t* __restrict__ hits,
-                                                                    const uint32_t* __restrict__ counts, uint32_t words_per_cluster, uint32_t light_blocks) {
+template <bool kGrid>
+__device__ __forceinline__ void light_lists_body(const ClusterParams& p, const uint32_t* __restrict__ hits, const uint32_t* __restrict__ counts,
+                                                 uint32_t words_per_cluster, uint32_t light_blocks) {
     __shared__ uint32_t s_cnt[kLlWarps], s_part[kLlWarps];
     __shared__ uint32_t s_base;
     __shared__ uint32_t s_blocks[kLlWarps][ORBIT_MAX_LIGHTS_PER_CLUSTER];   // block << 9 | rank of its first hit (< 256), per hit block of the warp's cluster
@@ -527,7 +472,10 @@ __global__ void __launch_bounds__(kLlWarps * 32) light_lists_kernel(const __grid
         }
         if (!have) continue;
         const uint32_t off = base + before;
-        if (lane == 0u) { p.offset_count_image[2u * (size_t)idx] = off; p.offset_count_image[2u * (size_t)idx + 1u] = count; }
+        if (lane == 0u) {
+            if constexpr (kGrid) grid_store(p, idx, off, count);
+            else { p.offset_count_image[2u * (size_t)idx] = off; p.offset_count_image[2u * (size_t)idx + 1u] = count; }
+        }
         if (count == 0u) continue;
         // ---- hit blocks of the cluster in ascending order, with the rank of their first hit. The block counts were requested
         // with the round's other loads (kept[]: 8 x 32 blocks = 131 072 lights in registers, indexed by compile-time constants
@@ -577,6 +525,15 @@ __global__ void __launch_bounds__(kLlWarps * 32) light_lists_kernel(const __grid
     }
 }
 
+__global__ void __launch_bounds__(kLlWarps * 32) light_lists_kernel(const __grid_constant__ ClusterParams p, const uint32_t* __restrict__ hits,
+                                                                    const uint32_t* __restrict__ counts, uint32_t words_per_cluster, uint32_t light_blocks) {
+    light_lists_body<false>(p, hits, counts, words_per_cluster, light_blocks);
+}
+__global__ void __launch_bounds__(kLlWarps * 32) light_lists_grid_kernel(const __grid_constant__ ClusterParams p, const uint32_t* __restrict__ hits,
+                                                                         const uint32_t* __restrict__ counts, uint32_t words_per_cluster, uint32_t light_blocks) {
+    light_lists_body<true>(p, hits, counts, words_per_cluster, light_blocks);
+}
+
 uint32_t light_hits_blocks(uint32_t n_lights) { return (n_lights + kLhLightsPerCta - 1u) / kLhLightsPerCta; }
 
 cudaError_t launch_light_hits(const ClusterParams& p, uint32_t* hits, uint32_t* counts, uint32_t words_per_cluster, uint32_t max_clusters, cudaStream_t s) {
@@ -587,8 +544,11 @@ cudaError_t launch_light_hits(const ClusterParams& p, uint32_t* hits, uint32_t* 
     light_hits_kernel<<<dim3(gx, gy ? gy : 1u), 256, 0, s>>>(p, hits, counts, words_per_cluster);
     return cudaGetLastError();
 }
-cudaError_t launch_light_lists(const ClusterParams& p, const uint32_t* hits, const uint32_t* counts, uint32_t words_per_cluster, int grid, cudaStream_t s) {
-    light_lists_kernel<<<grid, kLlWarps * 32, 0, s>>>(p, hits, counts, words_per_cluster, light_hits_blocks(p.info.global_light_count));
+// to_grid: the offset / count grid goes to p.offset_count_surf (the same for the compaction and CTA-per-cluster launchers)
+cudaError_t launch_light_lists(const ClusterParams& p, const uint32_t* hits, const uint32_t* counts, uint32_t words_per_cluster, int grid, cudaStream_t s,
+                               bool to_grid) {
+    (to_grid ? light_lists_grid_kernel : light_lists_kernel)<<<grid, kLlWarps * 32, 0, s>>>(p, hits, counts, words_per_cluster,
+                                                                                           light_hits_blocks(p.info.global_light_count));
     return cudaGetLastError();
 }
 
@@ -597,9 +557,9 @@ cudaError_t launch_mark_active(const ClusterParams& p, int grid, cudaStream_t s,
     else mark_active_kernel<<<grid, 256, 0, s>>>(p);
     return cudaGetLastError();
 }
-cudaError_t launch_compact_clusters(const ClusterParams& p, cudaStream_t s) {
+cudaError_t launch_compact_clusters(const ClusterParams& p, cudaStream_t s, bool grid) {
     const uint32_t total = p.info.cluster_count[0] * p.info.cluster_count[1] * p.info.cluster_count[2];
-    compact_clusters_kernel<<<(total + 255u) / 256u, 256, 0, s>>>(p);
+    (grid ? compact_clusters_grid_kernel : compact_clusters_kernel)<<<(total + 255u) / 256u, 256, 0, s>>>(p);
     return cudaGetLastError();
 }
 cudaError_t launch_light_view(const ClusterParams& p, cudaStream_t s) {
@@ -612,11 +572,13 @@ static constexpr size_t light_culling_smem_bytes() { return (size_t)kLcWarps * O
 
 // More than 48 KB of dynamic shared memory: opt in once per DEVICE (called from orbit_ctx_create with the context's device current).
 cudaError_t light_cluster_configure_device() {
-    return cudaFuncSetAttribute(light_culling_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)light_culling_smem_bytes());
+    const cudaError_t e = cudaFuncSetAttribute(light_culling_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)light_culling_smem_bytes());
+    if (e != cudaSuccess) return e;
+    return cudaFuncSetAttribute(light_culling_grid_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)light_culling_smem_bytes());
 }
 
-cudaError_t launch_light_culling(const ClusterParams& p, int grid, cudaStream_t s) {
-    light_culling_kernel<<<grid, kLcWarps * 32, light_culling_smem_bytes(), s>>>(p);
+cudaError_t launch_light_culling(const ClusterParams& p, int grid, cudaStream_t s, bool to_grid) {
+    (to_grid ? light_culling_grid_kernel : light_culling_kernel)<<<grid, kLcWarps * 32, light_culling_smem_bytes(), s>>>(p);
     return cudaGetLastError();
 }
 

@@ -19,6 +19,19 @@ inline cudaError_t launch_kernel(void (*kernel)(const P), dim3 grid, dim3 block,
     cfg.numAttrs = pdl_enabled() ? 1 : 0;
     return cudaLaunchKernelEx(&cfg, kernel, params);
 }
+// the same for a kernel with a second parameter block
+template <typename P, typename Q>
+inline cudaError_t launch_kernel(void (*kernel)(const P, const Q), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, const P& params,
+                                 const Q& extra) {
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = stream;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = pdl_enabled() ? 1 : 0;
+    return cudaLaunchKernelEx(&cfg, kernel, params, extra);
+}
 
 struct MeshletCullParams {
     OrbitCullInfo cull;
@@ -134,6 +147,18 @@ struct HizBuildViewsParams {
     HizBuildParams view[ORBIT_MAX_BATCH_VIEWS];
     uint32_t n_views;
 };
+// Mirror of a pyramid in a caller's mipmapped CUDA array (orbit_hiz_attach_image): one surface per level, written by the
+// mirror variants of the build next to every store of the linear level. A second kernel parameter, so that HizBuildParams
+// and HizBuildViewsParams (and the kernels that take them alone) stay as they are.
+struct HizMirror {
+    cudaSurfaceObject_t level[ORBIT_HIZ_MAX_LEVELS];
+};
+// orbit_hiz_build_views: pyramid v is mirrored into view[v] when bit v of `mirrored` is set (mixed batches)
+struct HizMirrorViews {
+    HizMirror view[ORBIT_MAX_BATCH_VIEWS];
+    uint32_t mirrored;
+};
+static_assert(sizeof(HizBuildViewsParams) + sizeof(HizMirrorViews) <= 32764, "kernel parameter space is 32 764 bytes");
 
 struct ClusterParams {
     OrbitClusterCullInfo info;
@@ -149,7 +174,10 @@ struct ClusterParams {
     uint32_t* tile_masks;
     uint32_t* depth_bounds;           // 2 words per cluster
     uint32_t* unique_clusters;        // 4-word header + indices
-    uint32_t* offset_count_image;     // 2 words per cluster
+    union {                           // the storing kernels' template parameter picks the member (same 8 bytes, same offset)
+        uint32_t* offset_count_image;         // 2 words per cluster, linear
+        cudaSurfaceObject_t offset_count_surf;// a 3-D R32G32_UINT array [cz][cy][cx] (orbit_cluster_grid): texel (x, y, z)
+    };
     uint32_t* light_index_words;      // count + indices
     uint32_t* overflow_flag;
     uint64_t capacity_indices;
@@ -174,18 +202,19 @@ cudaError_t launch_meshlet_cull_views(const MeshletViewsParams&, int grid, int e
 int meshlet_cull_views_max_ctas_per_sm(const OrbitCullInfo&);
 int entity_cull_max_ctas_per_sm(bool defer_wait);
 int entity_cull_views_max_ctas_per_sm(uint32_t occlusion_pass);
-cudaError_t launch_hiz_build(const HizBuildParams&, cudaStream_t, bool image = false);
-cudaError_t launch_hiz_build_views(const HizBuildViewsParams&, cudaStream_t, bool image = false);
+cudaError_t launch_hiz_build(const HizBuildParams&, cudaStream_t, bool image = false, const HizMirror* mirror = nullptr);
+cudaError_t launch_hiz_build_views(const HizBuildViewsParams&, cudaStream_t, bool image = false, const HizMirrorViews* mirror = nullptr);
 cudaError_t launch_meshlet_bounds(const MeshletBoundsParams&, int grid, cudaStream_t);
 cudaError_t launch_mesh_bounds(const MeshBoundsParams&, int grid, cudaStream_t);
 cudaError_t launch_scene_update(const SceneUpdateParams&, cudaStream_t);
 cudaError_t launch_mark_active(const ClusterParams&, int grid, cudaStream_t, bool image = false);
-cudaError_t launch_compact_clusters(const ClusterParams&, cudaStream_t);
+cudaError_t launch_compact_clusters(const ClusterParams&, cudaStream_t, bool grid = false);
 cudaError_t launch_light_view(const ClusterParams&, cudaStream_t);
-cudaError_t launch_light_culling(const ClusterParams&, int grid, cudaStream_t);
+cudaError_t launch_light_culling(const ClusterParams&, int grid, cudaStream_t, bool to_grid = false);
 uint32_t light_hits_blocks(uint32_t n_lights);
 cudaError_t launch_light_hits(const ClusterParams&, uint32_t* hits, uint32_t* counts, uint32_t words_per_cluster, uint32_t max_clusters, cudaStream_t);
-cudaError_t launch_light_lists(const ClusterParams&, const uint32_t* hits, const uint32_t* counts, uint32_t words_per_cluster, int grid, cudaStream_t);
+cudaError_t launch_light_lists(const ClusterParams&, const uint32_t* hits, const uint32_t* counts, uint32_t words_per_cluster, int grid, cudaStream_t,
+                               bool to_grid = false);
 cudaError_t launch_draws_scatter(const uint32_t* src, uint64_t src_capacity, uint32_t* dst, uint32_t dst_first, uint32_t total_count,
                                  uint64_t dst_capacity, int grid, cudaStream_t s, const uint32_t* rank_counts, uint32_t rank, uint32_t world);
 

@@ -43,10 +43,11 @@ class ViewState:
     """Cross-frame state of one view: the two visibility bitmasks (forward.rs:104-106,150-157; scene.rs:364) and
     the depth pyramid. The reference never clears the bitmasks; the harness defines frame 0 as all zeros."""
 
-    def __init__(self, context, dscene, size, name="view"):
+    def __init__(self, context, dscene, size, name="view", pyramid_image=None):
+        """pyramid_image: a cudaMipmappedArray_t (integer) the pyramid is mirrored into on every build (DepthPyramid)."""
         self.entity_visibility = torch.zeros((dscene.n_entities + 31) // 32 + 1, dtype=torch.int32, device=context.device)
         self.meshlet_visibility = torch.zeros(max(dscene.n_visibility_words, 1), dtype=torch.int32, device=context.device)
-        self.depth_pyramid = DepthPyramid(context, name + "_depth_pyramid", size)
+        self.depth_pyramid = DepthPyramid(context, name + "_depth_pyramid", size, image=pyramid_image)
 
 
 def projection_of(view):

@@ -241,18 +241,49 @@ class DepthImage:
             pass
 
 
-class DepthPyramid:
-    """draw_gen.rs:451-567. One linear f32 allocation holding all mips back to back."""
+class ClusterGridImage:
+    """The cluster offset/count grid held in a 3-D CUDA array with two 32-bit unsigned channels and surface load/store
+    (orbit_cluster_grid_wrap): the form the reference's R32G32_UINT cluster image takes when imported from Vulkan.
+    `cuda_array` is the cudaArray_t as an integer; the array stays the caller's and must outlive this object and every
+    enqueued or captured call that writes it. compute_clusters(..., light_offset_image=grid) writes the grid into it."""
 
-    def __init__(self, context, name, size):
+    def __init__(self, context, cuda_array):
+        self.context = context
+        self._h = C.c_void_p()
+        _lib.check(_lib.lib().orbit_cluster_grid_wrap(context._h, C.c_void_p(int(cuda_array)), C.byref(self._h)), "orbit_cluster_grid_wrap")
+        self.cuda_array = int(cuda_array)
+
+    def close(self):
+        if self._h:
+            _lib.lib().orbit_cluster_grid_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class DepthPyramid:
+    """draw_gen.rs:451-567. One linear f32 allocation holding all mips back to back. With `image` (a cudaMipmappedArray_t
+    as an integer, e.g. mapped from the renderer's imported pyramid VkImage) every build also stores level l into level l of
+    that array (orbit_hiz_attach_image); the linear texels stay what the culling stages read."""
+
+    def __init__(self, context, name, size, image=None):
         self.context, self.name = context, name
         self._h = C.c_void_p()
         self.usable = False
         self.texels = None
         self.size = None
+        self.image = int(image) if image is not None else None
         self._make(size)
 
-    new = classmethod(lambda cls, context, name, size: cls(context, name, size))
+    new = classmethod(lambda cls, context, name, size, image=None: cls(context, name, size, image))
+
+    def _attach(self):
+        if self.image is not None:
+            _lib.check(_lib.lib().orbit_hiz_attach_image(self.context._h, self._h, C.c_void_p(self.image)), "orbit_hiz_attach_image")
 
     def _make(self, size):
         w, h = int(size[0]), int(size[1])
@@ -266,10 +297,27 @@ class DepthPyramid:
         _lib.check(_lib.lib().orbit_hiz_wrap(self.context._h, w, h, _ptr(self.texels), C.byref(self._h)), "orbit_hiz_wrap")
         self.size = (w, h)
         self.usable = False
+        self._attach()
 
-    def resize(self, size):
+    def resize(self, size, image=None):
+        """A mirrored pyramid needs `image`: the array for the new size (the old one no longer fits)."""
         if (int(size[0]), int(size[1])) != self.size:
+            if self.image is not None and image is None:
+                raise ValueError("DepthPyramid.resize: the pyramid has an image; pass the array for the new size")
+            if image is not None:
+                self.image = int(image)
             self._make(size)
+
+    def attach_image(self, image):
+        """Mirrors every later build into `image` (a cudaMipmappedArray_t as an integer; see the class comment)."""
+        if self.image is not None:
+            raise ValueError("DepthPyramid.attach_image: the pyramid already has an image")
+        self.image = int(image)
+        try:
+            self._attach()
+        except Exception:
+            self.image = None
+            raise
 
     def rebind_external(self, device_ptr):
         """Moves the pyramid onto caller-owned device memory of info.total_texels floats (orbit_hiz_wrap): peer-shareable
@@ -285,6 +333,7 @@ class DepthPyramid:
             self._h = C.c_void_p()
         _lib.check(_lib.lib().orbit_hiz_wrap(self.context._h, w, h, C.c_void_p(int(device_ptr)), C.byref(self._h)), "orbit_hiz_wrap")
         self.usable = False
+        self._attach()
 
     def update(self, depth_buffer):
         """depth_buffer: float32 device tensor [H, W] (reverse-Z), or a DepthImage of the same size."""
@@ -379,7 +428,7 @@ class ClusterSettings:
 @dataclass
 class GraphClusterInfo:
     """cluster.rs:352-366"""
-    light_offset_image: torch.Tensor      # uint8 view of uint2[cz][cy][cx]
+    light_offset_image: object            # uint8 tensor view of uint2[cz][cy][cx], or the ClusterGridImage it was written to
     light_index_buffer: torch.Tensor      # ClusterLightIndices
     tile_depth_slice_mask: torch.Tensor
     cluster_depth_bounds: torch.Tensor
@@ -391,11 +440,16 @@ class GraphClusterInfo:
     tile_size_px: int
 
 
-def compute_clusters(context, settings, view_matrix, projection_matrix, near, depth_buffer, scene, name="clusters"):
+def compute_clusters(context, settings, view_matrix, projection_matrix, near, depth_buffer, scene, name="clusters",
+                     light_offset_image=None):
     """cluster.rs:368-397 = mark_active_clusters + compact_active_clusters + cluster_light_assignment.
     view_matrix / projection_matrix: 4x4 math convention (Camera in the reference).
-    depth_buffer: float32 device tensor [H, W], or a DepthImage."""
+    depth_buffer: float32 device tensor [H, W], or a DepthImage.
+    light_offset_image: a ClusterGridImage of extent cluster_counts() to write the offset/count grid into (orbit_light_cluster
+    _image_grid) instead of a buffer; needs a DepthImage depth. The returned info's light_offset_image is then that object."""
     image = isinstance(depth_buffer, DepthImage)
+    if light_offset_image is not None and not image:
+        raise TypeError("compute_clusters: light_offset_image needs a DepthImage depth buffer")
     w, h = depth_buffer.size if image else (depth_buffer.shape[1], depth_buffer.shape[0])
     assert (w, h) == tuple(settings.screen_resolution)
     cx, cy, cz = settings.cluster_counts()
@@ -412,11 +466,17 @@ def compute_clusters(context, settings, view_matrix, projection_matrix, near, de
     masks = context.create_transient(name + "_tile_depth_slice_mask", 4 * cx * cy)
     bounds = context.create_transient(name + "_cluster_depth_bounds", 8 * n)
     unique = context.create_transient(name + "_unique_cluster_buffer", 16 + 4 * n)
-    offsets = context.create_transient(name + "_cluster_offset_image", 8 * n)
     cap = L.MAX_LIGHTS_PER_CLUSTER * n          # MAX_LIGHT_INDEX_COUNT in the reference is a fixed constant
     index = context.create_transient(name + "_light_index_buffer", 4 + 4 * cap)
-    fn, name_ = ((_lib.lib().orbit_light_cluster_image, "orbit_light_cluster_image") if image
-                 else (_lib.lib().orbit_light_cluster, "orbit_light_cluster"))
-    _lib.check(fn(context._h, C.byref(p), depth_buffer._h if image else _ptr(depth_buffer), _ptr(scene.light_data_buffer),
-                  _ptr(masks), _ptr(bounds), _ptr(unique), _ptr(offsets), _ptr(index), cap, _stream(context)), name_)
+    if light_offset_image is not None:
+        offsets = light_offset_image
+        _lib.check(_lib.lib().orbit_light_cluster_image_grid(context._h, C.byref(p), depth_buffer._h, _ptr(scene.light_data_buffer),
+                                                             _ptr(masks), _ptr(bounds), _ptr(unique), light_offset_image._h, _ptr(index),
+                                                             cap, _stream(context)), "orbit_light_cluster_image_grid")
+    else:
+        offsets = context.create_transient(name + "_cluster_offset_image", 8 * n)
+        fn, name_ = ((_lib.lib().orbit_light_cluster_image, "orbit_light_cluster_image") if image
+                     else (_lib.lib().orbit_light_cluster, "orbit_light_cluster"))
+        _lib.check(fn(context._h, C.byref(p), depth_buffer._h if image else _ptr(depth_buffer), _ptr(scene.light_data_buffer),
+                      _ptr(masks), _ptr(bounds), _ptr(unique), _ptr(offsets), _ptr(index), cap, _stream(context)), name_)
     return GraphClusterInfo(offsets, index, masks, bounds, unique, (cx, cy), cz, p.z_scale, p.z_bias, settings.tile_px_size()), p

@@ -15,6 +15,7 @@ pub const ORBIT_HIZ_MAX_LEVELS: usize = 16;
 #[repr(C)] pub struct orbit_ctx { _p: [u8; 0] }
 #[repr(C)] pub struct orbit_hiz { _p: [u8; 0] }
 #[repr(C)] pub struct orbit_depth_image { _p: [u8; 0] }
+#[repr(C)] pub struct orbit_cluster_grid { _p: [u8; 0] }
 
 /// = `GpuCullInfo` (draw_gen.rs:208-237), 400 bytes.
 #[repr(C)]
@@ -196,6 +197,13 @@ extern "C" {
                                      tile_masks: *mut c_void, depth_bounds: *mut c_void, unique_clusters: *mut c_void,
                                      offset_count_image: *mut c_void, light_index_list: *mut c_void, capacity_indices: u64,
                                      stream: *mut c_void) -> c_int;
+    pub fn orbit_hiz_attach_image(ctx: *mut orbit_ctx, hiz: *mut orbit_hiz, cuda_mipmapped_array: *mut c_void) -> c_int;
+    pub fn orbit_cluster_grid_wrap(ctx: *mut orbit_ctx, cuda_array: *mut c_void, out: *mut *mut orbit_cluster_grid) -> c_int;
+    pub fn orbit_cluster_grid_destroy(grid: *mut orbit_cluster_grid);
+    pub fn orbit_light_cluster_image_grid(ctx: *mut orbit_ctx, params: *const OrbitClusterParams, image: *const orbit_depth_image,
+                                          lights: *const c_void, tile_masks: *mut c_void, depth_bounds: *mut c_void,
+                                          unique_clusters: *mut c_void, grid: *const orbit_cluster_grid, light_index_list: *mut c_void,
+                                          capacity_indices: u64, stream: *mut c_void) -> c_int;
 }
 
 /// Safe-ish wrappers shaped like the reference entry points (draw_gen.rs:327-389, 456-566).
@@ -371,5 +379,40 @@ impl Context {
                                               stream: *mut c_void) -> Result<(), Error> {
         check(orbit_light_cluster_image(self.0, params, image.image, lights, tile_masks, depth_bounds, unique_clusters, offset_count_image,
                                         light_index_list, capacity_indices, stream))
+    }
+}
+
+/// The cluster offset/count grid as a CUDA array (orbit_cluster_grid_wrap): the 3-D R32G32_UINT cluster image
+/// (cluster.rs:532-544) mapped from an imported VkImage (cudaExternalMemoryGetMappedMipmappedArray, level 0), created with
+/// surface load/store. The array stays the caller's; it, and this handle, must outlive every enqueued call and captured graph
+/// that writes them.
+pub struct ClusterGrid { grid: *mut orbit_cluster_grid }
+impl ClusterGrid {
+    pub unsafe fn wrap(ctx: &Context, cuda_array: *mut c_void) -> Result<Self, Error> {
+        let mut p = std::ptr::null_mut();
+        check(orbit_cluster_grid_wrap(ctx.0, cuda_array, &mut p))?;
+        Ok(Self { grid: p })
+    }
+    pub fn as_ptr(&self) -> *const orbit_cluster_grid { self.grid }
+}
+impl Drop for ClusterGrid { fn drop(&mut self) { unsafe { orbit_cluster_grid_destroy(self.grid) } } }
+
+impl DepthPyramid {
+    /// Mirrors every later build of this pyramid into `cuda_mipmapped_array` (a cudaMipmappedArray_t with exactly this
+    /// pyramid's levels, one f32 channel, surface load/store), e.g. the renderer's pyramid image imported from Vulkan
+    /// (orbit_hiz_attach_image). The culling calls keep reading the linear pyramid; the array must outlive the pyramid.
+    pub unsafe fn attach_image(&mut self, ctx: &Context, cuda_mipmapped_array: *mut c_void) -> Result<(), Error> {
+        check(orbit_hiz_attach_image(ctx.0, self.hiz, cuda_mipmapped_array))
+    }
+}
+
+impl Context {
+    /// compute_clusters_from_image() with the offset/count grid written into `grid` (orbit_light_cluster_image_grid).
+    pub unsafe fn compute_clusters_into_grid(&self, params: &OrbitClusterParams, image: &DepthImage, lights: *const c_void,
+                                             tile_masks: *mut c_void, depth_bounds: *mut c_void, unique_clusters: *mut c_void,
+                                             grid: &ClusterGrid, light_index_list: *mut c_void, capacity_indices: u64,
+                                             stream: *mut c_void) -> Result<(), Error> {
+        check(orbit_light_cluster_image_grid(self.0, params, image.image, lights, tile_masks, depth_bounds, unique_clusters, grid.grid,
+                                             light_index_list, capacity_indices, stream))
     }
 }
